@@ -14,6 +14,7 @@ SRC = os.path.join(HERE, "csrc", "acoc_api.cu")
 DEPS = [SRC, os.path.join(HERE, "csrc", "acoc_kernels.cuh"), os.path.join(HERE, "csrc", "acoc_math.cuh"), os.path.join(HERE, "csrc", "acoc_tma.cuh"),
         os.path.join(HERE, "..", "include", "acoc.h")]
 OUT = os.path.join(HERE, "libacoc.so")
+NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-fmad=false", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
 
@@ -21,8 +22,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
 def build(force: bool = False, verbose: bool = False) -> str:
     if not force and os.path.exists(OUT) and all(os.path.getmtime(OUT) >= os.path.getmtime(d) for d in DEPS):
         return OUT
-    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", OUT, SRC]
+    cmd = [NVCC] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-o", OUT, SRC]
     subprocess.check_call(cmd)
     return OUT
 

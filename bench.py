@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload step|acro|track|single-step|single-acro]
                     [--instances M] [--precision f64|f32] [--armijo lazy|speculative] [--state f32|f64] [--no-e2e] [--no-cpu]
+                    [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...          (one rank per GPU, launched by the driver)
 
 Workloads (config.workload):
@@ -252,6 +253,33 @@ def emit(line: dict):
 
 _REAL_STDOUT = os.dup(1)
 
+DUMP_SAMPLE = 512            # instances whose trajectories --dump-outputs writes: 512 x 8 x TT float64 = 33 MB
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_sample(n):
+    """The instances --dump-outputs writes: all of a small batch, else a fixed, seeded sample (sorted)."""
+    if n <= DUMP_SAMPLE:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+
+
+def dump_outputs(d, arrays):
+    """--dump-outputs: every array as d/<name>.npy, float32 kept, everything else as float64."""
+    arrays = {k: np.ascontiguousarray(a, dtype=np.float32 if a.dtype == np.float32 else np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError("--dump-outputs: %d bytes exceed the %d-byte budget" % (total, DUMP_MAX_BYTES))
+    os.makedirs(d, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), a)
+
+
+def dump_newton(d, bn, stats, idx):
+    """What a caller of BatchedNewton.iterate receives after it: the newest iterate (xx, uu) and the per-instance statistics."""
+    xx, uu = bn.iterate_at(0)
+    dump_outputs(d, dict(xx=xx[idx], uu=uu[idx], **{k: v[idx] for k, v in stats.items()}))
+
 
 def config_dict(args, n_per_gpu, world):
     names = {"step": "BASELINE.json configs[3]: batched step-maneuver Newton, randomised step references (zf~U(1.5,3.5), xf~U(14,18), seed 2024)",
@@ -465,6 +493,8 @@ def run_batched(args, rank, world, local):
     ms = tm["total_ms"]
     launches = tm["launches"]
     st = bn.stats()
+    if args.dump_outputs and rank == 0:
+        dump_newton(args.dump_outputs, bn, st, dump_sample(n))
     its_done = int(st["iters"].astype(np.int64).sum()) - its_before  # instance-iterations actually executed in the timed region
     if dist is not None:
         import torch
@@ -640,12 +670,15 @@ def run_track(args, rank, world, local):
     dev, walls = [], []
     for k in range(W + K):
         t0 = time.perf_counter()
-        lqr_tracking_batch(xo, uo, deltas, dyn=dyn, QQt=Q, RRt=R, QQT=QT)
+        xx_reg, uu_reg = lqr_tracking_batch(xo, uo, deltas, dyn=dyn, QQt=Q, RRt=R, QQT=QT)
         t1 = time.perf_counter()
         _lib.check(_lib.lib().acoc_last_pointwise_timing(C.addressof(ms3)))
         if k >= W:
             dev.append((ms3[0], ms3[1], ms3[2]))
             walls.append(t1 - t0)
+    if args.dump_outputs and rank == 0:
+        idx = dump_sample(n)
+        dump_outputs(args.dump_outputs, dict(xx=xx_reg[idx], uu=uu_reg[idx]))
     dev = np.array(dev)
     units = n * (TT - 1)
     ms = float(dev[:, 0].mean())
@@ -721,6 +754,15 @@ def single_inputs(workload):
     return d
 
 
+def single_steps(args, d):
+    """--steps of a single-trajectory workload: the timed iterations have to end before the trajectory converges."""
+    k_max = int(d["iters"]) - args.warmup - 1
+    if args.steps > k_max:
+        sys.exit("--workload %s converges after %d Newton iterations: with --warmup %d at most %d steps can be timed"
+                 % (args.workload, int(d["iters"]), args.warmup, k_max))
+    return args.steps
+
+
 def single_config(workload):
     return {"workload": ("BASELINE.json configs[0]: main_newton_method.py step maneuver, single trajectory" if workload == "single-step" else
                          "BASELINE.json configs[1]: acrobatic_newton.py acrobatic maneuver, single trajectory"),
@@ -733,9 +775,8 @@ def run_single(args, rank, world, local):
     if rank != 0:   # a single trajectory does not shard: replicas would only repeat rank 0
         return
     d = single_inputs(args.workload)
-    K, W = args.steps, args.warmup
+    K, W = single_steps(args, d), args.warmup
     iters_ref = int(d["iters"])
-    K = min(K, iters_ref - W - 1)
     sampler = ClockSampler(local)
     sampler.start()
     with pkg.BatchedNewton(1, TT=TT, device=local, state=args.state, refs_shared=True, armijo=args.armijo, precision=args.precision) as bn:
@@ -746,6 +787,8 @@ def run_single(args, rank, world, local):
         bn.iterate(K, count_active=False)
         tm = bn.timing()
         ms, launches = tm["total_ms"], tm["launches"]
+        if args.dump_outputs:
+            dump_newton(args.dump_outputs, bn, bn.stats(), dump_sample(1))
         solves = []
         for _ in range(3):
             bn.set_init(d["xx_init"][None], d["uu_init"][None])
@@ -805,7 +848,7 @@ def run_single_reference(args, rank):
     if rank != 0:
         return
     d = single_inputs(args.workload)
-    K = min(args.steps, int(d["iters"]) - args.warmup - 1)
+    K = single_steps(args, d)
     c = single_cpu(args.workload, args.warmup, K, args.state)
     emit({"impl": "reference", "metric": METRIC, "value": c["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": K, "warmup": args.warmup,
           "ms_per_step": 1e3 / c["value"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -843,8 +886,17 @@ def main():
     ap.add_argument("--no-e2e-host", action="store_true", help="skip the second end-to-end leg (reference arrays uploaded from the host)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0; trajectories of a fixed, seeded "
+                         "sample of %d instances, float64) so that two builds can be compared output for output" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of our arm; the reference arm has none to write")
     args.warmup = max(args.warmup, 0)
+    if args.workload != "track" and args.warmup + args.steps > 199:
+        ap.error("--warmup + --steps must not exceed 199, the Newton iterations optimize() runs at most (max_iters - 1, optcon.py:415)")
     args.instances_given = args.instances is not None
     if args.chunks_generated is None:
         args.chunks_generated = 4 if int(os.environ.get("WORLD_SIZE", "1")) >= 4 else 1

@@ -6,9 +6,12 @@ product package.  All functions take / return numpy arrays in the REFERENCE's la
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -20,9 +23,16 @@ DEFAULT_PARAMS = np.array([0.1716, 2.395, 3.256, 12.0, 9.81, 0.61, 1.2, 0.24, 1e
 
 
 def build(force: bool = False) -> str:
+    """Compile libacoc_oracle.so beside its source when it is missing or older than the source; in a read-only tree it is compiled
+    into a temporary directory (removed at exit) and loaded from there."""
+    global _SO
     src = os.path.join(_HERE, "acoc_oracle.c")
     if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
-        subprocess.check_call(["make", "-C", _HERE, "-s", "-B"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        if not os.access(_HERE, os.W_OK):
+            tmp = tempfile.mkdtemp(prefix="acoc_oracle_")
+            atexit.register(shutil.rmtree, tmp, True)
+            _SO = os.path.join(tmp, "libacoc_oracle.so")
+        subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "OUT=" + _SO], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
     return _SO
 
 

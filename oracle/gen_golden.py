@@ -172,7 +172,9 @@ def _newton_job(args):
 
 
 def gen_newton(jobs):
-    work = [("step", False, (0, 9)), ("step", True, (0, 5, 9, 15)), ("acro", False, (0, 5, 9, 15)), ("acro", True, (0, 9))]
+    # step/f64 leaves out iteration 0: its LQ sub-problem is that of step/f32 bit for bit (same initial guess), and without it the
+    # fixture stays under 1 MB
+    work = [("step", False, (0, 9)), ("step", True, (5, 9, 15)), ("acro", False, (0, 5, 9, 15)), ("acro", True, (0, 9))]
     with ProcessPoolExecutor(max_workers=jobs) as ex:
         for cfg, f64, iters, wall in ex.map(_newton_job, work):
             print("newton %s f64=%s: %d iterations, %.1f s" % (cfg, f64, iters, wall), flush=True)

@@ -10,14 +10,23 @@ import subprocess
 
 import pytest
 
+from aircraftoptimalcontrol_b200 import build
 from tests.util import ROOT
 
 SO = os.path.join(ROOT, "aircraftoptimalcontrol_b200", "libacoc.so")
-pytestmark = pytest.mark.skipif(shutil.which("cuobjdump") is None or not os.path.exists(SO), reason="cuobjdump or libacoc.so missing")
+
+
+def _tool(name):
+    """A CUDA binary utility from PATH, else the one beside the nvcc that builds the library."""
+    return shutil.which(name) or shutil.which(name, path=os.path.dirname(build.NVCC))
+
+
+CUOBJDUMP, CUFILT = _tool("cuobjdump"), _tool("cu++filt")
+pytestmark = pytest.mark.skipif(CUOBJDUMP is None or CUFILT is None or not os.path.exists(SO), reason="cuobjdump, cu++filt or libacoc.so missing")
 
 
 def _run(*args):
-    return subprocess.run(["cuobjdump", *args, SO], capture_output=True, text=True, check=True, timeout=300).stdout
+    return subprocess.run([CUOBJDUMP, *args, SO], capture_output=True, text=True, check=True, timeout=300).stdout
 
 
 def test_only_sm_100a_code():
@@ -28,7 +37,7 @@ def test_only_sm_100a_code():
 
 def test_register_budgets_of_the_hot_kernels():
     res = _run("-res-usage")
-    names = subprocess.run(["cu++filt"], input="\n".join(re.findall(r"Function (\S+?):", res)), capture_output=True, text=True).stdout.split("\n")
+    names = subprocess.run([CUFILT], input="\n".join(re.findall(r"Function (\S+?):", res)), capture_output=True, text=True).stdout.split("\n")
     regs = {}
     for (_, usage), name in zip(re.findall(r"Function (\S+?):\s*\n\s*(.*)", res), names):
         short = re.sub(r"\(.*", "", name.replace("acoc::", "").replace("(bool)", "").replace("(int)", "").replace("void ", ""))
