@@ -75,6 +75,11 @@ def _sig(lib):
         "acoc_get_gains": [vp, vp, vp],
         "acoc_get_history": [vp, vp, vp, vp, vp],
         "acoc_get_stats": [vp, vp, vp, vp, vp, vp],
+        "acoc_track": [vp] * 8,
+        "acoc_get_tracked": [vp, vp, vp],
+        "acoc_get_track_gains": [vp, vp],
+        "acoc_get_track_timing": [vp, vp],
+        "acoc_lqr_tracking_many": [i, i, i, vp, i] + [vp] * 9,
         "acoc_eval_cost": [vp, vp],
         "acoc_set_deltau": [vp, vp],
         "acoc_set_scalars": [vp, vp, vp],

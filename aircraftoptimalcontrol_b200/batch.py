@@ -287,6 +287,52 @@ class BatchedNewton:
         L.check(L.lib().acoc_get_stats(self._h, L.ptr(it), L.ptr(st), L.ptr(J), L.ptr(d), L.ptr(nr)))
         return dict(iters=it, status=st, J=J, descent=d, n_reg=nr)
 
+    # -- closed-loop tracking of every instance (lqr_tracking.py:245-283 per instance) ---------------------------------------------
+    def track(self, delta=None, QQt=None, RRt=None, QQT=None):
+        """Fly the closed loop of the reference's lqr_tracking around EVERY instance's own result (what result() returns now), on the
+        device: gains of the time-varying LQR along that nominal with the tracking weights (default lqr_tracking.default_weights(),
+        independent of the Newton weights), then u = u* + K (x - x*) from x*_0 + delta.  delta (N,6), (6,) broadcast, or None (zero).
+        Returns dict(err_max (N,6) = max_t |x_t - x*_t|, err_final (N,6) at t = TT-1, n_reg (N) = steps that took the +0.5 I gain
+        branch); NaN summaries mark an instance whose nominal is not finite.  Trajectories: tracked(); gains: track_gains().
+        Changes nothing of the solve."""
+        from .lqr_tracking import default_weights
+        dQ, dR, dQT = default_weights()
+        Q = L.f64(dQ if QQt is None else QQt, (6, 6), "QQt")
+        R = L.f64(dR if RRt is None else RRt, (2, 2), "RRt")
+        QT = L.f64(dQT if QQT is None else QQT, (6, 6), "QQT")
+        d = None
+        if delta is not None:
+            d = np.asarray(delta, dtype=np.float64)
+            if d.shape == (6,):
+                d = np.broadcast_to(d, (self.N, 6))
+            d = L.f64(d, (self.N, 6), "delta")
+        em, ef, nr = np.empty((self.N, 6)), np.empty((self.N, 6)), np.empty(self.N, dtype=np.int32)
+        L.check(L.lib().acoc_track(self._h, L.ptr(Q), L.ptr(R), L.ptr(QT), L.ptr(d), L.ptr(em), L.ptr(ef), L.ptr(nr)))
+        return dict(err_max=em, err_final=ef, n_reg=nr)
+
+    def tracked(self, out=None):
+        """(xx_reg (N,6,TT), uu_reg (N,2,TT)) of the last track()."""
+        if out is None:
+            xr, ur = np.empty((self.N, 6, self.TT)), np.empty((self.N, 2, self.TT))
+        else:
+            xr, ur = out
+            L.out_array(xr, (self.N, 6, self.TT), np.float64, "xx_reg")
+            L.out_array(ur, (self.N, 2, self.TT), np.float64, "uu_reg")
+        L.check(L.lib().acoc_get_tracked(self._h, L.ptr(xr), L.ptr(ur)))
+        return xr, ur
+
+    def track_gains(self):
+        """K (N,2,6,TT) of the last track(): lqr_tracking's KK for every instance."""
+        K = np.empty((self.N, 2, 6, self.TT))
+        L.check(L.lib().acoc_get_track_gains(self._h, L.ptr(K)))
+        return K
+
+    def track_timing(self):
+        """Device time (ms) of the last track(): total and per kernel (nominal, gains sweep, rollout)."""
+        ms = (C.c_double * 4)()
+        L.check(L.lib().acoc_get_track_timing(self._h, C.addressof(ms)))
+        return dict(total_ms=ms[0], nominal_ms=ms[1], gains_ms=ms[2], rollout_ms=ms[3])
+
     def set_profiling(self, on=True):
         L.check(L.lib().acoc_set_profiling(self._h, int(bool(on))))
 
@@ -429,3 +475,24 @@ class PipelinedNewton:
         if f32:
             stats["x0"] = x0_out
         return xs, us, stats
+
+    def track(self, delta=None, QQt=None, RRt=None, QQT=None):
+        """BatchedNewton.track on every sub-batch (each on its own context): delta (N,6) or (6,); returns the concatenated summaries."""
+        d = None
+        if delta is not None:
+            d = np.asarray(delta, dtype=np.float64)
+            if d.shape == (6,):
+                d = np.broadcast_to(d, (self.N, 6))
+            if d.shape != (self.N, 6):
+                raise ValueError("delta has shape %s, expected %s or (6,)" % (d.shape, (self.N, 6)))
+        res = [p.track(None if d is None else d[lo:hi], QQt, RRt, QQT) for p, lo, hi in zip(self.parts, self.bounds[:-1], self.bounds[1:])]
+        return {k: np.concatenate([r[k] for r in res]) for k in ("err_max", "err_final", "n_reg")}
+
+    def tracked(self, out=None):
+        """(xx_reg (N,6,TT), uu_reg (N,2,TT)) of the last track()."""
+        xr, ur = out if out is not None else (np.empty((self.N, 6, self.TT)), np.empty((self.N, 2, self.TT)))
+        L.out_array(xr, (self.N, 6, self.TT), np.float64, "xx_reg")
+        L.out_array(ur, (self.N, 2, self.TT), np.float64, "uu_reg")
+        for p, lo, hi in zip(self.parts, self.bounds[:-1], self.bounds[1:]):
+            p.tracked(out=(xr[lo:hi], ur[lo:hi]))
+        return xr, ur

@@ -68,6 +68,7 @@ static int fail(int code, const char* fmt, ...)
 // ======================================================================================================
 constexpr int ST_PAD = 4;  // padding lanes beyond N: never active
 constexpr unsigned ACOC_CTX_LITE = 0x40000000u;  // internal flag of acoc_ctx_create (not part of the ABI), see there
+constexpr unsigned ACOC_CTX_NO_SLOTS = 0x20000000u;  // internal, with ACOC_CTX_LITE: no iterate slot either (acoc_lqr_tracking_many)
 
 // granularity of the active-work list of the sweeps: groups of 2^shift consecutive instances that still contain an active one
 #ifndef ACOC_ACT_SHIFT
@@ -467,6 +468,57 @@ __global__ void __launch_bounds__(ROLL_THREADS) k_track(Problem P, const double*
     track_instance<Q32>(P, Kt, xopt, uopt, xstart, Xn, Un, i);
 }
 
+// ---- closed-loop tracking of every instance (acoc_track) --------------------------------------------------------------------------
+// The nominal of each instance = what acoc_get_result returns (slot per instance, -1 = all zeros, u[TT-1] = u[TT-2], exact row 0), copied
+// into dedicated warp-tiled buffers: the lanes of one tile may have their results in different slots, and a warp-private TMA ring copies
+// the block of ONE array.  Thread = (instance, chunk of tchunk time steps).
+template <typename XT>
+__global__ void __launch_bounds__(128) k_track_nominal(const XT* __restrict__ X0, const XT* __restrict__ X1, const XT* __restrict__ X2,
+                                                       const double* __restrict__ U0, const double* __restrict__ U1,
+                                                       const double* __restrict__ U2, const int* __restrict__ slot,
+                                                       const double* __restrict__ x0, XT* __restrict__ Xnom, double* __restrict__ Unom,
+                                                       double* __restrict__ xnom0, int N, int Np, int TT, int tchunk)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const int sl = slot[i];
+    const XT* X = sl == 0 ? X0 : (sl == 1 ? X1 : X2);
+    const double* U = sl == 0 ? U0 : (sl == 1 ? U1 : U2);
+    const int t0 = blockIdx.y * tchunk, t1 = min(TT, t0 + tchunk);
+    for (int t = t0; t < t1; ++t) {
+        const int tu = t == TT - 1 ? TT - 2 : t;  // uu_star[:,-1] = uu_star[:,-2], optcon.py:505
+#pragma unroll
+        for (int c = 0; c < NS; ++c) Xnom[at(t, NS, c, Np, i)] = sl < 0 ? XT(0) : X[at(t, NS, c, Np, i)];
+#pragma unroll
+        for (int c = 0; c < NI; ++c) Unom[at(t, NI, c, Np, i)] = sl < 0 ? 0.0 : U[at(tu, NI, c, Np, i)];
+    }
+    if (blockIdx.y == 0) {
+#pragma unroll
+        for (int c = 0; c < NS; ++c)
+            xnom0[(size_t)c * Np + i] = sl < 0 ? 0.0 : (std::is_same<XT, float>::value ? x0[(size_t)c * Np + i] : (double)X[at(0, NS, c, Np, i)]);
+    }
+}
+
+// the tracking sweeps with plain global loads (ACOC_NO_TMA): same per-instance functions as the TMA rings
+template <int DG, typename XT>
+__global__ void __launch_bounds__(64) k_track_gains(Problem P, const XT* __restrict__ Xnom, const double* __restrict__ Unom,
+                                                    double* __restrict__ Ktrk, int* __restrict__ n_reg)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P.N) return;
+    n_reg[i] = track_gains_instance<DG>(P, Xnom, Unom, Ktrk, i);
+}
+template <bool Q32, typename XT>
+__global__ void __launch_bounds__(64) k_track_rollout(Problem P, const XT* __restrict__ Xnom, const double* __restrict__ Unom,
+                                                      const double* __restrict__ Ktrk, const double* __restrict__ delta, XT* __restrict__ Xtrk,
+                                                      double* __restrict__ xtrk0, double* __restrict__ Utrk, double* __restrict__ err_max,
+                                                      double* __restrict__ err_final)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P.N) return;
+    track_rollout_instance<Q32>(P, Xnom, Unom, Ktrk, delta, Xtrk, xtrk0, Utrk, err_max, err_final, i);
+}
+
 // dx0 and x0_out may alias (each thread reads its dx0 before it writes its x0)
 template <bool Q32, typename F, typename XT>
 __global__ void __launch_bounds__(ROLL_THREADS) k_init_guess(ProblemT<F> P, double kp, double kt, const F* dx0, XT* __restrict__ Xn,
@@ -860,6 +912,15 @@ struct acoc_ctx {
     double* candJ = nullptr;    // [Np] cost of the row k_pick copied
     size_t cand_bytes_x = 0, cand_bytes_u = 0;
     bool cand_failed = false;   // the buffers could not be allocated: separate sweeps
+    // closed-loop tracking (acoc_track, acoc_lqr_tracking_many), allocated on the first call: nominal Xnom / Unom + exact row 0, gains
+    // Ktrk, tracked Xtrk / Utrk + exact row 0 (warp-tiled), delta and summaries [6][Np], n_reg [Np].  State buffers hold tk_es-byte elements.
+    void *tk_xnom = nullptr, *tk_unom = nullptr, *tk_xnom0 = nullptr, *tk_K = nullptr, *tk_x = nullptr, *tk_x0 = nullptr, *tk_u = nullptr;
+    void *tk_delta = nullptr, *tk_emax = nullptr, *tk_efin = nullptr;
+    int* tk_nreg = nullptr;
+    size_t tk_es = 0;           // 0: not allocated
+    bool tk_done = false, tk_xfloat = false;  // Xtrk holds the result of a tracking call; its element type
+    cudaEvent_t tk_ev[4] = {};
+    double tk_ms[4] = {0, 0, 0, 0};
 };
 
 static int dalloc_bytes(acoc_ctx* c, void** p, size_t bytes)
@@ -1265,7 +1326,8 @@ int acoc_ctx_create(int device, int n_instances, int TT, unsigned flags, acoc_ct
     int rc = 0;
     // (internal) a context that only hosts one trajectory slot: acoc_lqr_tracking rolls out into X[0]/U[0] and needs no Newton state
     const bool lite = (flags & ACOC_CTX_LITE) != 0;
-    for (int s = 0; s < (lite ? 1 : 3) && !rc; ++s) { rc = dalloc_bytes(c, &c->X[s], T * 6 * Np * es); if (!rc) rc = dalloc_bytes(c, &c->U[s], T * 2 * Np * es); }
+    const int n_slots = lite ? ((flags & ACOC_CTX_NO_SLOTS) ? 0 : 1) : 3;
+    for (int s = 0; s < n_slots && !rc; ++s) { rc = dalloc_bytes(c, &c->X[s], T * 6 * Np * es); if (!rc) rc = dalloc_bytes(c, &c->U[s], T * 2 * Np * es); }
     if (!rc) rc = dalloc_bytes(c, &c->DU, lite ? 64 : T * 2 * Np * es);
     if (!rc) rc = dalloc_bytes(c, &c->KSG, lite ? 64 : T * 16 * Np * es);
     const bool shared = flags & ACOC_REFS_SHARED;
@@ -1330,6 +1392,7 @@ int acoc_ctx_destroy(acoc_ctx* c)
     }
     if (c->dstream) { cudaStreamSynchronize(c->dstream); cudaStreamDestroy(c->dstream); }
     if (c->ev_deliver) cudaEventDestroy(c->ev_deliver);
+    for (auto& e : c->tk_ev) if (e) cudaEventDestroy(e);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
     return 0;
@@ -2865,6 +2928,238 @@ int acoc_last_pointwise_timing(double* ms)
 {
     REQUIRE(ms, "NULL output");
     for (int k = 0; k < 3; ++k) ms[k] = g_pt_ms[k];
+    return 0;
+}
+
+// ======================================================================================================
+// closed-loop LQR tracking of every instance along its own nominal (lqr_tracking.py:245-283 per instance)
+// ======================================================================================================
+static void free_track_buffers(acoc_ctx* c)
+{
+    dfree(c, &c->tk_xnom); dfree(c, &c->tk_unom); dfree(c, &c->tk_xnom0); dfree(c, &c->tk_K); dfree(c, &c->tk_x); dfree(c, &c->tk_x0);
+    dfree(c, &c->tk_u); dfree(c, &c->tk_delta); dfree(c, &c->tk_emax); dfree(c, &c->tk_efin); dfree(c, &c->tk_nreg);
+    c->tk_es = 0;
+    c->tk_done = false;
+}
+
+// the tracking buffers for state elements of es bytes (reallocated when the storage type changes); ACOC_ERR_NOMEM leaves none behind
+static int ensure_track_buffers(acoc_ctx* c, size_t es)
+{
+    if (c->tk_es == es) return 0;
+    CK(cudaStreamSynchronize(c->stream));
+    free_track_buffers(c);
+    const size_t T = c->TT, Np = c->Np, d = sizeof(double);
+    int rc = dalloc_bytes(c, &c->tk_xnom, T * NS * Np * es);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_unom, T * NI * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_K, T * 2 * NS * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_x, T * NS * Np * es);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_u, T * NI * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_xnom0, NS * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_x0, NS * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_delta, NS * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_emax, NS * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_efin, NS * Np * d);
+    if (!rc) rc = dalloc(c, &c->tk_nreg, Np);
+    for (auto& e : c->tk_ev)
+        if (!rc && !e && cudaEventCreate(&e) != cudaSuccess) rc = fail(ACOC_ERR_CUDA, "cudaEventCreate failed");
+    if (rc) { free_track_buffers(c); return rc; }
+    c->tk_es = es;
+    return 0;
+}
+
+// Q, R, QT of the tracking cost: symmetric like acoc_set_weights (the gains sweep carries P as its upper triangle)
+static int track_weights(const double* Q, const double* R, const double* QT, Weights* W)
+{
+    REQUIRE(Q && R && QT, "tracking weights: NULL argument");
+    REQUIRE(is_sym(Q, 6) && is_sym(R, 2) && is_sym(QT, 6), "tracking weights: Q, R and QT must be symmetric");
+    fill_weights(W, Q, R, QT);
+    return 0;
+}
+
+// host delta (N,6) or NULL (zeros) -> device [6][Np]
+static int upload_delta(acoc_ctx* c, const double* delta)
+{
+    if (!delta) { CK(cudaMemsetAsync(c->tk_delta, 0, (size_t)NS * c->Np * sizeof(double), c->stream)); return 0; }
+    std::vector<double> tmp((size_t)NS * c->Np, 0.0);
+    for (int i = 0; i < c->N; ++i) for (int k = 0; k < NS; ++k) tmp[(size_t)k * c->Np + i] = delta[(size_t)i * NS + k];
+    CK(cudaMemcpyAsync(c->tk_delta, tmp.data(), tmp.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaStreamSynchronize(c->stream));  // tmp goes out of scope
+    return 0;
+}
+
+// gains sweep + closed-loop rollout over the nominal in tk_xnom / tk_unom / tk_xnom0 (events tk_ev[1..3])
+template <typename XT>
+static int launch_track_sweeps(acoc_ctx* c, const Weights& W)
+{
+    Problem P = prob<double>(c);
+    P.W = W;
+    P.x0 = (const double*)c->tk_xnom0;  // exact row 0 of the nominal (finish_x)
+    const XT* Xn = (const XT*)c->tk_xnom;
+    const double *Un = (const double*)c->tk_unom, *dl = (const double*)c->tk_delta;
+    double *K = (double*)c->tk_K, *x0 = (double*)c->tk_x0, *U = (double*)c->tk_u, *em = (double*)c->tk_emax, *ef = (double*)c->tk_efin;
+    XT* X = (XT*)c->tk_x;
+    cudaStream_t st = c->stream;
+    const int g = (c->N + 63) / 64;  // 64 threads = two tiles per CTA
+    CK(cudaEventRecord(c->tk_ev[1], st));
+    if (use_tma(c)) {
+        const size_t sm = WarpRing<TRK_GAIN_STAGES, TrkGainStage<XT>::BYTES>::smem_bytes(2);
+        if (W.diag) { TRY(prefer_smem(k_track_gains_tma<1, XT>)); k_track_gains_tma<1, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, c->tk_nreg); }
+        else { TRY(prefer_smem(k_track_gains_tma<0, XT>)); k_track_gains_tma<0, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, c->tk_nreg); }
+    } else if (W.diag) k_track_gains<1, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, c->tk_nreg);
+    else k_track_gains<0, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, c->tk_nreg);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(c->tk_ev[2], st));
+    if (use_tma(c)) {
+        const size_t sm = WarpRing<TRK_ROLL_STAGES, TrkRollStage<XT>::BYTES>::smem_bytes(2);
+        if (c->P.q32) {
+            TRY(prefer_smem(k_track_rollout_tma<true, XT>));
+            k_track_rollout_tma<true, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, dl, X, x0, U, em, ef);
+        } else {
+            TRY(prefer_smem(k_track_rollout_tma<false, XT>));
+            k_track_rollout_tma<false, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, dl, X, x0, U, em, ef);
+        }
+    } else LAUNCH_Q32(c->P.q32, k_track_rollout, (XT), g, 64, st, P, Xn, Un, K, dl, X, x0, U, em, ef);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(c->tk_ev[3], st));
+    return 0;
+}
+
+// after the sweeps: wait, read the event times, mark the outputs valid
+static int track_finish(acoc_ctx* c, bool xfloat)
+{
+    CK(cudaStreamSynchronize(c->stream));
+    float a = 0, b = 0, r = 0;
+    CK(cudaEventElapsedTime(&a, c->tk_ev[0], c->tk_ev[1]));
+    CK(cudaEventElapsedTime(&b, c->tk_ev[1], c->tk_ev[2]));
+    CK(cudaEventElapsedTime(&r, c->tk_ev[2], c->tk_ev[3]));
+    c->tk_ms[0] = (double)a + b + r; c->tk_ms[1] = a; c->tk_ms[2] = b; c->tk_ms[3] = r;
+    c->tk_done = true;
+    c->tk_xfloat = xfloat;
+    return 0;
+}
+
+static int download_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg)
+{
+    const double* row0 = (const double*)c->tk_x0;
+    if (xx_reg) {
+        if (c->tk_xfloat) TRY((download_soa_t<float>(c, c->tk_x, nullptr, nullptr, nullptr, row0, xx_reg, c->N, NS, c->Np, 0)));
+        else TRY((download_soa_t<double>(c, c->tk_x, nullptr, nullptr, nullptr, row0, xx_reg, c->N, NS, c->Np, 0)));
+    }
+    if (uu_reg) TRY((download_soa_t<double>(c, c->tk_u, nullptr, nullptr, nullptr, nullptr, uu_reg, c->N, NI, c->Np, 0)));
+    return 0;
+}
+
+// device [6][Np] -> host (N,6)
+template <typename T>
+static int download_rows(acoc_ctx* c, const void* dev, T* host, int rows)
+{
+    if (!host) return 0;
+    std::vector<T> tmp((size_t)rows * c->Np);
+    CK(cudaMemcpyAsync(tmp.data(), dev, tmp.size() * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    for (int i = 0; i < c->N; ++i) for (int k = 0; k < rows; ++k) host[(size_t)i * rows + k] = tmp[(size_t)k * c->Np + i];
+    return 0;
+}
+
+int acoc_track(acoc_ctx* c, const double* Q, const double* R, const double* QT, const double* delta, double* err_max, double* err_final,
+               int* n_reg)
+{
+    REQUIRE(c, "ctx is NULL");
+    if (c->fp32) return fail(ACOC_ERR_STATE, "acoc_track: not available in the FP32 mode (ACOC_FP32)");
+    if (!c->have_init) return fail(ACOC_ERR_STATE, "acoc_track: no iterate to track yet: call acoc_set_init or acoc_init_guess first");
+    Weights W;
+    TRY(track_weights(Q, R, QT, &W));
+    TRY(use_device(c->device));
+    const bool xf = c->x_float;
+    TRY(ensure_track_buffers(c, xf ? sizeof(float) : sizeof(double)));
+    TRY(upload_delta(c, delta));
+    CK(cudaEventRecord(c->tk_ev[0], c->stream));
+    k_result_slot_default<<<(c->N + 255) / 256, 256, 0, c->stream>>>(c->S.status, c->slot_tmp, c->S.result_slot, c->kk % 3, c->N);
+    const int tchunk = 8;
+    const dim3 grid((unsigned)((c->N + 127) / 128), (unsigned)((c->TT + tchunk - 1) / tchunk));
+    if (xf)
+        k_track_nominal<float><<<grid, 128, 0, c->stream>>>((const float*)c->X[0], (const float*)c->X[1], (const float*)c->X[2], (const double*)c->U[0],
+                                                            (const double*)c->U[1], (const double*)c->U[2], c->slot_tmp, (const double*)c->x0,
+                                                            (float*)c->tk_xnom, (double*)c->tk_unom, (double*)c->tk_xnom0, c->N, c->Np, c->TT, tchunk);
+    else
+        k_track_nominal<double><<<grid, 128, 0, c->stream>>>((const double*)c->X[0], (const double*)c->X[1], (const double*)c->X[2],
+                                                             (const double*)c->U[0], (const double*)c->U[1], (const double*)c->U[2], c->slot_tmp,
+                                                             (const double*)c->x0, (double*)c->tk_xnom, (double*)c->tk_unom, (double*)c->tk_xnom0,
+                                                             c->N, c->Np, c->TT, tchunk);
+    CK(cudaGetLastError());
+    TRY(xf ? launch_track_sweeps<float>(c, W) : launch_track_sweeps<double>(c, W));
+    TRY(track_finish(c, xf));
+    TRY(download_rows(c, c->tk_emax, err_max, NS));
+    TRY(download_rows(c, c->tk_efin, err_final, NS));
+    TRY(download_rows(c, c->tk_nreg, n_reg, 1));
+    return 0;
+}
+
+int acoc_get_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg)
+{
+    REQUIRE(c, "ctx is NULL");
+    if (!c->tk_done) return fail(ACOC_ERR_STATE, "acoc_get_tracked: call acoc_track first");
+    TRY(use_device(c->device));
+    return download_tracked(c, xx_reg, uu_reg);
+}
+
+int acoc_get_track_gains(acoc_ctx* c, double* K)
+{
+    REQUIRE(c && K, "NULL argument");
+    if (!c->tk_done) return fail(ACOC_ERR_STATE, "acoc_get_track_gains: call acoc_track first");
+    TRY(use_device(c->device));
+    // Ktrk as a trajectory with 12 components downloads to (N,12,TT) = (N,2,6,TT)
+    return download_soa_t<double>(c, c->tk_K, nullptr, nullptr, nullptr, nullptr, K, c->N, 2 * NS, c->Np, 0);
+}
+
+int acoc_get_track_timing(acoc_ctx* c, double* ms)
+{
+    REQUIRE(c && ms, "NULL argument");
+    if (!c->tk_done) return fail(ACOC_ERR_STATE, "acoc_get_track_timing: call acoc_track first");
+    for (int k = 0; k < 4; ++k) ms[k] = c->tk_ms[k];
+    return 0;
+}
+
+int acoc_lqr_tracking_many(int device, int n, int TT, const double* params, int state_f64, const double* Q, const double* R, const double* QT,
+                           const double* xx_opt, const double* uu_opt, const double* delta, double* xx_reg, double* uu_reg, double* K)
+{
+    REQUIRE(n > 0 && TT >= 3 && params && xx_opt && uu_opt && delta && xx_reg && uu_reg, "acoc_lqr_tracking_many: bad argument");
+    REQUIRE(params[3] != 0.0 && params[7] != 0.0, "acoc_lqr_tracking_many: mass and inertia must be non-zero");
+    Weights W;
+    TRY(track_weights(Q, R, QT, &W));
+    // one context without iterate slots per (device, n, TT, quantisation), kept between calls: no allocation once it exists
+    static std::mutex mu;
+    static acoc_ctx* cached = nullptr;
+    std::lock_guard<std::mutex> lock(mu);
+    const unsigned flags = (state_f64 ? ACOC_STATE_F64 : 0) | ACOC_REFS_SHARED | ACOC_CTX_LITE | ACOC_CTX_NO_SLOTS;
+    if (cached && (cached->device != device || cached->N != n || cached->TT != TT || cached->flags != flags)) { acoc_ctx_destroy(cached); cached = nullptr; }
+    if (!cached) TRY(acoc_ctx_create(device, n, TT, flags, &cached));
+    acoc_ctx* c = cached;
+    TRY(use_device(device));
+    TRY(acoc_set_model(c, params));
+    // the nominals go straight into Xnom / Unom: float storage when every state at t >= 1 is a float32 value (as acoc_set_init decides),
+    // the exact row 0 always
+    bool xf = false;
+    if (c->P.q32) {
+        TRY(ensure_track_buffers(c, sizeof(float)));
+        CK(cudaMemsetAsync(c->counters + 3, 0, sizeof(int), c->stream));
+        TRY((upload_soa_t<float, double>(c, xx_opt, c->tk_xnom, n, NS, c->Np, (double*)c->tk_xnom0, c->counters + 3)));
+        int inexact = 0;
+        CK(cudaMemcpyAsync(&inexact, c->counters + 3, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        xf = !inexact;
+    }
+    if (!xf) {
+        TRY(ensure_track_buffers(c, sizeof(double)));
+        TRY((upload_soa_t<double, double>(c, xx_opt, c->tk_xnom, n, NS, c->Np, (double*)c->tk_xnom0, (int*)nullptr)));
+    }
+    TRY((upload_soa_t<double, double>(c, uu_opt, c->tk_unom, n, NI, c->Np, (double*)nullptr, (int*)nullptr)));
+    TRY(upload_delta(c, delta));
+    CK(cudaEventRecord(c->tk_ev[0], c->stream));
+    TRY(xf ? launch_track_sweeps<float>(c, W) : launch_track_sweeps<double>(c, W));
+    TRY(track_finish(c, xf));
+    TRY(download_tracked(c, xx_reg, uu_reg));
+    if (K) TRY(download_soa_t<double>(c, c->tk_K, nullptr, nullptr, nullptr, nullptr, K, n, 2 * NS, c->Np, 0));
     return 0;
 }
 

@@ -18,6 +18,8 @@
 //   rollout_instance      optcon.py:247-264 (one Armijo candidate) and :176-200 (get_update)
 //   armijo_select_instance optcon.py:266-273, :327 and the bookkeeping of :488-501
 //   track_instance        lqr_tracking.py:279-281
+//   track_gains_instance, lqr_tracking.py:245-283 along each instance's own nominal (gains, closed loop, summaries)
+//   track_rollout_instance
 //   init_guess_instance   aircraft_simplified.py:142-147
 //
 // Types: F is the arithmetic type and the storage type of U, DU, KSG, the references and x0 (double = the parity path,
@@ -822,6 +824,20 @@ ACOC_HD void newton_finish_instance(const NewtonOpts& O, const NewtonState& S, d
 // ------------------------------------------------------------------------------------------------------
 // closed-loop tracking rollout, lqr_tracking.py:279-281: u = u_opt + K (x - x_opt) with shared K, nominal
 // ------------------------------------------------------------------------------------------------------
+// the input of one closed-loop step: u = u_opt + K@(x - x_opt), K row-major 2x6.  Plain sums in index order (the reference's 2x6
+// matvec), then u_opt + (.)
+template <typename F>
+ACOC_HD void track_input(const F* K, const F* x, const F* xopt, const F* uopt, F* u)
+{
+#pragma unroll
+    for (int a = 0; a < NI; ++a) {
+        F s = F(0.0);
+#pragma unroll
+        for (int c = 0; c < NS; ++c) s += K[a * NS + c] * (x[c] - xopt[c]);
+        u[a] = uopt[a] + s;
+    }
+}
+
 // Kt: [TT][12] (row-major 2x6), xopt [TT][6], uopt [TT][2] shared by all instances; x_start [6][Np].
 template <bool Q32, typename F, typename XT>
 ACOC_HD void track_instance(const ProblemT<F>& P, const F* Kt, const F* xopt, const F* uopt,
@@ -832,15 +848,7 @@ ACOC_HD void track_instance(const ProblemT<F>& P, const F* Kt, const F* xopt, co
 #pragma unroll
     for (int c = 0; c < NS; ++c) x[c] = xstart[(size_t)c * Np + i];
     for (int t = 0; t < TT - 1; ++t) {
-        const F* K = Kt + (size_t)t * 12;
-        // K@(x - x_opt): plain sums in index order (the reference's 2x6 matvec), then u_opt + (.)
-#pragma unroll
-        for (int a = 0; a < NI; ++a) {
-            F s = F(0.0);
-#pragma unroll
-            for (int c = 0; c < NS; ++c) s += K[a * NS + c] * (x[c] - xopt[t * NS + c]);
-            u[a] = uopt[t * NI + a] + s;
-        }
+        track_input(Kt + (size_t)t * 12, x, xopt + (size_t)t * NS, uopt + (size_t)t * NI, u);
         store_x(Xn, t, Np, i, x);
 #pragma unroll
         for (int c = 0; c < NI; ++c) Un[at(t, NI, c, Np, i)] = u[c];
@@ -852,6 +860,124 @@ ACOC_HD void track_instance(const ProblemT<F>& P, const F* Kt, const F* xopt, co
     store_x(Xn, TT - 1, Np, i, x);
     Un[at(TT - 1, NI, 0, Np, i)] = F(0.0);
     Un[at(TT - 1, NI, 1, Np, i)] = F(0.0);
+}
+
+// ------------------------------------------------------------------------------------------------------
+// closed-loop LQR tracking of every instance along its OWN nominal, lqr_tracking.py:245-283 (acoc_track, acoc_lqr_tracking_many)
+// ------------------------------------------------------------------------------------------------------
+// Each instance is one call of the reference's lqr_tracking: nominal Xnom/Unom (warp-tiled like the iterates, Ktrk [TT][Np/32][12][32]),
+// P.W = the TRACKING weights, P.x0 = the exact row 0 of the nominal (finish_x reads it when Xnom is float).
+// Gains (:276, non-augmented ltv_LQR): riccati_matrix<false> with q = r = 0 on the linearisation at (x*_t, u*_t), from P_{TT-1} = QT; the
+// affine terms it also carries stay zero (NaN along a non-finite nominal) and do not enter K.  K_{TT-1} = 0 (ltv_LQR never assigns it).
+template <int DG = -1, typename F>
+ACOC_HD void track_terminal(const WeightsT<F>& W, F* Pm, F* p)
+{
+#pragma unroll
+    for (int a = 0; a < NS; ++a) {
+        p[a] = F(0.0);
+#pragma unroll
+        for (int b = a; b < NS; ++b) Pm[sym(a, b)] = weights_diag<DG>(W) ? (a == b ? W.QT[a * 7] : F(0.0)) : W.QT[a * 6 + b];
+    }
+}
+
+// one step of the gains sweep: (x*_t, u*_t) and the carried (P, p) -> K_t.  Returns 1 if the gain took the +0.5 I branch.
+template <int DG = -1, typename F>
+ACOC_HD int track_gains_step(const ModelT<F>& M, const WeightsT<F>& W, const F* x, const F* u, F* Pm, F* p, F* K)
+{
+    const F q[NS] = {F(0.0), F(0.0), F(0.0), F(0.0), F(0.0), F(0.0)}, r[NI] = {F(0.0), F(0.0)};
+    const Trig<F> tg = make_trig(x);
+    const Lin<F> l = linearize(M, x, u, tg);
+    Hess<F> h;
+    F sig[NI];
+    return riccati_matrix<false, DG, F>(M, W, l, h, q, r, Pm, p, K, sig);
+}
+
+template <int DG, typename F, typename XT>
+ACOC_HD int track_gains_instance(const ProblemT<F>& P, const XT* Xnom, const F* Unom, F* Ktrk, int i)
+{
+    const int TT = P.TT, Np = P.Np;
+    F Pm[21], p[NS], x[NS], u[NI], K[2 * NS];
+    track_terminal<DG>(P.W, Pm, p);
+#pragma unroll
+    for (int c = 0; c < 2 * NS; ++c) Ktrk[at(TT - 1, 2 * NS, c, Np, i)] = F(0.0);
+    int nreg = 0;
+    for (int t = TT - 2; t >= 0; --t) {
+        load_x(P, Xnom, t, i, x);
+#pragma unroll
+        for (int c = 0; c < NI; ++c) u[c] = Unom[at(t, NI, c, Np, i)];
+        nreg += track_gains_step<DG>(P.M, P.W, x, u, Pm, p, K);
+#pragma unroll
+        for (int c = 0; c < 2 * NS; ++c) Ktrk[at(t, 2 * NS, c, Np, i)] = K[c];
+    }
+    return nreg;
+}
+
+// running max that keeps a NaN once it has seen one (fmax would drop it)
+template <typename F>
+ACOC_HD F max_nan(F m, F v) { return (v > m || v != v) ? v : m; }
+
+// closed loop (:279-281): x_0 = x*_0 + delta; u_t = u*_t + K_t (x_t - x*_t), x_{t+1} = f(x_t, u_t) for t < TT-1; u_{TT-1} = 0.
+// Summaries: err_max[c] = max_t |x_t[c] - x*_t[c]|, err_final[c] at t = TT-1 ([6][Np] each).  Row 0 of a float Xtrk is not exact:
+// the exact x_0 goes to xtrk0 [6][Np].
+template <typename F>
+ACOC_HD void track_error(const F* x, const F* xnom, F* emax)
+{
+#pragma unroll
+    for (int c = 0; c < NS; ++c) emax[c] = max_nan(emax[c], F(fabs(x[c] - xnom[c])));
+}
+template <bool Q32, typename F>
+ACOC_HD void track_advance(const ModelT<F>& M, F* x, const F* u)
+{
+    const Trig<F> tg = make_trig(x);
+    F xn[NS];
+    next_state<Q32>(M, x, u, tg, xn);
+#pragma unroll
+    for (int c = 0; c < NS; ++c) x[c] = xn[c];
+}
+template <typename F>
+ACOC_HD void track_start(const ProblemT<F>& P, const F* delta, int i, F* x, F* emax)
+{
+#pragma unroll
+    for (int c = 0; c < NS; ++c) { x[c] = P.x0[(size_t)c * P.Np + i] + delta[(size_t)c * P.Np + i]; emax[c] = F(0.0); }
+}
+template <typename F>
+ACOC_HD void track_final(const F* x, const F* xnom, F* emax, F* err_max, F* err_final, int Np, int i)
+{
+    track_error(x, xnom, emax);
+#pragma unroll
+    for (int c = 0; c < NS; ++c) {
+        err_max[(size_t)c * Np + i] = emax[c];
+        err_final[(size_t)c * Np + i] = F(fabs(x[c] - xnom[c]));
+    }
+}
+
+template <bool Q32, typename F, typename XT>
+ACOC_HD void track_rollout_instance(const ProblemT<F>& P, const XT* Xnom, const F* Unom, const F* Ktrk, const F* delta, XT* Xtrk, F* xtrk0,
+                                    F* Utrk, F* err_max, F* err_final, int i)
+{
+    const int TT = P.TT, Np = P.Np;
+    F x[NS], emax[NS], xn[NS], un[NI], u[NI], K[2 * NS];
+    track_start(P, delta, i, x, emax);
+#pragma unroll
+    for (int c = 0; c < NS; ++c) xtrk0[(size_t)c * Np + i] = x[c];
+    for (int t = 0; t < TT - 1; ++t) {
+        load_x(P, Xnom, t, i, xn);
+#pragma unroll
+        for (int c = 0; c < NI; ++c) un[c] = Unom[at(t, NI, c, Np, i)];
+#pragma unroll
+        for (int c = 0; c < 2 * NS; ++c) K[c] = Ktrk[at(t, 2 * NS, c, Np, i)];
+        track_error(x, xn, emax);
+        track_input(K, x, xn, un, u);
+        store_x(Xtrk, t, Np, i, x);
+#pragma unroll
+        for (int c = 0; c < NI; ++c) Utrk[at(t, NI, c, Np, i)] = u[c];
+        track_advance<Q32>(P.M, x, u);
+    }
+    load_x(P, Xnom, TT - 1, i, xn);
+    store_x(Xtrk, TT - 1, Np, i, x);
+    Utrk[at(TT - 1, NI, 0, Np, i)] = F(0.0);
+    Utrk[at(TT - 1, NI, 1, Np, i)] = F(0.0);
+    track_final(x, xn, emax, err_max, err_final, Np, i);
 }
 
 // ------------------------------------------------------------------------------------------------------

@@ -1331,4 +1331,144 @@ k_candidates_list(ProblemT<F> P, WorkList L, const F* __restrict__ U, const F* _
     }
 }
 
+// =================================================================================================================
+// closed-loop LQR tracking of every instance along its own nominal (track_gains_instance / track_rollout_instance)
+// =================================================================================================================
+// gains sweep: in x*_t, u*_t (walking t = TT-2 .. 0); out K_t.  40 B read + 96 B written per instance and step with float states; the
+// Riccati step is a chain of dependent FP64 operations like k_backward_tma's Gauss-Newton sweep, minus the costate and the references.
+constexpr int TRK_GAIN_STAGES = 3;
+template <typename XT>
+struct TrkGainStage {
+    static constexpr int X_B = NS * TILE * sizeof(XT), U_B = NI * TILE * sizeof(double);
+    static constexpr int X_O = 0, U_O = X_B, BYTES = X_B + U_B;
+};
+
+template <int DG, typename XT>
+__global__ void __launch_bounds__(64) k_track_gains_tma(Problem P, const XT* __restrict__ Xnom, const double* __restrict__ Unom,
+                                                        double* __restrict__ Ktrk, int* __restrict__ n_reg)
+{
+    using St = TrkGainStage<XT>;
+    extern __shared__ __align__(128) unsigned char smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const int tile = blockIdx.x * nw + warp;
+    if (tile * TILE >= P.N) return;  // warp-uniform
+    WarpRing<TRK_GAIN_STAGES, St::BYTES> ring;
+    ring.init(smem, warp, nw, lane);
+    const int TT = P.TT, Np = P.Np, i = tile * TILE + lane, nsteps = TT - 1;
+    const bool live = i < P.N;
+    auto issue = [&](int k) {  // ring step k <-> time t = TT-2-k
+        const int t = TT - 2 - k;
+        unsigned char* st = ring.stage(k);
+        uint64_t* b = ring.barrier(k);
+        mbar_arrive_expect_tx(b, St::BYTES);
+        tma_load(st + St::X_O, Xnom + tile_base(t, NS, Np, tile), St::X_B, b);
+        tma_load(st + St::U_O, Unom + tile_base(t, NI, Np, tile), St::U_B, b);
+    };
+    if (lane == 0)
+        for (int k = 0; k < TRK_GAIN_STAGES && k < nsteps; ++k) issue(k);
+    double Pm[21], p[NS];
+    track_terminal<DG>(P.W, Pm, p);
+    {
+        double* out = Ktrk + tile_base(TT - 1, 2 * NS, Np, tile) + lane;
+#pragma unroll
+        for (int c = 0; c < 2 * NS; ++c) out[c * TILE] = 0.0;
+    }
+    int nreg = 0;
+    for (int k = 0; k < nsteps; ++k) {
+        const int t = TT - 2 - k;
+        ring.wait(k);
+        const unsigned char* st = ring.stage(k);
+        XT xraw[NS];
+        double x[NS], u[NI];
+#pragma unroll
+        for (int c = 0; c < NS; ++c) xraw[c] = reinterpret_cast<const XT*>(st + St::X_O)[c * TILE + lane];
+#pragma unroll
+        for (int c = 0; c < NI; ++c) u[c] = reinterpret_cast<const double*>(st + St::U_O)[c * TILE + lane];
+        stage_release();
+        if (lane == 0 && k + TRK_GAIN_STAGES < nsteps) issue(k + TRK_GAIN_STAGES);
+        if (live) {
+            finish_x(P, t, i, xraw, x);
+            double K[2 * NS];
+            nreg += track_gains_step<DG>(P.M, P.W, x, u, Pm, p, K);
+            double* out = Ktrk + tile_base(t, 2 * NS, Np, tile) + lane;
+#pragma unroll
+            for (int c = 0; c < 2 * NS; ++c) out[c * TILE] = K[c];
+        }
+    }
+    if (live) n_reg[i] = nreg;
+}
+
+// closed-loop rollout: in K_t, x*_t, u*_t per step; out x_t, u_t and the per-instance summaries.  136 B read + 40 B written per instance
+// and step with float states, a few dozen FP64 operations and one sincos per step: bandwidth-bound like k_forward_cand0_tma.
+constexpr int TRK_ROLL_STAGES = 3;
+template <typename XT>
+struct TrkRollStage {
+    static constexpr int K_B = 2 * NS * TILE * sizeof(double), X_B = NS * TILE * sizeof(XT), U_B = NI * TILE * sizeof(double);
+    static constexpr int K_O = 0, X_O = K_B, U_O = K_B + X_B, BYTES = K_B + X_B + U_B;
+};
+
+template <bool Q32, typename XT>
+__global__ void __launch_bounds__(64, 7) k_track_rollout_tma(Problem P, const XT* __restrict__ Xnom, const double* __restrict__ Unom,
+                                                             const double* __restrict__ Ktrk, const double* __restrict__ delta,
+                                                             XT* __restrict__ Xtrk, double* __restrict__ xtrk0, double* __restrict__ Utrk,
+                                                             double* __restrict__ err_max, double* __restrict__ err_final)
+{
+    using St = TrkRollStage<XT>;
+    extern __shared__ __align__(128) unsigned char smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const int tile = blockIdx.x * nw + warp;
+    if (tile * TILE >= P.N) return;  // warp-uniform
+    WarpRing<TRK_ROLL_STAGES, St::BYTES> ring;
+    ring.init(smem, warp, nw, lane);
+    const int TT = P.TT, Np = P.Np, i = tile * TILE + lane, nsteps = TT - 1;
+    const bool live = i < P.N;
+    auto issue = [&](int t) {
+        unsigned char* st = ring.stage(t);
+        uint64_t* b = ring.barrier(t);
+        mbar_arrive_expect_tx(b, St::BYTES);
+        tma_load(st + St::K_O, Ktrk + tile_base(t, 2 * NS, Np, tile), St::K_B, b);
+        tma_load(st + St::X_O, Xnom + tile_base(t, NS, Np, tile), St::X_B, b);
+        tma_load(st + St::U_O, Unom + tile_base(t, NI, Np, tile), St::U_B, b);
+    };
+    if (lane == 0)
+        for (int t = 0; t < TRK_ROLL_STAGES && t < nsteps; ++t) issue(t);
+    double x[NS], emax[NS];
+    if (live) {
+        track_start(P, delta, i, x, emax);
+#pragma unroll
+        for (int c = 0; c < NS; ++c) xtrk0[(size_t)c * Np + i] = x[c];
+    }
+    for (int t = 0; t < nsteps; ++t) {
+        ring.wait(t);
+        const unsigned char* st = ring.stage(t);
+        double K[2 * NS], un[NI];
+        XT xraw[NS];
+#pragma unroll
+        for (int c = 0; c < 2 * NS; ++c) K[c] = reinterpret_cast<const double*>(st + St::K_O)[c * TILE + lane];
+#pragma unroll
+        for (int c = 0; c < NS; ++c) xraw[c] = reinterpret_cast<const XT*>(st + St::X_O)[c * TILE + lane];
+#pragma unroll
+        for (int c = 0; c < NI; ++c) un[c] = reinterpret_cast<const double*>(st + St::U_O)[c * TILE + lane];
+        stage_release();
+        if (lane == 0 && t + TRK_ROLL_STAGES < nsteps) issue(t + TRK_ROLL_STAGES);
+        if (live) {
+            double xn[NS], u[NI];
+            finish_x(P, t, i, xraw, xn);
+            track_error(x, xn, emax);
+            track_input(K, x, xn, un, u);
+            store_x(Xtrk, t, Np, i, x);
+#pragma unroll
+            for (int c = 0; c < NI; ++c) Utrk[at(t, NI, c, Np, i)] = u[c];
+            track_advance<Q32>(P.M, x, u);
+        }
+    }
+    if (!live) return;
+    double xn[NS];
+    load_x(P, Xnom, TT - 1, i, xn);
+    store_x(Xtrk, TT - 1, Np, i, x);
+    Utrk[at(TT - 1, NI, 0, Np, i)] = 0.0;
+    Utrk[at(TT - 1, NI, 1, Np, i)] = 0.0;
+    track_final(x, xn, emax, err_max, err_final, Np, i);
+}
+
 }  // namespace acoc

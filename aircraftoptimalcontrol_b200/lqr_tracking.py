@@ -45,6 +45,34 @@ def lqr_tracking_batch(xx_opt, uu_opt, delta, dyn=None, QQt=None, RRt=None, QQT=
     return xr, ur
 
 
+def lqr_tracking_many(xx_opt, uu_opt, delta, dyn=None, QQt=None, RRt=None, QQT=None, return_gains=False):
+    """One call of the reference's lqr_tracking per nominal: xx_opt (N,6,TT), uu_opt (N,2,TT), delta (N,6) (or (6,), broadcast) ->
+    xx_reg (N,6,TT), uu_reg (N,2,TT) [, KK (N,2,6,TT)].  Each nominal gets its own gains; the kernels are those of
+    BatchedNewton.track (acoc_lqr_tracking_many).  The weights must be symmetric."""
+    dyn = dyn or Dynamics()
+    dQ, dR, dQT = default_weights()
+    Q = L.f64(dQ if QQt is None else QQt, (6, 6), "QQt")
+    R = L.f64(dR if RRt is None else RRt, (2, 2), "RRt")
+    QT = L.f64(dQT if QQT is None else QQT, (6, 6), "QQT")
+    xo, uo = L.f64(xx_opt), L.f64(uu_opt)
+    if xo.ndim != 3 or xo.shape[1] != 6 or xo.shape[2] < 3:
+        raise ValueError("xx_opt must be (N,6,TT) with TT >= 3, got %s" % (xo.shape,))
+    N, _, TT = xo.shape
+    if uo.shape != (N, 2, TT):
+        raise ValueError("uu_opt has shape %s, expected %s" % (uo.shape, (N, 2, TT)))
+    d = np.asarray(delta, dtype=np.float64)
+    if d.shape == (6,):
+        d = np.broadcast_to(d, (N, 6))
+    d = L.f64(d, (N, 6), "delta")
+    xr, ur = np.empty((N, 6, TT)), np.empty((N, 2, TT))
+    K = np.empty((N, 2, 6, TT)) if return_gains else None
+    L.check(L.lib().acoc_lqr_tracking_many(dyn.device, N, TT, L.ptr(dyn.params), int(dyn.state == "f64"), L.ptr(Q), L.ptr(R), L.ptr(QT),
+                                           L.ptr(xo), L.ptr(uo), L.ptr(d), L.ptr(xr), L.ptr(ur), L.ptr(K)))
+    if return_gains:
+        return xr, ur, K
+    return xr, ur
+
+
 def lqr_tracking(xx_opt, uu_opt, tt, dyn=None, QQt=None, RRt=None, QQT=None):
     """(xx_reg (6,TT), uu_reg (2,TT)) for the shipped perturbation 0.1*ones(6) (lqr_tracking.py:259)."""
     TT = np.asarray(tt).shape[0]

@@ -218,6 +218,36 @@ int acoc_get_history(acoc_ctx* ctx, double* JJ, double* descent, double* stepsiz
  * the newest iterate, last descent, number of +0.5*I regularisations. */
 int acoc_get_stats(acoc_ctx* ctx, int* iters, int* status, double* J, double* descent, int* n_reg);
 
+/* ------------------------------------------ closed-loop tracking of every instance ----------------------- */
+/* lqr_tracking(xx_opt, uu_opt, tt) -- lqr_tracking.py:245-283 -- for EVERY instance of the context along its own result: the nominal of
+ * instance i is what acoc_get_result returns now (iterate kk-1 with uu[:,-1] = uu[:,-2]; all zeros for an instance stopped at kk = 0;
+ * the newest iterate while still active; column 0 the exact x0).  Gains of the non-augmented ltv_LQR (:276) linearised along the nominal
+ * (:268-273) with the tracking weights Q, R, QT (P_{TT-1} = QT); closed loop (:279-281) from x*_0 + delta[i] under the context's model and
+ * state quantisation: u_t = u*_t + K_t (x_t - x*_t), u_{TT-1} = 0.
+ * Q, R, QT symmetric (ACOC_ERR_INVALID otherwise, same contract as acoc_set_weights; the pointwise acoc_lqr_tracking accepts any); they
+ * are independent of the context's Newton weights.  delta (N,6) or NULL (= 0).  Per-instance summaries computed on the device (any may
+ * be NULL): err_max (N,6) = max_t |x_t - x*_t|, err_final (N,6) = |x_{TT-1} - x*_{TT-1}| (a NaN anywhere gives NaN), n_reg (N) = steps
+ * whose gain took the +0.5*I branch (optcon.py:745-749).  An instance whose nominal is the zero slot or not finite is computed as the
+ * reference would (its outputs are NaN) and disturbs no other.
+ * The tracking buffers (~176 B per instance and time step with float32-valued states) are allocated on the first call and freed with
+ * the context (ACOC_ERR_NOMEM if they do not fit; the Newton state is untouched).  Tracking writes no iterate, gain, deltau, history or
+ * statistic of the Newton solve: solving or reading back afterwards behaves as if it had not been called.
+ * ACOC_ERR_STATE for ACOC_FP32 contexts and before acoc_set_init / acoc_init_guess. */
+int acoc_track(acoc_ctx* ctx, const double* Q, const double* R, const double* QT, const double* delta, double* err_max, double* err_final,
+               int* n_reg);
+/* trajectories of the last acoc_track: xx_reg (N,6,TT), uu_reg (N,2,TT); either may be NULL */
+int acoc_get_tracked(acoc_ctx* ctx, double* xx_reg, double* uu_reg);
+/* gains of the last acoc_track: K (N,2,6,TT), lqr_tracking's KK per instance (K[:,:,:,TT-1] = 0) */
+int acoc_get_track_gains(acoc_ctx* ctx, double* K);
+/* device time (CUDA events, ms) of the last acoc_track: ms[0] total, ms[1] nominal (k_track_nominal), ms[2] gains sweep, ms[3] rollout */
+int acoc_get_track_timing(acoc_ctx* ctx, double* ms);
+/* lqr_tracking (lqr_tracking.py:245-283) for n independent nominals from host arrays: xx_opt (n,6,TT), uu_opt (n,2,TT), delta (n,6);
+ * outputs xx_reg (n,6,TT), uu_reg (n,2,TT), K (n,2,6,TT) or NULL.  The same kernels as acoc_track (bit-identical results for the same
+ * nominals); states are stored as float32 only when that is lossless.  Q, R, QT symmetric as above. */
+int acoc_lqr_tracking_many(int device, int n, int TT, const double* params, int state_f64, const double* Q, const double* R,
+                           const double* QT, const double* xx_opt, const double* uu_opt, const double* delta, double* xx_reg,
+                           double* uu_reg, double* K);
+
 /* Single pieces of the loop on the context's current iterate, exposed for parity tests and for the
  * reference's own method names:
  *   acoc_eval_cost        optcon.py:417-424   -> J[N]

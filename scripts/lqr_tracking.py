@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Headless drop-in for the reference's lqr_tracking.py __main__ block (:321-342): LQR tracking of a saved optimum
-from perturbed initial states (config 3 with --instances 4096).
+from perturbed initial states (config 3 with --instances 4096).  When --xx holds a batch of optima (N,6,TT) (and --uu (N,2,TT)), every
+optimum is tracked along its own gains from its own perturbation (config3_deltas(N)), one lqr_tracking call per optimum.
     python scripts/lqr_tracking.py --xx Data/xx_star.npy --uu Data/uu_star.npy [--instances 4096] [--out Data]
 """
 import argparse
@@ -10,7 +11,7 @@ import numpy as np
 import _common  # noqa: F401
 from aircraftoptimalcontrol_b200 import refgen
 from aircraftoptimalcontrol_b200.aircraft_simplified import Dynamics
-from aircraftoptimalcontrol_b200.lqr_tracking import lqr_tracking_batch
+from aircraftoptimalcontrol_b200.lqr_tracking import lqr_tracking_batch, lqr_tracking_many
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--xx", default="Data/xx_star.npy")
@@ -22,6 +23,14 @@ args = ap.parse_args()
 
 xx_opt, uu_opt = np.load(args.xx), np.load(args.uu)
 QQt, RRt, QQT = refgen.weights("track")
+if xx_opt.ndim == 3:
+    deltas = refgen.config3_deltas(xx_opt.shape[0])
+    xx_lqr, uu_lqr = lqr_tracking_many(xx_opt, uu_opt, deltas, Dynamics(state=args.state), QQt, RRt, QQT)
+    _common.save("xx_lqr.npy", xx_lqr, args.out)
+    _common.save("uu_lqr.npy", uu_lqr, args.out)
+    err = np.abs(xx_lqr[:, :, -1] - xx_opt[:, :, -1])
+    print("tracked %d optima along their own gains; largest final tracking error per state: %s" % (xx_opt.shape[0], err.max(0)))
+    raise SystemExit(0)
 deltas = refgen.config3_deltas(args.instances)  # instance 0 = the shipped 0.1*ones(6) (lqr_tracking.py:259)
 xx_lqr, uu_lqr = lqr_tracking_batch(xx_opt, uu_opt, deltas, Dynamics(state=args.state), QQt, RRt, QQT)
 _common.save("xx_lqr.npy", xx_lqr[0] if args.instances == 1 else xx_lqr, args.out)
