@@ -38,6 +38,12 @@ class NewtonOptions(C.Structure):
                 ("stepsize_0", C.c_double), ("cc", C.c_double), ("beta", C.c_double), ("term_cond", C.c_double)]
 
 
+class TrackMcOut(C.Structure):
+    """acoc_track_mc_out: output addresses (0 = not wanted)."""
+    _fields_ = [("err_max", C.c_void_p), ("err_final", C.c_void_p), ("worst_max", C.c_void_p), ("mean_final", C.c_void_p),
+                ("n_within", C.c_void_p), ("n_reg", C.c_void_p)]
+
+
 _dp = C.c_void_p  # double* / int* passed as raw addresses
 
 
@@ -80,6 +86,8 @@ def _sig(lib):
         "acoc_get_track_gains": [vp, vp],
         "acoc_get_track_timing": [vp, vp],
         "acoc_lqr_tracking_many": [i, i, i, vp, i] + [vp] * 9,
+        "acoc_track_mc": [vp] * 4 + [i, vp, i, vp, vp],
+        "acoc_lqr_tracking_mc": [i, i, i, i, vp, i] + [vp] * 6 + [i, vp, vp],
         "acoc_eval_cost": [vp, vp],
         "acoc_set_deltau": [vp, vp],
         "acoc_set_scalars": [vp, vp, vp],

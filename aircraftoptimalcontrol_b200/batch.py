@@ -310,6 +310,23 @@ class BatchedNewton:
         L.check(L.lib().acoc_track(self._h, L.ptr(Q), L.ptr(R), L.ptr(QT), L.ptr(d), L.ptr(em), L.ptr(ef), L.ptr(nr)))
         return dict(err_max=em, err_final=ef, n_reg=nr)
 
+    def track_mc(self, delta, QQt=None, RRt=None, QQT=None, tol=None, per_sample=False):
+        """Monte Carlo dispersion of track(): M closed loops per instance, on the device, along the same nominal (what result() returns
+        now) and gains as track().  delta (M,6) (the same perturbations for every instance) or (N,M,6); tol (6,) or None.  Returns
+        dict(worst_max (N,6) = max over samples of max_t |x_t - x*_t| (NaN if any sample is NaN), mean_final (N,6) = mean over samples
+        of |x_{TT-1} - x*_{TT-1}|, n_reg (N)[, n_within (N) = samples whose max error is within tol in every state, with tol]
+        [, err_max, err_final (N,M,6) per sample, with per_sample=True]).  The per-sample summaries are bit-identical to
+        track(delta[:, m]); no trajectory is kept (fly track(delta[:, m]) for the trajectory of sample m).  Afterwards track_gains() and
+        track_timing() report this call and tracked() raises until the next track().  Changes nothing of the solve."""
+        from .lqr_tracking import default_weights, mc_call, mc_deltas
+        dQ, dR, dQT = default_weights()
+        Q = L.f64(dQ if QQt is None else QQt, (6, 6), "QQt")
+        R = L.f64(dR if RRt is None else RRt, (2, 2), "RRt")
+        QT = L.f64(dQT if QQT is None else QQT, (6, 6), "QQT")
+        d, shared, M = mc_deltas(delta, self.N)
+        return mc_call(lambda t, out: L.lib().acoc_track_mc(self._h, L.ptr(Q), L.ptr(R), L.ptr(QT), M, L.ptr(d), int(shared), t, out),
+                       self.N, M, tol, per_sample)
+
     def tracked(self, out=None):
         """(xx_reg (N,6,TT), uu_reg (N,2,TT)) of the last track()."""
         if out is None:
@@ -487,6 +504,14 @@ class PipelinedNewton:
                 raise ValueError("delta has shape %s, expected %s or (6,)" % (d.shape, (self.N, 6)))
         res = [p.track(None if d is None else d[lo:hi], QQt, RRt, QQT) for p, lo, hi in zip(self.parts, self.bounds[:-1], self.bounds[1:])]
         return {k: np.concatenate([r[k] for r in res]) for k in ("err_max", "err_final", "n_reg")}
+
+    def track_mc(self, delta, QQt=None, RRt=None, QQT=None, tol=None, per_sample=False):
+        """BatchedNewton.track_mc on every sub-batch: delta (M,6) as it is, (N,M,6) sliced; returns the concatenated results."""
+        from .lqr_tracking import mc_deltas
+        d, shared, _ = mc_deltas(delta, self.N)
+        res = [p.track_mc(d if shared else d[lo:hi], QQt, RRt, QQT, tol, per_sample)
+               for p, lo, hi in zip(self.parts, self.bounds[:-1], self.bounds[1:])]
+        return {k: np.concatenate([r[k] for r in res]) for k in res[0]}
 
     def tracked(self, out=None):
         """(xx_reg (N,6,TT), uu_reg (N,2,TT)) of the last track()."""

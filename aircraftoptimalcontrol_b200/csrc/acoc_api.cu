@@ -518,6 +518,38 @@ __global__ void __launch_bounds__(64) k_track_rollout(Problem P, const XT* __res
     if (i >= P.N) return;
     track_rollout_instance<Q32>(P, Xnom, Unom, Ktrk, delta, Xtrk, xtrk0, Utrk, err_max, err_final, i);
 }
+// the dispersion rollout with plain global loads (ACOC_NO_TMA): thread = (instance i, sample m), g = m * N + i
+template <bool Q32, typename XT>
+__global__ void __launch_bounds__(64) k_track_mc_rollout(Problem P, const XT* __restrict__ Xnom, const double* __restrict__ Unom,
+                                                         const double* __restrict__ Ktrk, const double* __restrict__ delta, long long dstride,
+                                                         int M, double* __restrict__ em, double* __restrict__ ef)
+{
+    const long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= (long long)P.N * M) return;
+    const int i = (int)(g % P.N), m = (int)(g / P.N);
+    const size_t o = ((size_t)i * M + m) * NS;
+    track_mc_sample<Q32>(P, Xnom, Unom, Ktrk, delta + (size_t)i * (size_t)dstride + (size_t)m * NS, i, em + o, ef + o);
+}
+// per-instance aggregates of the dispersion in sample order; worst / mean [6][Np]
+struct TrackTol {
+    double v[NS];
+    int on;  // 0: no tolerance, n_within is not computed
+};
+__global__ void __launch_bounds__(128) k_track_mc_reduce(const double* __restrict__ em, const double* __restrict__ ef, int N, int Np, int M,
+                                                         TrackTol tol, double* __restrict__ worst, double* __restrict__ mean,
+                                                         int* __restrict__ n_within)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    double tl[NS], w[NS], mf[NS];
+#pragma unroll
+    for (int c = 0; c < NS; ++c) tl[c] = tol.v[c];
+    const size_t o = (size_t)i * M * NS;
+    const int nw = track_mc_reduce(em + o, ef + o, M, tol.on ? tl : (const double*)nullptr, w, mf);
+#pragma unroll
+    for (int c = 0; c < NS; ++c) { worst[(size_t)c * Np + i] = w[c]; mean[(size_t)c * Np + i] = mf[c]; }
+    n_within[i] = nw;
+}
 
 // dx0 and x0_out may alias (each thread reads its dx0 before it writes its x0)
 template <bool Q32, typename F, typename XT>
@@ -918,7 +950,13 @@ struct acoc_ctx {
     void *tk_delta = nullptr, *tk_emax = nullptr, *tk_efin = nullptr;
     int* tk_nreg = nullptr;
     size_t tk_es = 0;           // 0: not allocated
-    bool tk_done = false, tk_xfloat = false;  // Xtrk holds the result of a tracking call; its element type
+    bool tk_done = false, tk_xfloat = false;  // Xtrk holds the result of acoc_track; its element type
+    bool tk_swept = false;      // Ktrk and tk_ms hold the result of acoc_track or acoc_track_mc
+    // dispersion (acoc_track_mc), allocated on the first call and grown with N*M: per-sample summaries em | ef [2][N][M][6], the
+    // deltas as given ((M,6) or (N,M,6)), n_within [Np]; capacities in bytes
+    void *mc_sum = nullptr, *mc_delta = nullptr;
+    int* mc_nw = nullptr;
+    size_t mc_sum_cap = 0, mc_delta_cap = 0;
     cudaEvent_t tk_ev[4] = {};
     double tk_ms[4] = {0, 0, 0, 0};
 };
@@ -2940,9 +2978,11 @@ static void free_track_buffers(acoc_ctx* c)
     dfree(c, &c->tk_u); dfree(c, &c->tk_delta); dfree(c, &c->tk_emax); dfree(c, &c->tk_efin); dfree(c, &c->tk_nreg);
     c->tk_es = 0;
     c->tk_done = false;
+    c->tk_swept = false;
 }
 
-// the tracking buffers for state elements of es bytes (reallocated when the storage type changes); ACOC_ERR_NOMEM leaves none behind
+// the buffers of the nominal, the gains and the per-instance summaries, for state elements of es bytes (reallocated when the storage
+// type changes); ACOC_ERR_NOMEM leaves none behind
 static int ensure_track_buffers(acoc_ctx* c, size_t es)
 {
     if (c->tk_es == es) return 0;
@@ -2952,10 +2992,7 @@ static int ensure_track_buffers(acoc_ctx* c, size_t es)
     int rc = dalloc_bytes(c, &c->tk_xnom, T * NS * Np * es);
     if (!rc) rc = dalloc_bytes(c, &c->tk_unom, T * NI * Np * d);
     if (!rc) rc = dalloc_bytes(c, &c->tk_K, T * 2 * NS * Np * d);
-    if (!rc) rc = dalloc_bytes(c, &c->tk_x, T * NS * Np * es);
-    if (!rc) rc = dalloc_bytes(c, &c->tk_u, T * NI * Np * d);
     if (!rc) rc = dalloc_bytes(c, &c->tk_xnom0, NS * Np * d);
-    if (!rc) rc = dalloc_bytes(c, &c->tk_x0, NS * Np * d);
     if (!rc) rc = dalloc_bytes(c, &c->tk_delta, NS * Np * d);
     if (!rc) rc = dalloc_bytes(c, &c->tk_emax, NS * Np * d);
     if (!rc) rc = dalloc_bytes(c, &c->tk_efin, NS * Np * d);
@@ -2964,6 +3001,38 @@ static int ensure_track_buffers(acoc_ctx* c, size_t es)
         if (!rc && !e && cudaEventCreate(&e) != cudaSuccess) rc = fail(ACOC_ERR_CUDA, "cudaEventCreate failed");
     if (rc) { free_track_buffers(c); return rc; }
     c->tk_es = es;
+    return 0;
+}
+
+// the tracked trajectories Xtrk / Utrk and their exact row 0, which only acoc_track and acoc_lqr_tracking_many write (after
+// ensure_track_buffers); ACOC_ERR_NOMEM leaves no tracking buffer behind
+static int ensure_tracked_buffers(acoc_ctx* c)
+{
+    if (c->tk_x) return 0;
+    const size_t T = c->TT, Np = c->Np, d = sizeof(double);
+    int rc = dalloc_bytes(c, &c->tk_x, T * NS * Np * c->tk_es);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_u, T * NI * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->tk_x0, NS * Np * d);
+    if (rc) free_track_buffers(c);
+    return rc;
+}
+
+// the dispersion buffers for n * m samples (96 B each) and `delta_bytes` of deltas, grown when too small.  The new buffers are allocated
+// before the old ones are released, so ACOC_ERR_NOMEM leaves the context as it was.
+static int ensure_mc_buffers(acoc_ctx* c, size_t samples, size_t delta_bytes)
+{
+    const size_t sum_bytes = samples * 2 * NS * sizeof(double);
+    void *ns = nullptr, *nd = nullptr;
+    int* nw = nullptr;
+    int rc = 0;
+    if (c->mc_sum_cap < sum_bytes) rc = dalloc_bytes(c, &ns, sum_bytes);
+    if (!rc && c->mc_delta_cap < delta_bytes) rc = dalloc_bytes(c, &nd, delta_bytes);
+    if (!rc && !c->mc_nw) rc = dalloc(c, &nw, c->Np);
+    if (rc) { dfree(c, &ns); dfree(c, &nd); dfree(c, &nw); return rc; }
+    if (ns || nd) CK(cudaStreamSynchronize(c->stream));
+    if (ns) { dfree(c, &c->mc_sum); c->mc_sum = ns; c->mc_sum_cap = sum_bytes; }
+    if (nd) { dfree(c, &c->mc_delta); c->mc_delta = nd; c->mc_delta_cap = delta_bytes; }
+    if (nw) c->mc_nw = nw;
     return 0;
 }
 
@@ -2987,28 +3056,48 @@ static int upload_delta(acoc_ctx* c, const double* delta)
     return 0;
 }
 
-// gains sweep + closed-loop rollout over the nominal in tk_xnom / tk_unom / tk_xnom0 (events tk_ev[1..3])
-template <typename XT>
-static int launch_track_sweeps(acoc_ctx* c, const Weights& W)
+// the problem the tracking sweeps see: tracking weights, x0 = the exact row 0 of the nominal (finish_x)
+static Problem track_problem(acoc_ctx* c, const Weights& W)
 {
     Problem P = prob<double>(c);
     P.W = W;
-    P.x0 = (const double*)c->tk_xnom0;  // exact row 0 of the nominal (finish_x)
+    P.x0 = (const double*)c->tk_xnom0;
+    return P;
+}
+
+// gains sweep over the nominal in tk_xnom / tk_unom / tk_xnom0 (events tk_ev[1..2])
+template <typename XT>
+static int launch_track_gains(acoc_ctx* c, const Problem& P)
+{
     const XT* Xn = (const XT*)c->tk_xnom;
-    const double *Un = (const double*)c->tk_unom, *dl = (const double*)c->tk_delta;
-    double *K = (double*)c->tk_K, *x0 = (double*)c->tk_x0, *U = (double*)c->tk_u, *em = (double*)c->tk_emax, *ef = (double*)c->tk_efin;
-    XT* X = (XT*)c->tk_x;
+    const double* Un = (const double*)c->tk_unom;
+    double* K = (double*)c->tk_K;
     cudaStream_t st = c->stream;
     const int g = (c->N + 63) / 64;  // 64 threads = two tiles per CTA
     CK(cudaEventRecord(c->tk_ev[1], st));
     if (use_tma(c)) {
         const size_t sm = WarpRing<TRK_GAIN_STAGES, TrkGainStage<XT>::BYTES>::smem_bytes(2);
-        if (W.diag) { TRY(prefer_smem(k_track_gains_tma<1, XT>)); k_track_gains_tma<1, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, c->tk_nreg); }
+        if (P.W.diag) { TRY(prefer_smem(k_track_gains_tma<1, XT>)); k_track_gains_tma<1, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, c->tk_nreg); }
         else { TRY(prefer_smem(k_track_gains_tma<0, XT>)); k_track_gains_tma<0, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, c->tk_nreg); }
-    } else if (W.diag) k_track_gains<1, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, c->tk_nreg);
+    } else if (P.W.diag) k_track_gains<1, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, c->tk_nreg);
     else k_track_gains<0, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, c->tk_nreg);
     CK(cudaGetLastError());
     CK(cudaEventRecord(c->tk_ev[2], st));
+    return 0;
+}
+
+// gains sweep + closed-loop rollout over the nominal (events tk_ev[1..3])
+template <typename XT>
+static int launch_track_sweeps(acoc_ctx* c, const Weights& W)
+{
+    const Problem P = track_problem(c, W);
+    TRY(launch_track_gains<XT>(c, P));
+    const XT* Xn = (const XT*)c->tk_xnom;
+    const double *Un = (const double*)c->tk_unom, *dl = (const double*)c->tk_delta;
+    double *K = (double*)c->tk_K, *x0 = (double*)c->tk_x0, *U = (double*)c->tk_u, *em = (double*)c->tk_emax, *ef = (double*)c->tk_efin;
+    XT* X = (XT*)c->tk_x;
+    cudaStream_t st = c->stream;
+    const int g = (c->N + 63) / 64;
     if (use_tma(c)) {
         const size_t sm = WarpRing<TRK_ROLL_STAGES, TrkRollStage<XT>::BYTES>::smem_bytes(2);
         if (c->P.q32) {
@@ -3024,8 +3113,48 @@ static int launch_track_sweeps(acoc_ctx* c, const Weights& W)
     return 0;
 }
 
-// after the sweeps: wait, read the event times, mark the outputs valid
-static int track_finish(acoc_ctx* c, bool xfloat)
+// gains sweep + dispersion rollout of m samples per instance + per-instance reduction (events tk_ev[1..3]); deltas in mc_delta with
+// instance stride dstride (doubles)
+template <typename XT>
+static int launch_track_mc(acoc_ctx* c, const Weights& W, int m, long long dstride, const double* tol)
+{
+    const Problem P = track_problem(c, W);
+    TRY(launch_track_gains<XT>(c, P));
+    const XT* Xn = (const XT*)c->tk_xnom;
+    const double *Un = (const double*)c->tk_unom, *K = (const double*)c->tk_K, *dl = (const double*)c->mc_delta;
+    double* em = (double*)c->mc_sum;
+    double* ef = em + (size_t)c->N * m * NS;
+    cudaStream_t st = c->stream;
+    if (use_tma(c)) {
+        const long long lanes = std::min(c->N, TILE);  // live lanes of the fullest tile
+        const int cpt = (int)((lanes * m + TRK_MC_WARPS * TILE - 1) / (TRK_MC_WARPS * TILE));
+        const long long grid = (long long)n_tiles(c) * cpt;
+        REQUIRE(grid <= 0x7fffffffLL, "acoc_track_mc: %d instances x %d samples is too many for one launch", c->N, m);
+        const size_t sm = track_mc_smem<XT>();
+        if (c->P.q32) {
+            TRY(prefer_smem(k_track_mc_rollout_tma<true, XT>));
+            k_track_mc_rollout_tma<true, XT><<<(unsigned)grid, TRK_MC_THREADS, sm, st>>>(P, Xn, Un, K, dl, dstride, m, cpt, em, ef);
+        } else {
+            TRY(prefer_smem(k_track_mc_rollout_tma<false, XT>));
+            k_track_mc_rollout_tma<false, XT><<<(unsigned)grid, TRK_MC_THREADS, sm, st>>>(P, Xn, Un, K, dl, dstride, m, cpt, em, ef);
+        }
+    } else {
+        const long long grid = ((long long)c->N * m + 63) / 64;
+        REQUIRE(grid <= 0x7fffffffLL, "acoc_track_mc: %d instances x %d samples is too many for one launch", c->N, m);
+        LAUNCH_Q32(c->P.q32, k_track_mc_rollout, (XT), (unsigned)grid, 64, st, P, Xn, Un, K, dl, dstride, m, em, ef);
+    }
+    CK(cudaGetLastError());
+    TrackTol tl{};
+    tl.on = tol != nullptr;
+    for (int k = 0; k < NS && tol; ++k) tl.v[k] = tol[k];
+    k_track_mc_reduce<<<(c->N + 127) / 128, 128, 0, st>>>(em, ef, c->N, c->Np, m, tl, (double*)c->tk_emax, (double*)c->tk_efin, c->mc_nw);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(c->tk_ev[3], st));
+    return 0;
+}
+
+// after the sweeps: wait, read the event times, mark the gains valid and the tracked trajectories valid (acoc_track) or not
+static int track_finish(acoc_ctx* c, bool xfloat, bool trajectories)
 {
     CK(cudaStreamSynchronize(c->stream));
     float a = 0, b = 0, r = 0;
@@ -3033,7 +3162,8 @@ static int track_finish(acoc_ctx* c, bool xfloat)
     CK(cudaEventElapsedTime(&b, c->tk_ev[1], c->tk_ev[2]));
     CK(cudaEventElapsedTime(&r, c->tk_ev[2], c->tk_ev[3]));
     c->tk_ms[0] = (double)a + b + r; c->tk_ms[1] = a; c->tk_ms[2] = b; c->tk_ms[3] = r;
-    c->tk_done = true;
+    c->tk_swept = true;
+    c->tk_done = trajectories;
     c->tk_xfloat = xfloat;
     return 0;
 }
@@ -3061,18 +3191,9 @@ static int download_rows(acoc_ctx* c, const void* dev, T* host, int rows)
     return 0;
 }
 
-int acoc_track(acoc_ctx* c, const double* Q, const double* R, const double* QT, const double* delta, double* err_max, double* err_final,
-               int* n_reg)
+// the nominal of every lane = its current result (k_result_slot_default + k_track_nominal; event tk_ev[0])
+static int copy_track_nominal(acoc_ctx* c, bool xf)
 {
-    REQUIRE(c, "ctx is NULL");
-    if (c->fp32) return fail(ACOC_ERR_STATE, "acoc_track: not available in the FP32 mode (ACOC_FP32)");
-    if (!c->have_init) return fail(ACOC_ERR_STATE, "acoc_track: no iterate to track yet: call acoc_set_init or acoc_init_guess first");
-    Weights W;
-    TRY(track_weights(Q, R, QT, &W));
-    TRY(use_device(c->device));
-    const bool xf = c->x_float;
-    TRY(ensure_track_buffers(c, xf ? sizeof(float) : sizeof(double)));
-    TRY(upload_delta(c, delta));
     CK(cudaEventRecord(c->tk_ev[0], c->stream));
     k_result_slot_default<<<(c->N + 255) / 256, 256, 0, c->stream>>>(c->S.status, c->slot_tmp, c->S.result_slot, c->kk % 3, c->N);
     const int tchunk = 8;
@@ -3087,12 +3208,82 @@ int acoc_track(acoc_ctx* c, const double* Q, const double* R, const double* QT, 
                                                              (const double*)c->x0, (double*)c->tk_xnom, (double*)c->tk_unom, (double*)c->tk_xnom0,
                                                              c->N, c->Np, c->TT, tchunk);
     CK(cudaGetLastError());
+    return 0;
+}
+
+static int track_ctx_check(acoc_ctx* c, const char* fn)
+{
+    REQUIRE(c, "ctx is NULL");
+    if (c->fp32) return fail(ACOC_ERR_STATE, "%s: not available in the FP32 mode (ACOC_FP32)", fn);
+    if (!c->have_init) return fail(ACOC_ERR_STATE, "%s: no iterate to track yet: call acoc_set_init or acoc_init_guess first", fn);
+    return 0;
+}
+
+int acoc_track(acoc_ctx* c, const double* Q, const double* R, const double* QT, const double* delta, double* err_max, double* err_final,
+               int* n_reg)
+{
+    TRY(track_ctx_check(c, "acoc_track"));
+    Weights W;
+    TRY(track_weights(Q, R, QT, &W));
+    TRY(use_device(c->device));
+    const bool xf = c->x_float;
+    TRY(ensure_track_buffers(c, xf ? sizeof(float) : sizeof(double)));
+    TRY(ensure_tracked_buffers(c));
+    TRY(upload_delta(c, delta));
+    TRY(copy_track_nominal(c, xf));
     TRY(xf ? launch_track_sweeps<float>(c, W) : launch_track_sweeps<double>(c, W));
-    TRY(track_finish(c, xf));
+    TRY(track_finish(c, xf, true));
     TRY(download_rows(c, c->tk_emax, err_max, NS));
     TRY(download_rows(c, c->tk_efin, err_final, NS));
     TRY(download_rows(c, c->tk_nreg, n_reg, 1));
     return 0;
+}
+
+// the common part of acoc_track_mc and acoc_lqr_tracking_mc once the nominal is in place: deltas (one copy, as given), the sweeps, the
+// outputs
+static int track_mc_run(acoc_ctx* c, bool xf, const Weights& W, int m, const double* delta, int delta_shared, const double* tol,
+                        acoc_track_mc_out* out)
+{
+    const size_t per = (size_t)m * NS;
+    CK(cudaMemcpyAsync(c->mc_delta, delta, (delta_shared ? 1 : (size_t)c->N) * per * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    const long long dstride = delta_shared ? 0 : (long long)per;
+    TRY(xf ? launch_track_mc<float>(c, W, m, dstride, tol) : launch_track_mc<double>(c, W, m, dstride, tol));
+    TRY(track_finish(c, xf, false));
+    if (!out) return 0;
+    const size_t bytes = (size_t)c->N * per * sizeof(double);
+    if (out->err_max) CK(cudaMemcpyAsync(out->err_max, c->mc_sum, bytes, cudaMemcpyDeviceToHost, c->stream));
+    if (out->err_final) CK(cudaMemcpyAsync(out->err_final, (const char*)c->mc_sum + bytes, bytes, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    TRY(download_rows(c, c->tk_emax, out->worst_max, NS));
+    TRY(download_rows(c, c->tk_efin, out->mean_final, NS));
+    if (tol) TRY(download_rows(c, c->mc_nw, out->n_within, 1));
+    TRY(download_rows(c, c->tk_nreg, out->n_reg, 1));
+    return 0;
+}
+
+static int track_mc_args(int m, const double* delta, const double* tol, acoc_track_mc_out* out, const char* fn)
+{
+    REQUIRE(m >= 1, "%s: m = %d, need at least one sample", fn, m);
+    REQUIRE(delta, "%s: delta is NULL", fn);
+    REQUIRE(!(out && out->n_within && !tol), "%s: n_within needs a tolerance", fn);
+    return 0;
+}
+
+int acoc_track_mc(acoc_ctx* c, const double* Q, const double* R, const double* QT, int m, const double* delta, int delta_shared,
+                  const double* tol, acoc_track_mc_out* out)
+{
+    TRY(track_ctx_check(c, "acoc_track_mc"));
+    TRY(track_mc_args(m, delta, tol, out, "acoc_track_mc"));
+    Weights W;
+    TRY(track_weights(Q, R, QT, &W));
+    TRY(use_device(c->device));
+    const size_t per = (size_t)m * NS * sizeof(double);
+    TRY(ensure_mc_buffers(c, (size_t)c->N * m, delta_shared ? per : (size_t)c->N * per));
+    const bool xf = c->x_float;
+    TRY(ensure_track_buffers(c, xf ? sizeof(float) : sizeof(double)));
+    c->tk_done = false;  // the nominal and gains buffers are about to change
+    TRY(copy_track_nominal(c, xf));
+    return track_mc_run(c, xf, W, m, delta, delta_shared, tol, out);
 }
 
 int acoc_get_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg)
@@ -3106,7 +3297,7 @@ int acoc_get_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg)
 int acoc_get_track_gains(acoc_ctx* c, double* K)
 {
     REQUIRE(c && K, "NULL argument");
-    if (!c->tk_done) return fail(ACOC_ERR_STATE, "acoc_get_track_gains: call acoc_track first");
+    if (!c->tk_swept) return fail(ACOC_ERR_STATE, "acoc_get_track_gains: call acoc_track or acoc_track_mc first");
     TRY(use_device(c->device));
     // Ktrk as a trajectory with 12 components downloads to (N,12,TT) = (N,2,6,TT)
     return download_soa_t<double>(c, c->tk_K, nullptr, nullptr, nullptr, nullptr, K, c->N, 2 * NS, c->Np, 0);
@@ -3115,30 +3306,28 @@ int acoc_get_track_gains(acoc_ctx* c, double* K)
 int acoc_get_track_timing(acoc_ctx* c, double* ms)
 {
     REQUIRE(c && ms, "NULL argument");
-    if (!c->tk_done) return fail(ACOC_ERR_STATE, "acoc_get_track_timing: call acoc_track first");
+    if (!c->tk_swept) return fail(ACOC_ERR_STATE, "acoc_get_track_timing: call acoc_track or acoc_track_mc first");
     for (int k = 0; k < 4; ++k) ms[k] = c->tk_ms[k];
     return 0;
 }
 
-int acoc_lqr_tracking_many(int device, int n, int TT, const double* params, int state_f64, const double* Q, const double* R, const double* QT,
-                           const double* xx_opt, const double* uu_opt, const double* delta, double* xx_reg, double* uu_reg, double* K)
+// One context without iterate slots per (device, n, TT, quantisation) for the host-array tracking calls, kept between calls: no
+// allocation once it exists.  The caller holds g_host_track_mu while it uses the context.
+static std::mutex g_host_track_mu;
+static acoc_ctx* g_host_track_ctx = nullptr;
+
+// that context with the nominals xx_opt (n,6,TT) / uu_opt (n,2,TT) in Xnom / Unom: float storage when every state at t >= 1 is a
+// float32 value (as acoc_set_init decides), the exact row 0 always
+static int host_track_ctx(int device, int n, int TT, const double* params, int state_f64, const double* xx_opt, const double* uu_opt,
+                          acoc_ctx** out, bool* xf_out)
 {
-    REQUIRE(n > 0 && TT >= 3 && params && xx_opt && uu_opt && delta && xx_reg && uu_reg, "acoc_lqr_tracking_many: bad argument");
-    REQUIRE(params[3] != 0.0 && params[7] != 0.0, "acoc_lqr_tracking_many: mass and inertia must be non-zero");
-    Weights W;
-    TRY(track_weights(Q, R, QT, &W));
-    // one context without iterate slots per (device, n, TT, quantisation), kept between calls: no allocation once it exists
-    static std::mutex mu;
-    static acoc_ctx* cached = nullptr;
-    std::lock_guard<std::mutex> lock(mu);
     const unsigned flags = (state_f64 ? ACOC_STATE_F64 : 0) | ACOC_REFS_SHARED | ACOC_CTX_LITE | ACOC_CTX_NO_SLOTS;
+    acoc_ctx*& cached = g_host_track_ctx;
     if (cached && (cached->device != device || cached->N != n || cached->TT != TT || cached->flags != flags)) { acoc_ctx_destroy(cached); cached = nullptr; }
     if (!cached) TRY(acoc_ctx_create(device, n, TT, flags, &cached));
     acoc_ctx* c = cached;
     TRY(use_device(device));
     TRY(acoc_set_model(c, params));
-    // the nominals go straight into Xnom / Unom: float storage when every state at t >= 1 is a float32 value (as acoc_set_init decides),
-    // the exact row 0 always
     bool xf = false;
     if (c->P.q32) {
         TRY(ensure_track_buffers(c, sizeof(float)));
@@ -3154,13 +3343,49 @@ int acoc_lqr_tracking_many(int device, int n, int TT, const double* params, int 
         TRY((upload_soa_t<double, double>(c, xx_opt, c->tk_xnom, n, NS, c->Np, (double*)c->tk_xnom0, (int*)nullptr)));
     }
     TRY((upload_soa_t<double, double>(c, uu_opt, c->tk_unom, n, NI, c->Np, (double*)nullptr, (int*)nullptr)));
+    *out = c;
+    *xf_out = xf;
+    return 0;
+}
+
+int acoc_lqr_tracking_many(int device, int n, int TT, const double* params, int state_f64, const double* Q, const double* R, const double* QT,
+                           const double* xx_opt, const double* uu_opt, const double* delta, double* xx_reg, double* uu_reg, double* K)
+{
+    REQUIRE(n > 0 && TT >= 3 && params && xx_opt && uu_opt && delta && xx_reg && uu_reg, "acoc_lqr_tracking_many: bad argument");
+    REQUIRE(params[3] != 0.0 && params[7] != 0.0, "acoc_lqr_tracking_many: mass and inertia must be non-zero");
+    Weights W;
+    TRY(track_weights(Q, R, QT, &W));
+    std::lock_guard<std::mutex> lock(g_host_track_mu);
+    acoc_ctx* c = nullptr;
+    bool xf = false;
+    TRY(host_track_ctx(device, n, TT, params, state_f64, xx_opt, uu_opt, &c, &xf));
+    TRY(ensure_tracked_buffers(c));
     TRY(upload_delta(c, delta));
     CK(cudaEventRecord(c->tk_ev[0], c->stream));
     TRY(xf ? launch_track_sweeps<float>(c, W) : launch_track_sweeps<double>(c, W));
-    TRY(track_finish(c, xf));
+    TRY(track_finish(c, xf, true));
     TRY(download_tracked(c, xx_reg, uu_reg));
     if (K) TRY(download_soa_t<double>(c, c->tk_K, nullptr, nullptr, nullptr, nullptr, K, n, 2 * NS, c->Np, 0));
     return 0;
+}
+
+int acoc_lqr_tracking_mc(int device, int n, int m, int TT, const double* params, int state_f64, const double* Q, const double* R,
+                         const double* QT, const double* xx_opt, const double* uu_opt, const double* delta, int delta_shared, const double* tol,
+                         acoc_track_mc_out* out)
+{
+    REQUIRE(n > 0 && TT >= 3 && params && xx_opt && uu_opt, "acoc_lqr_tracking_mc: bad argument");
+    REQUIRE(params[3] != 0.0 && params[7] != 0.0, "acoc_lqr_tracking_mc: mass and inertia must be non-zero");
+    TRY(track_mc_args(m, delta, tol, out, "acoc_lqr_tracking_mc"));
+    Weights W;
+    TRY(track_weights(Q, R, QT, &W));
+    std::lock_guard<std::mutex> lock(g_host_track_mu);
+    acoc_ctx* c = nullptr;
+    bool xf = false;
+    TRY(host_track_ctx(device, n, TT, params, state_f64, xx_opt, uu_opt, &c, &xf));
+    const size_t per = (size_t)m * NS * sizeof(double);
+    TRY(ensure_mc_buffers(c, (size_t)n * m, delta_shared ? per : (size_t)n * per));
+    CK(cudaEventRecord(c->tk_ev[0], c->stream));
+    return track_mc_run(c, xf, W, m, delta, delta_shared, tol, out);
 }
 
 // ======================================================================================================

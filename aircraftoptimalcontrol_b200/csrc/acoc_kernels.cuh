@@ -20,6 +20,8 @@
 //   track_instance        lqr_tracking.py:279-281
 //   track_gains_instance, lqr_tracking.py:245-283 along each instance's own nominal (gains, closed loop, summaries)
 //   track_rollout_instance
+//   track_mc_sample,      the same closed loop from M perturbed starts per instance (summaries only) and their fixed-order
+//   track_mc_reduce       per-instance aggregates
 //   init_guess_instance   aircraft_simplified.py:142-147
 //
 // Types: F is the arithmetic type and the storage type of U, DU, KSG, the references and x0 (double = the parity path,
@@ -934,20 +936,38 @@ ACOC_HD void track_advance(const ModelT<F>& M, F* x, const F* u)
 #pragma unroll
     for (int c = 0; c < NS; ++c) x[c] = xn[c];
 }
+// x_0 = x*_0 + d6 (d6 = this start's perturbation, 6 values): the one start expression of acoc_track and acoc_track_mc
+template <typename F>
+ACOC_HD void track_start_from(const ProblemT<F>& P, int i, const F* d6, F* x, F* emax)
+{
+#pragma unroll
+    for (int c = 0; c < NS; ++c) { x[c] = P.x0[(size_t)c * P.Np + i] + d6[c]; emax[c] = F(0.0); }
+}
 template <typename F>
 ACOC_HD void track_start(const ProblemT<F>& P, const F* delta, int i, F* x, F* emax)
 {
+    F d6[NS];
 #pragma unroll
-    for (int c = 0; c < NS; ++c) { x[c] = P.x0[(size_t)c * P.Np + i] + delta[(size_t)c * P.Np + i]; emax[c] = F(0.0); }
+    for (int c = 0; c < NS; ++c) d6[c] = delta[(size_t)c * P.Np + i];
+    track_start_from(P, i, d6, x, emax);
+}
+// summaries at t = TT-1: emax takes the last error, efin = |x_{TT-1} - x*_{TT-1}|
+template <typename F>
+ACOC_HD void track_final_err(const F* x, const F* xnom, F* emax, F* efin)
+{
+    track_error(x, xnom, emax);
+#pragma unroll
+    for (int c = 0; c < NS; ++c) efin[c] = F(fabs(x[c] - xnom[c]));
 }
 template <typename F>
 ACOC_HD void track_final(const F* x, const F* xnom, F* emax, F* err_max, F* err_final, int Np, int i)
 {
-    track_error(x, xnom, emax);
+    F efin[NS];
+    track_final_err(x, xnom, emax, efin);
 #pragma unroll
     for (int c = 0; c < NS; ++c) {
         err_max[(size_t)c * Np + i] = emax[c];
-        err_final[(size_t)c * Np + i] = F(fabs(x[c] - xnom[c]));
+        err_final[(size_t)c * Np + i] = efin[c];
     }
 }
 
@@ -978,6 +998,60 @@ ACOC_HD void track_rollout_instance(const ProblemT<F>& P, const XT* Xnom, const 
     Utrk[at(TT - 1, NI, 0, Np, i)] = F(0.0);
     Utrk[at(TT - 1, NI, 1, Np, i)] = F(0.0);
     track_final(x, xn, emax, err_max, err_final, Np, i);
+}
+
+// ------------------------------------------------------------------------------------------------------
+// Monte Carlo dispersion of the closed loop (acoc_track_mc, acoc_lqr_tracking_mc): M perturbed starts per instance, same nominal and
+// gains.  One sample is acoc_track's closed loop without the trajectory stores: its summaries are bit-identical to acoc_track's with
+// delta[i] = d6.  Per-sample summaries are stored sample-major, em / ef [N][M][6].
+// ------------------------------------------------------------------------------------------------------
+template <bool Q32, typename F, typename XT>
+ACOC_HD void track_mc_sample(const ProblemT<F>& P, const XT* Xnom, const F* Unom, const F* Ktrk, const F* d6, int i, F* em, F* ef)
+{
+    const int TT = P.TT, Np = P.Np;
+    F x[NS], emax[NS], xn[NS], un[NI], u[NI], K[2 * NS];
+    track_start_from(P, i, d6, x, emax);
+    for (int t = 0; t < TT - 1; ++t) {
+        load_x(P, Xnom, t, i, xn);
+#pragma unroll
+        for (int c = 0; c < NI; ++c) un[c] = Unom[at(t, NI, c, Np, i)];
+#pragma unroll
+        for (int c = 0; c < 2 * NS; ++c) K[c] = Ktrk[at(t, 2 * NS, c, Np, i)];
+        track_error(x, xn, emax);
+        track_input(K, x, xn, un, u);
+        track_advance<Q32>(P.M, x, u);
+    }
+    load_x(P, Xnom, TT - 1, i, xn);
+    track_final_err(x, xn, emax, ef);
+#pragma unroll
+    for (int c = 0; c < NS; ++c) em[c] = emax[c];
+}
+
+// Fixed-order aggregates of one instance over its M samples (em, ef: [M][6] of that instance): worst[c] = max_nan over m in sample
+// order, mean[c] = (((ef_0 + ef_1) + ef_2) + ...) / M, and (tol != nullptr) the number of samples with em[m][c] <= tol[c] for every c
+// (a NaN is never within).
+template <typename F>
+ACOC_HD int track_mc_reduce(const F* em, const F* ef, int M, const F* tol, F* worst, F* mean)
+{
+    int within = 0;
+#pragma unroll
+    for (int c = 0; c < NS; ++c) { worst[c] = em[c]; mean[c] = ef[c]; }
+    for (int m = 0; m < M; ++m) {
+        const F* e = em + (size_t)m * NS;
+        if (m > 0) {
+#pragma unroll
+            for (int c = 0; c < NS; ++c) { worst[c] = max_nan(worst[c], e[c]); mean[c] += ef[(size_t)m * NS + c]; }
+        }
+        if (tol) {
+            bool in = true;
+#pragma unroll
+            for (int c = 0; c < NS; ++c) in = in && e[c] <= tol[c];
+            within += in ? 1 : 0;
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < NS; ++c) mean[c] /= F(M);
+    return within;
 }
 
 // ------------------------------------------------------------------------------------------------------

@@ -1471,4 +1471,106 @@ __global__ void __launch_bounds__(64, 7) k_track_rollout_tma(Problem P, const XT
     track_final(x, xn, emax, err_max, err_final, Np, i);
 }
 
+// =================================================================================================================
+// Monte Carlo dispersion of the closed loop (track_mc_sample): M perturbed starts per instance along the same nominal and gains.
+// The gains and the nominal of an instance are the same for all of its samples, so a CTA flies many (instance, sample) pairs of ONE
+// tile through one CTA-shared ring: a producer warp issues the bulk copies of the tile's K / x* / u* block of step t (the TrkRollStage
+// of k_track_rollout_tma, 4,352 B with float states) and TRK_MC_WARPS consumer warps read it, full / empty mbarriers per stage as in
+// k_candidates_list.  The 136 B an instance-step needs are read once per CTA and step instead of once per sample, which turns the
+// bandwidth-bound sweep into an FP64-bound one.
+// Pairs of a tile: p -> (lane column j = p mod L, sample m = p div L), L = live lanes of the tile; CTA r of the tile covers pairs
+// [r, r+1) * TRK_MC_WARPS * 32, consumer warp w the 32 of them at offset 32 w.  With N >= 32 that is lane = instance, warp = sample;
+// with N = 1 every lane flies a sample of the one instance and reads the same shared-memory column (a broadcast).  blockIdx.x =
+// tile * ctas_per_tile + r: the CTAs of one tile are adjacent and their copies of its blocks mostly hit L2.
+// Same per-step functions as k_track_rollout_tma (finish_x, track_error, track_input, track_advance, track_final_err): bit-identical
+// summaries.
+// =================================================================================================================
+#ifndef ACOC_TRK_MC_WARPS
+#define ACOC_TRK_MC_WARPS 8
+#endif
+#ifndef ACOC_TRK_MC_MINB
+#define ACOC_TRK_MC_MINB 2
+#endif
+constexpr int TRK_MC_WARPS = ACOC_TRK_MC_WARPS, TRK_MC_STAGES = 4;
+constexpr int TRK_MC_THREADS = TILE * (TRK_MC_WARPS + 1);
+template <typename XT>
+constexpr size_t track_mc_smem() { return (size_t)TRK_MC_STAGES * TrkRollStage<XT>::BYTES + 2 * TRK_MC_STAGES * sizeof(uint64_t); }
+
+// delta: per-sample perturbations, d6 of (instance i, sample m) at delta + i * dstride + m * 6 (dstride = 0: shared (M,6), M * 6: (N,M,6))
+template <bool Q32, typename XT>
+__global__ void __launch_bounds__(TRK_MC_THREADS, ACOC_TRK_MC_MINB)
+k_track_mc_rollout_tma(Problem P, const XT* __restrict__ Xnom, const double* __restrict__ Unom, const double* __restrict__ Ktrk,
+                       const double* __restrict__ delta, long long dstride, int M, int ctas_per_tile, double* __restrict__ em,
+                       double* __restrict__ ef)
+{
+    using St = TrkRollStage<XT>;
+    extern __shared__ __align__(128) unsigned char smem[];
+    uint64_t* const full = reinterpret_cast<uint64_t*>(smem + (size_t)TRK_MC_STAGES * St::BYTES);
+    uint64_t* const empty = full + TRK_MC_STAGES;
+    const int tile = blockIdx.x / ctas_per_tile, r = blockIdx.x % ctas_per_tile;
+    const int L = min(TILE, P.N - tile * TILE), lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const long long pairs = (long long)L * M, p0 = (long long)r * TRK_MC_WARPS * TILE;
+    if (p0 >= pairs) return;  // CTA-uniform: a partial tile needs fewer CTAs
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < TRK_MC_STAGES; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, TRK_MC_WARPS); }
+        mbar_fence_init();
+    }
+    __syncthreads();
+    const int TT = P.TT, Np = P.Np, nsteps = TT - 1;
+    if (warp == TRK_MC_WARPS) {  // ---- producer warp
+        if (lane == 0)
+            for (int t = 0; t < nsteps; ++t) {
+                const int s = t % TRK_MC_STAGES;
+                if (t >= TRK_MC_STAGES) mbar_wait(empty + s, (uint32_t)((t / TRK_MC_STAGES - 1) & 1));
+                unsigned char* st = smem + (size_t)s * St::BYTES;
+                mbar_arrive_expect_tx(full + s, St::BYTES);
+                tma_load(st + St::K_O, Ktrk + tile_base(t, 2 * NS, Np, tile), St::K_B, full + s);
+                tma_load(st + St::X_O, Xnom + tile_base(t, NS, Np, tile), St::X_B, full + s);
+                tma_load(st + St::U_O, Unom + tile_base(t, NI, Np, tile), St::U_B, full + s);
+            }
+        return;  // the consumers wait for every copy before they exit
+    }
+    // ---- consumer warps
+    const long long p = p0 + (long long)warp * TILE + lane;
+    const bool work = p < pairs;
+    const int j = work ? (int)(p % L) : 0, m = work ? (int)(p / L) : 0, i = tile * TILE + j;
+    double x[NS], emax[NS];
+    if (work) {
+        double d6[NS];
+        const double* d = delta + (size_t)i * (size_t)dstride + (size_t)m * NS;
+#pragma unroll
+        for (int c = 0; c < NS; ++c) d6[c] = d[c];
+        track_start_from(P, i, d6, x, emax);
+    }
+    for (int t = 0; t < nsteps; ++t) {
+        const int s = t % TRK_MC_STAGES;
+        mbar_wait(full + s, (uint32_t)((t / TRK_MC_STAGES) & 1));
+        const unsigned char* st = smem + (size_t)s * St::BYTES;
+        double K[2 * NS], un[NI];
+        XT xraw[NS];
+#pragma unroll
+        for (int c = 0; c < 2 * NS; ++c) K[c] = reinterpret_cast<const double*>(st + St::K_O)[c * TILE + j];
+#pragma unroll
+        for (int c = 0; c < NS; ++c) xraw[c] = reinterpret_cast<const XT*>(st + St::X_O)[c * TILE + j];
+#pragma unroll
+        for (int c = 0; c < NI; ++c) un[c] = reinterpret_cast<const double*>(st + St::U_O)[c * TILE + j];
+        stage_release();  // proxy fence before the stage goes back to the bulk-copy engine
+        if (lane == 0) mbar_arrive(empty + s);
+        if (work) {
+            double xn[NS], u[NI];
+            finish_x(P, t, i, xraw, xn);
+            track_error(x, xn, emax);
+            track_input(K, x, xn, un, u);
+            track_advance<Q32>(P.M, x, u);
+        }
+    }
+    if (!work) return;
+    double xn[NS], efin[NS];
+    load_x(P, Xnom, TT - 1, i, xn);
+    track_final_err(x, xn, emax, efin);
+    const size_t o = ((size_t)i * M + m) * NS;
+#pragma unroll
+    for (int c = 0; c < NS; ++c) { em[o + c] = emax[c]; ef[o + c] = efin[c]; }
+}
+
 }  // namespace acoc

@@ -5,6 +5,8 @@ with ONE shared LQ solve (the gains depend only on the nominal trajectory).
 """
 from __future__ import annotations
 
+import ctypes as C
+
 import numpy as np
 
 from . import _lib as L
@@ -71,6 +73,64 @@ def lqr_tracking_many(xx_opt, uu_opt, delta, dyn=None, QQt=None, RRt=None, QQT=N
     if return_gains:
         return xr, ur, K
     return xr, ur
+
+
+def mc_deltas(delta, N):
+    """Perturbations of a dispersion study: (M,6) shared by all N instances or (N,M,6) -> (contiguous float64 array, shared, M)."""
+    d = np.asarray(delta, dtype=np.float64)
+    if d.ndim == 2 and d.shape[1] == 6:
+        shared, M = True, d.shape[0]
+    elif d.ndim == 3 and d.shape[0] == N and d.shape[2] == 6:
+        shared, M = False, d.shape[1]
+    else:
+        raise ValueError("delta has shape %s, expected (M,6) or %s" % (d.shape, (N, "M", 6)))
+    if M < 1:
+        raise ValueError("delta holds no sample (M = 0)")
+    return np.ascontiguousarray(d), shared, M
+
+
+def mc_call(call, N, M, tol, per_sample):
+    """Run acoc_track_mc / acoc_lqr_tracking_mc through call(tol_ptr, out_ptr) and collect its outputs as a dict."""
+    t = None if tol is None else L.f64(tol, (6,), "tol")
+    res = dict(worst_max=np.empty((N, 6)), mean_final=np.empty((N, 6)), n_reg=np.empty(N, dtype=np.int32))
+    if t is not None:
+        res["n_within"] = np.empty(N, dtype=np.int32)
+    if per_sample:
+        res["err_max"], res["err_final"] = np.empty((N, M, 6)), np.empty((N, M, 6))
+    out = L.TrackMcOut(*(L.ptr(res.get(k)) for k in ("err_max", "err_final", "worst_max", "mean_final", "n_within", "n_reg")))
+    L.check(call(L.ptr(t), C.addressof(out)))
+    return res
+
+
+def lqr_tracking_mc(xx_opt, uu_opt, delta, dyn=None, QQt=None, RRt=None, QQT=None, tol=None, per_sample=False, return_gains=False):
+    """Monte Carlo dispersion of the reference's lqr_tracking around each of N nominals: xx_opt (6,TT) or (N,6,TT), uu_opt (2,TT) or
+    (N,2,TT); delta (M,6) (the same M perturbations for every nominal) or (N,M,6).  Each nominal gets its own gains; sample (i, m) is the
+    closed loop from x*_0 + delta[i, m].  Returns dict(worst_max (N,6) = max over samples of max_t |x_t - x*_t| (NaN if any sample is
+    NaN), mean_final (N,6) = mean over samples of |x_{TT-1} - x*_{TT-1}|, n_reg (N)[, n_within (N) = samples whose max error is within
+    tol (6,) in every state][, err_max, err_final (N,M,6) per sample with per_sample=True][, K (N,2,6,TT) with return_gains=True]).
+    No trajectory is kept: the trajectory of sample m is lqr_tracking_many(xx_opt, uu_opt, delta[:, m]), whose summaries are bit-identical
+    to the per-sample ones here.  Same kernels as BatchedNewton.track_mc (acoc_lqr_tracking_mc).  The weights must be symmetric."""
+    dyn = dyn or Dynamics()
+    dQ, dR, dQT = default_weights()
+    Q = L.f64(dQ if QQt is None else QQt, (6, 6), "QQt")
+    R = L.f64(dR if RRt is None else RRt, (2, 2), "RRt")
+    QT = L.f64(dQT if QQT is None else QQT, (6, 6), "QQT")
+    xo, uo = L.f64(xx_opt), L.f64(uu_opt)
+    if xo.ndim == 2:
+        xo, uo = xo[None], uo[None]
+    if xo.ndim != 3 or xo.shape[1] != 6 or xo.shape[2] < 3:
+        raise ValueError("xx_opt must be (6,TT) or (N,6,TT) with TT >= 3, got %s" % (np.shape(xx_opt),))
+    N, _, TT = xo.shape
+    if uo.shape != (N, 2, TT):
+        raise ValueError("uu_opt has shape %s, expected %s" % (np.shape(uu_opt), (N, 2, TT)))
+    d, shared, M = mc_deltas(delta, N)
+    res = mc_call(lambda t, out: L.lib().acoc_lqr_tracking_mc(dyn.device, N, M, TT, L.ptr(dyn.params), int(dyn.state == "f64"), L.ptr(Q),
+                                                              L.ptr(R), L.ptr(QT), L.ptr(xo), L.ptr(uo), L.ptr(d), int(shared), t, out),
+                  N, M, tol, per_sample)
+    if return_gains:
+        # the gains depend on the nominals and weights alone: acoc_lqr_tracking_many runs the same gains sweep on them
+        res["K"] = lqr_tracking_many(xo, uo, np.zeros((N, 6)), dyn, Q, R, QT, return_gains=True)[2]
+    return res
 
 
 def lqr_tracking(xx_opt, uu_opt, tt, dyn=None, QQt=None, RRt=None, QQT=None):

@@ -237,9 +237,10 @@ int acoc_track(acoc_ctx* ctx, const double* Q, const double* R, const double* QT
                int* n_reg);
 /* trajectories of the last acoc_track: xx_reg (N,6,TT), uu_reg (N,2,TT); either may be NULL */
 int acoc_get_tracked(acoc_ctx* ctx, double* xx_reg, double* uu_reg);
-/* gains of the last acoc_track: K (N,2,6,TT), lqr_tracking's KK per instance (K[:,:,:,TT-1] = 0) */
+/* gains of the last acoc_track or acoc_track_mc: K (N,2,6,TT), lqr_tracking's KK per instance (K[:,:,:,TT-1] = 0) */
 int acoc_get_track_gains(acoc_ctx* ctx, double* K);
-/* device time (CUDA events, ms) of the last acoc_track: ms[0] total, ms[1] nominal (k_track_nominal), ms[2] gains sweep, ms[3] rollout */
+/* device time (CUDA events, ms) of the last acoc_track (or acoc_track_mc): ms[0] total, ms[1] nominal (k_track_nominal), ms[2] gains
+ * sweep, ms[3] rollout (acoc_track_mc: dispersion rollout + reduction) */
 int acoc_get_track_timing(acoc_ctx* ctx, double* ms);
 /* lqr_tracking (lqr_tracking.py:245-283) for n independent nominals from host arrays: xx_opt (n,6,TT), uu_opt (n,2,TT), delta (n,6);
  * outputs xx_reg (n,6,TT), uu_reg (n,2,TT), K (n,2,6,TT) or NULL.  The same kernels as acoc_track (bit-identical results for the same
@@ -247,6 +248,35 @@ int acoc_get_track_timing(acoc_ctx* ctx, double* ms);
 int acoc_lqr_tracking_many(int device, int n, int TT, const double* params, int state_f64, const double* Q, const double* R,
                            const double* QT, const double* xx_opt, const double* uu_opt, const double* delta, double* xx_reg,
                            double* uu_reg, double* K);
+
+/* ------------------------------------------ Monte Carlo dispersion of the closed loop -------------------- */
+/* Outputs of acoc_track_mc / acoc_lqr_tracking_mc; any pointer may be NULL.  M = samples per instance. */
+typedef struct acoc_track_mc_out {
+    double* err_max;    /* (N,M,6) per sample: max_t |x_t - x*_t| */
+    double* err_final;  /* (N,M,6) per sample: |x_{TT-1} - x*_{TT-1}| */
+    double* worst_max;  /* (N,6)  max over m of err_max[i,m,c], folded in sample order; one NaN sample gives NaN */
+    double* mean_final; /* (N,6)  (((e_0 + e_1) + e_2) + ...) / M of e_m = err_final[i,m,c] */
+    int* n_within;      /* (N)    samples with err_max[i,m,c] <= tol[c] for all six c (a NaN is never within); needs tol */
+    int* n_reg;         /* (N)    as acoc_track */
+} acoc_track_mc_out;
+/* acoc_track's closed loop from M perturbed starts per instance: nominal and gains exactly those of acoc_track (the instance's current
+ * result, tracking weights Q, R, QT symmetric), sample (i, m) flown from x*_0 + delta[i, m].  The per-sample summaries are bit-identical
+ * to acoc_track(delta = delta[:, m]) for instance i; the aggregates are computed on the device in a fixed order (no atomics).
+ * delta (M,6) when delta_shared (the same perturbations for every instance: common random numbers), else (N,M,6); copied as given.
+ * tol (6) or NULL: the tolerance of n_within.  No trajectory is kept: the trajectory of sample m is what acoc_track(delta[:, m]) returns.
+ * Reuses acoc_track's nominal and gains buffers: acoc_get_track_gains returns the gains it used, acoc_get_track_timing reports its
+ * kernels (ms[3] = dispersion rollout + reduction), and acoc_get_tracked returns ACOC_ERR_STATE until the next acoc_track.  It does
+ * not allocate the tracked-trajectory buffers; the per-sample buffers (96 B per sample, plus the deltas) are allocated on the first
+ * call, grow with N*M and are freed with the context (ACOC_ERR_NOMEM if they do not fit; the context is left as it was).  Writes
+ * nothing of the Newton solve.  ACOC_ERR_STATE for ACOC_FP32 contexts and before acoc_set_init / acoc_init_guess; ACOC_ERR_INVALID
+ * for m < 1, a NULL delta, non-symmetric weights, or n_within without tol. */
+int acoc_track_mc(acoc_ctx* ctx, const double* Q, const double* R, const double* QT, int m, const double* delta, int delta_shared,
+                  const double* tol, acoc_track_mc_out* out);
+/* acoc_track_mc for n nominals from host arrays xx_opt (n,6,TT), uu_opt (n,2,TT) (the twin of acoc_lqr_tracking_many, same cached
+ * context and float-storage decision; n = 1 with many deltas is the reference's single-optimum study, as summaries). */
+int acoc_lqr_tracking_mc(int device, int n, int m, int TT, const double* params, int state_f64, const double* Q, const double* R,
+                         const double* QT, const double* xx_opt, const double* uu_opt, const double* delta, int delta_shared,
+                         const double* tol, acoc_track_mc_out* out);
 
 /* Single pieces of the loop on the context's current iterate, exposed for parity tests and for the
  * reference's own method names:
