@@ -13,7 +13,9 @@
 //
 // Every sweep kernel is a template on the arithmetic/storage type F (double: the parity path; float: the optional FP32
 // mode, ACOC_FP32) and on the storage type XT of the state iterates (float whenever the states are float32 values anyway,
-// see acoc_kernels.cuh "Types").  The context keeps untyped device buffers; DISPATCH_FX / DISPATCH_F pick the instantiation.
+// see acoc_kernels.cuh "Types").  The context keeps untyped device buffers; DISPATCH_FX / DISPATCH_F pick the instantiation of a
+// host routine, and with_flag / with_flags / with_mode / with_real that of a kernel whose other template arguments (state
+// quantisation, diagonal weights, exact Hessians, reference mode, ...) are runtime facts of the context.
 #include <cuda_runtime.h>
 #include <stdarg.h>
 #include <stdint.h>
@@ -24,6 +26,8 @@
 #include <algorithm>
 #include <mutex>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "../../include/acoc.h"
@@ -86,30 +90,42 @@ constexpr int ROLL_THREADS = 64;
 constexpr int CAND_TILE = ACOC_CAND_TILE;  // instances per candidate CTA (one warp per candidate)
 constexpr int CAND_MAXY = 10;              // candidates per CTA; more candidates than this loop inside the thread
 
-// launch a kernel templated on the state quantisation (float32 rounding of aircraft_simplified.py:300 or none)
-#define LAUNCH_Q32(q32, kernel, targs, grid, block, stream, ...)                              \
-    do {                                                                                    \
-        if (q32) kernel<true, ACOC_UNPAREN targs><<<grid, block, 0, stream>>>(__VA_ARGS__);  \
-        else kernel<false, ACOC_UNPAREN targs><<<grid, block, 0, stream>>>(__VA_ARGS__);     \
-    } while (0)
-#define ACOC_UNPAREN(...) __VA_ARGS__
-// k_candidates<Q32, F, MAXY>: ny = candidates per CTA (blockDim.y <= CAND_MAXY); the 9-wide instantiation when it fits
-#define LAUNCH_CAND(q32, F_, grid, ny, stream, ...)                                                        \
-    do {                                                                                                  \
-        const dim3 blk__(CAND_TILE, (ny));                                                                \
-        if ((ny) <= 9) {                                                                                  \
-            if (q32) k_candidates<true, F_, 9><<<grid, blk__, 0, stream>>>(__VA_ARGS__);                  \
-            else k_candidates<false, F_, 9><<<grid, blk__, 0, stream>>>(__VA_ARGS__);                     \
-        } else {                                                                                          \
-            if (q32) k_candidates<true, F_, CAND_MAXY><<<grid, blk__, 0, stream>>>(__VA_ARGS__);          \
-            else k_candidates<false, F_, CAND_MAXY><<<grid, blk__, 0, stream>>>(__VA_ARGS__);             \
-        }                                                                                                 \
-    } while (0)
-
 // pick the instantiation of a host-side launch template for a context: <F, XT> or <F>
 #define DISPATCH_FX(c, fn, ...) \
     ((c)->fp32 ? fn<float, float>(__VA_ARGS__) : ((c)->x_float ? fn<double, float>(__VA_ARGS__) : fn<double, double>(__VA_ARGS__)))
 #define DISPATCH_F(c, fn, ...) ((c)->fp32 ? fn<float>(__VA_ARGS__) : fn<double>(__VA_ARGS__))
+
+// Pick the instantiation of a single launch: fn is called with the compile-time twin of a runtime value (std::true_type /
+// std::false_type, std::integral_constant<int, 0..2>, or type_tag<float> / type_tag<double>), which it uses as a template argument.
+// Every arm is instantiated, so a selector may only be used where every combination it produces is a kernel the library needs.
+template <typename Fn>
+static int with_flag(bool b, Fn&& fn) { return b ? fn(std::true_type{}) : fn(std::false_type{}); }
+template <typename Fn>
+static int with_flags(bool a, bool b, Fn&& fn)
+{
+    return with_flag(a, [&](auto A) { return with_flag(b, [&](auto B) { return fn(A, B); }); });
+}
+template <typename Fn>
+static int with_mode(int m, Fn&& fn)  // m = 0, 1 or 2
+{
+    return m == 2 ? fn(std::integral_constant<int, 2>{}) : m == 1 ? fn(std::integral_constant<int, 1>{}) : fn(std::integral_constant<int, 0>{});
+}
+template <typename T>
+struct type_tag { using type = T; };
+template <typename Fn>
+static int with_real(bool f32, Fn&& fn) { return f32 ? fn(type_tag<float>{}) : fn(type_tag<double>{}); }
+
+// launch a kernel that stages its inputs in dynamic shared memory (the TMA rings): the largest shared-memory carveout, and the
+// opt-in above the default 48 KB of dynamic shared memory where the kernel needs more
+template <typename... P, typename... A>
+static int launch_ring(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, A&&... a)
+{
+    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, block, smem, st>>>(std::forward<A>(a)...);
+    CK(cudaGetLastError());
+    return 0;
+}
 
 template <typename F, typename XT>
 __global__ void __launch_bounds__(128) k_traj_cost(ProblemT<F> P, const XT* __restrict__ X, const F* __restrict__ U,
@@ -1539,12 +1555,12 @@ int acoc_set_refs_generated(acoc_ctx* c, const double* tt, const double* zshape,
         return 0;
     }
     c->P.ref_param = 0;
-    if (c->fp32)
-        k_gen_refs<float><<<grid, 128, 0, c->stream>>>(c->N, c->Np, c->TT, d, d + T, vshape ? d + 2 * T : nullptr, d + 3 * T, d + 3 * T + N, K,
-                                                       (float*)c->xref, (float*)c->uref);
-    else
-        k_gen_refs<double><<<grid, 128, 0, c->stream>>>(c->N, c->Np, c->TT, d, d + T, vshape ? d + 2 * T : nullptr, d + 3 * T, d + 3 * T + N, K,
-                                                        (double*)c->xref, (double*)c->uref);
+    with_real(c->fp32, [&](auto R) {
+        using F = typename decltype(R)::type;
+        k_gen_refs<F><<<grid, 128, 0, c->stream>>>(c->N, c->Np, c->TT, d, d + T, vshape ? d + 2 * T : nullptr, d + 3 * T, d + 3 * T + N, K,
+                                                   (F*)c->xref, (F*)c->uref);
+        return 0;
+    });
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(c->stream));  // the staging buffer is free again; the host arrays may be reused
     c->have_refs = true;
@@ -1590,8 +1606,11 @@ static int init_guess_t(acoc_ctx* c, double kp, double kt, const double* dx0)
         CK(cudaStreamSynchronize(c->stream));
         d_dx0 = (F*)c->x0;
     }
-    LAUNCH_Q32(c->P.q32, k_init_guess, (F, XT), (c->N + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, c->stream, prob<F>(c), kp, kt, d_dx0,
-               (XT*)c->X[0], (F*)c->U[0], (F*)c->x0);
+    with_flag(c->P.q32, [&](auto Q) {
+        k_init_guess<Q, F, XT><<<(c->N + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, 0, c->stream>>>(prob<F>(c), kp, kt, d_dx0, (XT*)c->X[0],
+                                                                                                        (F*)c->U[0], (F*)c->x0);
+        return 0;
+    });
     CK(cudaGetLastError());
     return 0;
 }
@@ -1654,12 +1673,6 @@ static int sweep_grid(const acoc_ctx* c, int threads)
     const int tiles = std::max(1, std::min(n_tiles(c), c->ls_end) - c->ls_off);
     return (tiles * 32 + threads - 1) / threads;
 }
-template <typename K>
-static int prefer_smem(K kernel)
-{
-    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    return 0;
-}
 
 static WorkList act_list(acoc_ctx* c)
 {
@@ -1711,46 +1724,24 @@ static int launch_backward_t(acoc_ctx* c, bool exact)
     const ProblemT<F> P = prob<F>(c);
     const XT* X = (const XT*)c->X[cur];
     const F* U = (const F*)c->U[cur];
+    F* KSG = (F*)c->KSG;
+    const bool dg = c->P.W.diag != 0;
     if (use_tma(c) && bwd_cols(c)) {  // small batch: warp-role pipeline per tile (k_backward_cols)
-        const int gs = sweep_grid(c, TILE);
-        cudaStream_t st = sweep_stream(c);
-        const bool dg = c->P.W.diag != 0;
-#define ACOC_BC_LAUNCH(EX, DG)                                                                                                        \
-        do {                                                                                                                          \
-            const size_t sm = backward_cols_smem<EX, F, XT>();                                                                        \
-            TRY(prefer_smem(k_backward_cols<EX, F, XT, DG>));                                                                         \
-            if (sm > 48 * 1024) CK(cudaFuncSetAttribute(k_backward_cols<EX, F, XT, DG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm)); \
-            k_backward_cols<EX, F, XT, DG><<<gs, BC_THREADS, sm, st>>>(P, tile_list(c), X, U, (F*)c->KSG, c->S.status, c->S.n_reg);  \
-        } while (0)
-        if (exact) { if (dg) ACOC_BC_LAUNCH(true, 1); else ACOC_BC_LAUNCH(true, 0); }
-        else { if (dg) ACOC_BC_LAUNCH(false, 1); else ACOC_BC_LAUNCH(false, 0); }
-#undef ACOC_BC_LAUNCH
+        TRY(with_flags(exact, dg, [&](auto EX, auto DG) {
+            return launch_ring(k_backward_cols<EX, F, XT, DG>, sweep_grid(c, TILE), BC_THREADS, backward_cols_smem<EX, F, XT>(), sweep_stream(c), P,
+                               tile_list(c), X, U, KSG, c->S.status, c->S.n_reg);
+        }));
     } else if (use_tma(c) && bwd_split(c)) {  // small batch: costate warp + matrix warp per tile (k_backward_split)
-        const int gs = sweep_grid(c, TILE);
-        cudaStream_t st = sweep_stream(c);
-        const bool dg = c->P.W.diag != 0;
-#define ACOC_BS_LAUNCH(EX, DG)                                                                                                        \
-        do {                                                                                                                          \
-            const size_t sm = backward_split_smem<EX, F, XT>();                                                                       \
-            TRY(prefer_smem(k_backward_split<EX, F, XT, DG>));                                                                        \
-            k_backward_split<EX, F, XT, DG><<<gs, 64, sm, st>>>(P, tile_list(c), X, U, (F*)c->KSG, c->S.status, c->S.n_reg);         \
-        } while (0)
-        if (exact) { if (dg) ACOC_BS_LAUNCH(true, 1); else ACOC_BS_LAUNCH(true, 0); }
-        else { if (dg) ACOC_BS_LAUNCH(false, 1); else ACOC_BS_LAUNCH(false, 0); }
-#undef ACOC_BS_LAUNCH
+        TRY(with_flags(exact, dg, [&](auto EX, auto DG) {
+            return launch_ring(k_backward_split<EX, F, XT, DG>, sweep_grid(c, TILE), 64, backward_split_smem<EX, F, XT>(), sweep_stream(c), P,
+                               tile_list(c), X, U, KSG, c->S.status, c->S.n_reg);
+        }));
     } else if (use_tma(c)) {
         const size_t sm = WarpRing<BWD_STAGES, BwdStage<F, XT>::BYTES>::smem_bytes(BWD_THREADS / 32);
-        const int gs = sweep_grid(c, BWD_THREADS);
-        cudaStream_t st = sweep_stream(c);
-        const bool dg = c->P.W.diag != 0;
-#define ACOC_BWD_LAUNCH(EX, DG)                                                                                                  \
-        do {                                                                                                                     \
-            TRY(prefer_smem(k_backward_tma<EX, F, XT, DG>));                                                                     \
-            k_backward_tma<EX, F, XT, DG><<<gs, BWD_THREADS, sm, st>>>(P, tile_list(c), X, U, (F*)c->KSG, c->S.status, c->S.n_reg); \
-        } while (0)
-        if (exact) { if (dg) ACOC_BWD_LAUNCH(true, 1); else ACOC_BWD_LAUNCH(true, 0); }
-        else { if (dg) ACOC_BWD_LAUNCH(false, 1); else ACOC_BWD_LAUNCH(false, 0); }
-#undef ACOC_BWD_LAUNCH
+        TRY(with_flags(exact, dg, [&](auto EX, auto DG) {
+            return launch_ring(k_backward_tma<EX, F, XT, DG>, sweep_grid(c, BWD_THREADS), BWD_THREADS, sm, sweep_stream(c), P, tile_list(c), X, U,
+                               KSG, c->S.status, c->S.n_reg);
+        }));
         if (!c->bwd_wave_ctas) {  // resident CTAs of this sweep on the whole device (for the two-range split of acoc_newton_iterate)
             int nb = 0, sms = 0;
             CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_backward_tma<true, F, XT, 1>, BWD_THREADS, sm));
@@ -1758,8 +1749,11 @@ static int launch_backward_t(acoc_ctx* c, bool exact)
             c->bwd_wave_ctas = std::max(1, nb * sms);
             c->sm_count = sms;
         }
-    } else if (exact) k_backward<true, F, XT><<<g, BWD_THREADS, 0, c->stream>>>(P, act_list(c), X, U, (F*)c->KSG, c->S.status, c->S.n_reg);
-    else k_backward<false, F, XT><<<g, BWD_THREADS, 0, c->stream>>>(P, act_list(c), X, U, (F*)c->KSG, c->S.status, c->S.n_reg);
+    } else
+        with_flag(exact, [&](auto EX) {
+            k_backward<EX, F, XT><<<g, BWD_THREADS, 0, c->stream>>>(P, act_list(c), X, U, KSG, c->S.status, c->S.n_reg);
+            return 0;
+        });
     CK(cudaGetLastError());
     ++c->launches;
     return 0;
@@ -1776,9 +1770,8 @@ static int launch_gradient_t(acoc_ctx* c)
     const F* U = (const F*)c->U[cur];
     if (use_tma(c)) {
         const size_t sm = WarpRing<BWD_STAGES, BwdStage<F, XT>::BYTES>::smem_bytes(BWD_THREADS / 32);
-        TRY(prefer_smem(k_gradient_tma<F, XT>));
-        k_gradient_tma<F, XT><<<sweep_grid(c, BWD_THREADS), BWD_THREADS, sm, sweep_stream(c)>>>(P, tile_list(c), X, U, (F*)c->DU, c->S.status,
-                                                                                             c->S.descent);
+        TRY(launch_ring(k_gradient_tma<F, XT>, sweep_grid(c, BWD_THREADS), BWD_THREADS, sm, sweep_stream(c), P, tile_list(c), X, U, (F*)c->DU,
+                        c->S.status, c->S.descent));
     } else
         k_gradient<F, XT><<<(c->Np + FWD_THREADS - 1) / FWD_THREADS, FWD_THREADS, 0, c->stream>>>(P, act_list(c), X, U, (F*)c->DU, c->S.status,
                                                                                                c->S.descent);
@@ -1793,10 +1786,9 @@ static int launch_forward_t(acoc_ctx* c)
 {
     const int cur = c->kk % 3, g = (c->Np + FWD_THREADS - 1) / FWD_THREADS;
     if (use_tma(c)) {
-        TRY(prefer_smem(k_forward_tma<F, XT>));
-        k_forward_tma<F, XT><<<sweep_grid(c, FWD_THREADS), FWD_THREADS, WarpRing<FWD_STAGES, FwdStage<F, XT>::BYTES>::smem_bytes(FWD_THREADS / 32),
-                               sweep_stream(c)>>>(prob<F>(c), tile_list(c), (const XT*)c->X[cur], (const F*)c->U[cur], (const F*)c->KSG, (F*)c->DU,
-                                                  c->S.status, c->S.descent);
+        TRY(launch_ring(k_forward_tma<F, XT>, sweep_grid(c, FWD_THREADS), FWD_THREADS,
+                        WarpRing<FWD_STAGES, FwdStage<F, XT>::BYTES>::smem_bytes(FWD_THREADS / 32), sweep_stream(c), prob<F>(c), tile_list(c),
+                        (const XT*)c->X[cur], (const F*)c->U[cur], (const F*)c->KSG, (F*)c->DU, c->S.status, c->S.descent));
     } else
         k_forward<F, XT><<<g, FWD_THREADS, 0, c->stream>>>(prob<F>(c), act_list(c), (const XT*)c->X[cur], (const F*)c->U[cur], (const F*)c->KSG,
                                                            (F*)c->DU, (F*)nullptr, c->S.status, c->S.descent);
@@ -1830,21 +1822,16 @@ static int launch_cand0_t(acoc_ctx* c)
     const F *U = (const F*)c->U[cur], *DU = (const F*)c->DU;
     if (use_tma(c)) {
         const size_t sm = WarpRing<ROLL_STAGES, RollStage<F>::BYTES>::smem_bytes(ROLL_THREADS / 32);
-        const int g = sweep_grid(c, ROLL_THREADS);
-        cudaStream_t st = sweep_stream(c);
-        const bool dg = c->P.W.diag != 0;
-#define ACOC_RW0_LAUNCH(Q, DG)                                                                                                    \
-        do {                                                                                                                      \
-            TRY(prefer_smem(k_rollout_write_tma<Q, F, XT, 0, DG>));                                                               \
-            k_rollout_write_tma<Q, F, XT, 0, DG><<<g, ROLL_THREADS, sm, st>>>(P, tile_list(c), c->O, c->S, U, DU, c->cand_steps, (XT*)c->X[nxt], \
-                                                                             (F*)c->U[nxt], nullptr, c->kk, 0);                     \
-        } while (0)
-        if (c->P.q32) { if (dg) ACOC_RW0_LAUNCH(true, 1); else ACOC_RW0_LAUNCH(true, 0); }
-        else { if (dg) ACOC_RW0_LAUNCH(false, 1); else ACOC_RW0_LAUNCH(false, 0); }
-#undef ACOC_RW0_LAUNCH
+        TRY(with_flags(c->P.q32, c->P.W.diag != 0, [&](auto Q, auto DG) {
+            return launch_ring(k_rollout_write_tma<Q, F, XT, 0, DG>, sweep_grid(c, ROLL_THREADS), ROLL_THREADS, sm, sweep_stream(c), P,
+                               tile_list(c), c->O, c->S, U, DU, c->cand_steps, (XT*)c->X[nxt], (F*)c->U[nxt], nullptr, c->kk, 0);
+        }));
     } else
-        LAUNCH_Q32(c->P.q32, k_candidate0_write, (F, XT), (Np + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, c->stream, P, act_list(c), U, DU,
-                   c->cand_steps, (XT*)c->X[nxt], (F*)c->U[nxt], c->S.status, c->S.Jcand);
+        with_flag(c->P.q32, [&](auto Q) {
+            k_candidate0_write<Q, F, XT><<<(Np + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, 0, c->stream>>>(
+                P, act_list(c), U, DU, c->cand_steps, (XT*)c->X[nxt], (F*)c->U[nxt], c->S.status, c->S.Jcand);
+            return 0;
+        });
     CK(cudaGetLastError());
     ++c->launches;
     return 0;
@@ -1863,19 +1850,10 @@ static int launch_forward_cand0_t(acoc_ctx* c)
     const int cur = c->kk % 3, nxt = (c->kk + 1) % 3;
     const ProblemT<F> P = prob<F>(c);
     const size_t sm = WarpRing<FC_STAGES, FwdCandStage<F, XT>::BYTES>::smem_bytes(FWD_THREADS / 32);
-    const int g = sweep_grid(c, FWD_THREADS);
-    cudaStream_t st = sweep_stream(c);
-    const bool dg = c->P.W.diag != 0;
-#define ACOC_FC_LAUNCH(Q, DG)                                                                                                       \
-    do {                                                                                                                            \
-        TRY(prefer_smem(k_forward_cand0_tma<Q, F, XT, DG>));                                                                        \
-        k_forward_cand0_tma<Q, F, XT, DG><<<g, FWD_THREADS, sm, st>>>(P, tile_list(c), c->S, (const XT*)c->X[cur], (const F*)c->U[cur],  \
-                                                                     (const F*)c->KSG, (F*)c->DU, c->cand_steps, (XT*)c->X[nxt], (F*)c->U[nxt]); \
-    } while (0)
-    if (c->P.q32) { if (dg) ACOC_FC_LAUNCH(true, 1); else ACOC_FC_LAUNCH(true, 0); }
-    else { if (dg) ACOC_FC_LAUNCH(false, 1); else ACOC_FC_LAUNCH(false, 0); }
-#undef ACOC_FC_LAUNCH
-    CK(cudaGetLastError());
+    TRY(with_flags(c->P.q32, c->P.W.diag != 0, [&](auto Q, auto DG) {
+        return launch_ring(k_forward_cand0_tma<Q, F, XT, DG>, sweep_grid(c, FWD_THREADS), FWD_THREADS, sm, sweep_stream(c), P, tile_list(c), c->S,
+                           (const XT*)c->X[cur], (const F*)c->U[cur], (const F*)c->KSG, (F*)c->DU, c->cand_steps, (XT*)c->X[nxt], (F*)c->U[nxt]);
+    }));
     ++c->launches;
     return 0;
 }
@@ -1884,17 +1862,23 @@ static int launch_forward_cand0(acoc_ctx* c) { return DISPATCH_FX(c, launch_forw
 // candidates c0..c1-1 of the instances on a per-instance work list (n list slots at most): the ring kernel of acoc_tma.cuh (one
 // producer warp gathers the inputs for all candidate warps of a CTA) or, with ACOC_NO_TMA, the plain-load kernel
 constexpr int LIST_ROWS = 9;  // candidate warps per CTA of k_candidates_list (more candidates: several passes)
-template <typename K>
-static int list_smem_attr(K kernel, size_t bytes)
-{
-    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    if (bytes > 48 * 1024) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    return 0;
-}
 static bool list_ring(const acoc_ctx* c)
 {
     static const bool off = getenv("ACOC_NO_LIST_RING") != nullptr;  // tuning experiments
     return use_tma(c) && !off;
+}
+// the plain-load kernel k_candidates<Q32, F, MAXY> for candidates c0..c1-1 with step table `steps`: at most CAND_MAXY candidates
+// per CTA (blockDim.y), the 9-wide instantiation when it fits
+template <typename F>
+static void launch_candidates(acoc_ctx* c, const WorkList& L, int n, const F* U, const F* DU, const double* steps, int c0, int c1,
+                              cudaStream_t st)
+{
+    const int ny = std::min(c1 - c0, CAND_MAXY);
+    with_flags(c->P.q32, ny <= 9, [&](auto Q, auto Y9) {
+        k_candidates<Q, F, Y9 ? 9 : CAND_MAXY><<<(n + CAND_TILE - 1) / CAND_TILE, dim3(CAND_TILE, ny), 0, st>>>(prob<F>(c), L, U, DU, steps, c0, c1,
+                                                                                                               c->S.status, c->S.Jcand);
+        return 0;
+    });
 }
 template <typename F>
 static int launch_list_candidates(acoc_ctx* c, const WorkList& L, int n, int c0, int c1, cudaStream_t st)
@@ -1903,23 +1887,16 @@ static int launch_list_candidates(acoc_ctx* c, const WorkList& L, int n, int c0,
     const ProblemT<F> P = prob<F>(c);
     const F *U = (const F*)c->U[cur], *DU = (const F*)c->DU;
     if (list_ring(c)) {
-        const int rows = std::min(c1 - c0, LIST_ROWS);
-        const dim3 blk(TILE, rows + 1);
-        const size_t sm = candidates_list_smem<F>();
-        const bool dg = c->P.W.diag != 0;
+        const dim3 blk(TILE, std::min(c1 - c0, LIST_ROWS) + 1);
         const int rf = c->P.ref_param ? 2 : (c->P.ref_shared ? 1 : 0);
-#define ACOC_CL_LAUNCH(Q, DG, SH)                                                                                                   \
-        do {                                                                                                                        \
-            TRY(list_smem_attr(k_candidates_list<Q, F, LIST_ROWS, DG, SH>, sm));                                                    \
-            k_candidates_list<Q, F, LIST_ROWS, DG, SH><<<(n + TILE - 1) / TILE, blk, sm, st>>>(P, L, U, DU, c->cand_steps, c0, c1, c->S.Jcand); \
-        } while (0)
-#define ACOC_CL_LAUNCH2(Q, DG) do { if (rf == 2) ACOC_CL_LAUNCH(Q, DG, 2); else if (rf == 1) ACOC_CL_LAUNCH(Q, DG, 1); else ACOC_CL_LAUNCH(Q, DG, 0); } while (0)
-        if (c->P.q32) { if (dg) ACOC_CL_LAUNCH2(true, 1); else ACOC_CL_LAUNCH2(true, 0); }
-        else { if (dg) ACOC_CL_LAUNCH2(false, 1); else ACOC_CL_LAUNCH2(false, 0); }
-#undef ACOC_CL_LAUNCH2
-#undef ACOC_CL_LAUNCH
+        TRY(with_flags(c->P.q32, c->P.W.diag != 0, [&](auto Q, auto DG) {
+            return with_mode(rf, [&](auto REFS) {
+                return launch_ring(k_candidates_list<Q, F, LIST_ROWS, DG, REFS>, (n + TILE - 1) / TILE, blk, candidates_list_smem<F>(), st, P, L, U,
+                                   DU, c->cand_steps, c0, c1, c->S.Jcand);
+            });
+        }));
     } else
-        LAUNCH_CAND(c->P.q32, F, (n + CAND_TILE - 1) / CAND_TILE, std::min(c1 - c0, CAND_MAXY), st, P, L, U, DU, c->cand_steps, c0, c1, c->S.status, c->S.Jcand);
+        launch_candidates<F>(c, L, n, U, DU, c->cand_steps, c0, c1, st);
     CK(cudaGetLastError());
     return 0;
 }
@@ -1930,7 +1907,6 @@ template <typename F, typename XT>
 static int launch_armijo_t(acoc_ctx* c, bool* lazy_only)
 {
     const int cur = c->kk % 3, Np = c->Np, nc = c->O.armijo_maxiters;
-    const ProblemT<F> P = prob<F>(c);
     const F *U = (const F*)c->U[cur], *DU = (const F*)c->DU;
     *lazy_only = false;
     cudaStream_t st = sweep_stream(c);
@@ -1962,8 +1938,7 @@ static int launch_armijo_t(acoc_ctx* c, bool* lazy_only)
         }
         *lazy_only = true;
     } else {
-        LAUNCH_CAND(c->P.q32, F, (Np + CAND_TILE - 1) / CAND_TILE, std::min(nc, CAND_MAXY), c->stream, P, act_list(c), U, DU, c->cand_steps, 0, nc,
-                    c->S.status, c->S.Jcand);
+        launch_candidates<F>(c, act_list(c), Np, U, DU, c->cand_steps, 0, nc, c->stream);
         CK(cudaGetLastError());
         ++c->launches;
     }
@@ -1980,24 +1955,20 @@ static int launch_update_t(acoc_ctx* c, bool lazy_only, bool bookkeeping, bool u
     const int cur = c->kk % 3, nxt = (c->kk + 1) % 3;
     WorkList L = act_list(c);
     if (!use_list) L.groups = nullptr;
+    const int* only = lazy_only ? c->need : nullptr;
     if (use_tma(c)) {
         const size_t sm = WarpRing<ROLL_STAGES, RollStage<F>::BYTES>::smem_bytes(ROLL_THREADS / 32);
-        const int g = sweep_grid(c, ROLL_THREADS);
-        const int* only = lazy_only ? c->need : nullptr;
-        const bool dg = c->P.W.diag != 0;
-#define ACOC_RW1_LAUNCH(Q, DG)                                                                                                      \
-        do {                                                                                                                        \
-            TRY(prefer_smem(k_rollout_write_tma<Q, F, XT, 1, DG>));                                                                 \
-            k_rollout_write_tma<Q, F, XT, 1, DG><<<g, ROLL_THREADS, sm, sweep_stream(c)>>>(prob<F>(c), tile_list(c, use_list), c->O, c->S,        \
-                                                                                          (const F*)c->U[cur], (const F*)c->DU, c->cand_steps,   \
-                                                                                          (XT*)c->X[nxt], (F*)c->U[nxt], only, c->kk, bookkeeping ? 1 : 0); \
-        } while (0)
-        if (c->P.q32) { if (dg) ACOC_RW1_LAUNCH(true, 1); else ACOC_RW1_LAUNCH(true, 0); }
-        else { if (dg) ACOC_RW1_LAUNCH(false, 1); else ACOC_RW1_LAUNCH(false, 0); }
-#undef ACOC_RW1_LAUNCH
+        TRY(with_flags(c->P.q32, c->P.W.diag != 0, [&](auto Q, auto DG) {
+            return launch_ring(k_rollout_write_tma<Q, F, XT, 1, DG>, sweep_grid(c, ROLL_THREADS), ROLL_THREADS, sm, sweep_stream(c), prob<F>(c),
+                               tile_list(c, use_list), c->O, c->S, (const F*)c->U[cur], (const F*)c->DU, c->cand_steps, (XT*)c->X[nxt],
+                               (F*)c->U[nxt], only, c->kk, bookkeeping ? 1 : 0);
+        }));
     } else
-        LAUNCH_Q32(c->P.q32, k_update, (F, XT), (c->Np + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, c->stream, prob<F>(c), L, c->O, c->S,
-                   (const F*)c->U[cur], (const F*)c->DU, (XT*)c->X[nxt], (F*)c->U[nxt], lazy_only ? c->need : nullptr, c->kk, bookkeeping ? 1 : 0);
+        with_flag(c->P.q32, [&](auto Q) {
+            k_update<Q, F, XT><<<(c->Np + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, 0, c->stream>>>(
+                prob<F>(c), L, c->O, c->S, (const F*)c->U[cur], (const F*)c->DU, (XT*)c->X[nxt], (F*)c->U[nxt], only, c->kk, bookkeeping ? 1 : 0);
+            return 0;
+        });
     CK(cudaGetLastError());
     ++c->launches;
     return 0;
@@ -2044,14 +2015,12 @@ static int launch_fused_sweep_t(acoc_ctx* c)
     const int cur = c->kk % 3, rows = c->O.armijo_maxiters + 1;
     const size_t rx = (size_t)c->TT * NS * c->Np, ru = (size_t)c->TT * NI * c->Np;
     const dim3 blk(TILE, rows + 1);
-    if (c->P.q32)
-        k_search_fused<true, F, XT><<<n_tiles(c), blk, 0, c->stream>>>(prob<F>(c), tile_list(c), (const XT*)c->X[cur], (const F*)c->U[cur],
-                                                                      (const F*)c->KSG, (F*)c->DU, c->cand_steps, rows, (XT*)c->candX,
-                                                                      (F*)c->candU, rx, ru, c->S.status, c->S.descent, c->S.Jcand);
-    else
-        k_search_fused<false, F, XT><<<n_tiles(c), blk, 0, c->stream>>>(prob<F>(c), tile_list(c), (const XT*)c->X[cur], (const F*)c->U[cur],
-                                                                       (const F*)c->KSG, (F*)c->DU, c->cand_steps, rows, (XT*)c->candX,
-                                                                       (F*)c->candU, rx, ru, c->S.status, c->S.descent, c->S.Jcand);
+    with_flag(c->P.q32, [&](auto Q) {
+        k_search_fused<Q, F, XT><<<n_tiles(c), blk, 0, c->stream>>>(prob<F>(c), tile_list(c), (const XT*)c->X[cur], (const F*)c->U[cur],
+                                                                   (const F*)c->KSG, (F*)c->DU, c->cand_steps, rows, (XT*)c->candX, (F*)c->candU,
+                                                                   rx, ru, c->S.status, c->S.descent, c->S.Jcand);
+        return 0;
+    });
     CK(cudaGetLastError());
     ++c->launches;
     return 0;
@@ -2467,21 +2436,23 @@ static int deliver_finished(acoc_ctx* ctx, const Delivery& dv, int* n_new)
     static const int ctas = getenv("ACOC_DELIVER_CTAS") ? atoi(getenv("ACOC_DELIVER_CTAS")) : 64;  // (8: 536 ms, 16: 373, 32: 293, 64: 281 ms end to end; a machine-filling grid: 320)
     const int gx = std::max(1, ctas), gu = gx;
     const int *rs = ctx->S.result_slot, *rows = ctx->deliver_rows;
-    if (ctx->x_float) {
-        const float *a = (const float*)ctx->X[0], *b = (const float*)ctx->X[1], *c2 = (const float*)ctx->X[2];
-        if (dv.x_f32) k_deliver<float, float><<<gx, block, 0, dv.stream>>>(a, b, c2, rs, rows, nullptr, (float*)dv.xx, N, 6, TT, Np, 0);
-        else k_deliver<float, double><<<gx, block, 0, dv.stream>>>(a, b, c2, rs, rows, ctx->fp32 ? nullptr : (const double*)ctx->x0, (double*)dv.xx, N, 6, TT, Np, 0);
-    } else {
-        const double *a = (const double*)ctx->X[0], *b = (const double*)ctx->X[1], *c2 = (const double*)ctx->X[2];
-        k_deliver<double, double><<<gx, block, 0, dv.stream>>>(a, b, c2, rs, rows, nullptr, (double*)dv.xx, N, 6, TT, Np, 0);
-    }
-    CK(cudaGetLastError());
-    if (ctx->fp32)
-        k_deliver<float, double><<<gu, block, 0, dv.stream>>>((const float*)ctx->U[0], (const float*)ctx->U[1], (const float*)ctx->U[2], rs, rows, nullptr,
-                                                                dv.uu, N, 2, TT, Np, 1);
+    // k_deliver<D, O>: the three slots s (elements of type D) into dst (elements of type O)
+    const auto deliver = [&](auto d, auto o, int grid, void* const* s, const double* row0, void* dst, int C, int dup_last) {
+        using D = typename decltype(d)::type;
+        using O = typename decltype(o)::type;
+        k_deliver<D, O><<<grid, block, 0, dv.stream>>>((const D*)s[0], (const D*)s[1], (const D*)s[2], rs, rows, row0, (O*)dst, N, C, TT, Np, dup_last);
+        return 0;
+    };
+    if (ctx->x_float)  // float32 values: delivered as float, or as double with the exact row 0
+        with_real(dv.x_f32, [&](auto O) {
+            return deliver(type_tag<float>{}, O, gx, ctx->X, dv.x_f32 || ctx->fp32 ? nullptr : (const double*)ctx->x0, dv.xx, 6, 0);
+        });
     else
-        k_deliver<double, double><<<gu, block, 0, dv.stream>>>((const double*)ctx->U[0], (const double*)ctx->U[1], (const double*)ctx->U[2], rs, rows,
-                                                                 nullptr, dv.uu, N, 2, TT, Np, 1);  // uu_star[:,-1] = uu_star[:,-2], optcon.py:505
+        deliver(type_tag<double>{}, type_tag<double>{}, gx, ctx->X, nullptr, dv.xx, 6, 0);
+    CK(cudaGetLastError());
+    with_real(ctx->fp32, [&](auto D) {
+        return deliver(D, type_tag<double>{}, gu, ctx->U, nullptr, dv.uu, 2, 1);  // uu_star[:,-1] = uu_star[:,-2], optcon.py:505
+    });
     CK(cudaGetLastError());
     CK(cudaEventRecord(ctx->ev_deliver, dv.stream));  // the rows table is free again once these copies are done
     return 0;
@@ -2671,8 +2642,7 @@ static int launch_all_candidates_t(acoc_ctx* c)
     const int cur = c->kk % 3, N = c->N, nc = c->O.armijo_maxiters;
     WorkList L;
     L.groups = nullptr; L.count = c->counters + 1; L.shift = 0;
-    LAUNCH_CAND(c->P.q32, F, (N + CAND_TILE - 1) / CAND_TILE, std::min(nc, CAND_MAXY), c->stream, prob<F>(c), L, (const F*)c->U[cur],
-                (const F*)c->DU, c->cand_steps, 0, nc, c->S.status, c->S.Jcand);
+    launch_candidates<F>(c, L, N, (const F*)c->U[cur], (const F*)c->DU, c->cand_steps, 0, nc, c->stream);
     CK(cudaGetLastError());
     return 0;
 }
@@ -2704,8 +2674,7 @@ static int launch_sweep_candidates_t(acoc_ctx* c, const double* dsteps, int n)
     const int cur = c->kk % 3, N = c->N;
     WorkList L;
     L.groups = nullptr; L.count = c->counters + 1; L.shift = 0;
-    LAUNCH_CAND(c->P.q32, F, (N + CAND_TILE - 1) / CAND_TILE, std::min(n, CAND_MAXY), c->stream, prob<F>(c), L, (const F*)c->U[cur],
-                (const F*)c->DU, dsteps, 0, n, c->S.status, c->S.Jcand);
+    launch_candidates<F>(c, L, N, (const F*)c->U[cur], (const F*)c->DU, dsteps, 0, n, c->stream);
     CK(cudaGetLastError());
     return 0;
 }
@@ -2945,8 +2914,11 @@ int acoc_lqr_tracking(int device, int n, int TT, const double* params, int state
     TRY(lq_dense_dev(1, TT, false, dA, dB, dQ, dR, dS, dQf, dx0, nullptr, nullptr, nullptr, dK, nullptr, dxo, duo, nullptr, c->stream));
     CK(cudaEventRecord(c->ev[1], c->stream));
     const Problem P = prob<double>(c);
-    if (c->P.q32) k_track<true><<<(n + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, 0, c->stream>>>(P, dK, d_xopt, d_uopt, dstart, (double*)c->X[0], (double*)c->U[0]);
-    else k_track<false><<<(n + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, 0, c->stream>>>(P, dK, d_xopt, d_uopt, dstart, (double*)c->X[0], (double*)c->U[0]);
+    with_flag(c->P.q32, [&](auto Q) {
+        k_track<Q><<<(n + ROLL_THREADS - 1) / ROLL_THREADS, ROLL_THREADS, 0, c->stream>>>(P, dK, d_xopt, d_uopt, dstart, (double*)c->X[0],
+                                                                                          (double*)c->U[0]);
+        return 0;
+    });
     CK(cudaGetLastError());
     CK(cudaEventRecord(c->ev[2], c->stream));
     TRY(download_soa(c, c->X[0], nullptr, nullptr, nullptr, xx_reg, n, 6, c->Np, 0));
@@ -3075,12 +3047,13 @@ static int launch_track_gains(acoc_ctx* c, const Problem& P)
     cudaStream_t st = c->stream;
     const int g = (c->N + 63) / 64;  // 64 threads = two tiles per CTA
     CK(cudaEventRecord(c->tk_ev[1], st));
-    if (use_tma(c)) {
-        const size_t sm = WarpRing<TRK_GAIN_STAGES, TrkGainStage<XT>::BYTES>::smem_bytes(2);
-        if (P.W.diag) { TRY(prefer_smem(k_track_gains_tma<1, XT>)); k_track_gains_tma<1, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, c->tk_nreg); }
-        else { TRY(prefer_smem(k_track_gains_tma<0, XT>)); k_track_gains_tma<0, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, c->tk_nreg); }
-    } else if (P.W.diag) k_track_gains<1, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, c->tk_nreg);
-    else k_track_gains<0, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, c->tk_nreg);
+    TRY(with_flag(P.W.diag != 0, [&](auto DG) {
+        if (use_tma(c))
+            return launch_ring(k_track_gains_tma<DG, XT>, g, 64, WarpRing<TRK_GAIN_STAGES, TrkGainStage<XT>::BYTES>::smem_bytes(2), st, P, Xn, Un, K,
+                               c->tk_nreg);
+        k_track_gains<DG, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, c->tk_nreg);
+        return 0;
+    }));
     CK(cudaGetLastError());
     CK(cudaEventRecord(c->tk_ev[2], st));
     return 0;
@@ -3098,16 +3071,13 @@ static int launch_track_sweeps(acoc_ctx* c, const Weights& W)
     XT* X = (XT*)c->tk_x;
     cudaStream_t st = c->stream;
     const int g = (c->N + 63) / 64;
-    if (use_tma(c)) {
-        const size_t sm = WarpRing<TRK_ROLL_STAGES, TrkRollStage<XT>::BYTES>::smem_bytes(2);
-        if (c->P.q32) {
-            TRY(prefer_smem(k_track_rollout_tma<true, XT>));
-            k_track_rollout_tma<true, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, dl, X, x0, U, em, ef);
-        } else {
-            TRY(prefer_smem(k_track_rollout_tma<false, XT>));
-            k_track_rollout_tma<false, XT><<<g, 64, sm, st>>>(P, Xn, Un, K, dl, X, x0, U, em, ef);
-        }
-    } else LAUNCH_Q32(c->P.q32, k_track_rollout, (XT), g, 64, st, P, Xn, Un, K, dl, X, x0, U, em, ef);
+    TRY(with_flag(c->P.q32, [&](auto Q) {
+        if (use_tma(c))
+            return launch_ring(k_track_rollout_tma<Q, XT>, g, 64, WarpRing<TRK_ROLL_STAGES, TrkRollStage<XT>::BYTES>::smem_bytes(2), st, P, Xn, Un, K,
+                               dl, X, x0, U, em, ef);
+        k_track_rollout<Q, XT><<<g, 64, 0, st>>>(P, Xn, Un, K, dl, X, x0, U, em, ef);
+        return 0;
+    }));
     CK(cudaGetLastError());
     CK(cudaEventRecord(c->tk_ev[3], st));
     return 0;
@@ -3130,18 +3100,17 @@ static int launch_track_mc(acoc_ctx* c, const Weights& W, int m, long long dstri
         const int cpt = (int)((lanes * m + TRK_MC_WARPS * TILE - 1) / (TRK_MC_WARPS * TILE));
         const long long grid = (long long)n_tiles(c) * cpt;
         REQUIRE(grid <= 0x7fffffffLL, "acoc_track_mc: %d instances x %d samples is too many for one launch", c->N, m);
-        const size_t sm = track_mc_smem<XT>();
-        if (c->P.q32) {
-            TRY(prefer_smem(k_track_mc_rollout_tma<true, XT>));
-            k_track_mc_rollout_tma<true, XT><<<(unsigned)grid, TRK_MC_THREADS, sm, st>>>(P, Xn, Un, K, dl, dstride, m, cpt, em, ef);
-        } else {
-            TRY(prefer_smem(k_track_mc_rollout_tma<false, XT>));
-            k_track_mc_rollout_tma<false, XT><<<(unsigned)grid, TRK_MC_THREADS, sm, st>>>(P, Xn, Un, K, dl, dstride, m, cpt, em, ef);
-        }
+        TRY(with_flag(c->P.q32, [&](auto Q) {
+            return launch_ring(k_track_mc_rollout_tma<Q, XT>, (unsigned)grid, TRK_MC_THREADS, track_mc_smem<XT>(), st, P, Xn, Un, K, dl, dstride, m,
+                               cpt, em, ef);
+        }));
     } else {
         const long long grid = ((long long)c->N * m + 63) / 64;
         REQUIRE(grid <= 0x7fffffffLL, "acoc_track_mc: %d instances x %d samples is too many for one launch", c->N, m);
-        LAUNCH_Q32(c->P.q32, k_track_mc_rollout, (XT), (unsigned)grid, 64, st, P, Xn, Un, K, dl, dstride, m, em, ef);
+        with_flag(c->P.q32, [&](auto Q) {
+            k_track_mc_rollout<Q, XT><<<(unsigned)grid, 64, 0, st>>>(P, Xn, Un, K, dl, dstride, m, em, ef);
+            return 0;
+        });
     }
     CK(cudaGetLastError());
     TrackTol tl{};
@@ -3198,15 +3167,13 @@ static int copy_track_nominal(acoc_ctx* c, bool xf)
     k_result_slot_default<<<(c->N + 255) / 256, 256, 0, c->stream>>>(c->S.status, c->slot_tmp, c->S.result_slot, c->kk % 3, c->N);
     const int tchunk = 8;
     const dim3 grid((unsigned)((c->N + 127) / 128), (unsigned)((c->TT + tchunk - 1) / tchunk));
-    if (xf)
-        k_track_nominal<float><<<grid, 128, 0, c->stream>>>((const float*)c->X[0], (const float*)c->X[1], (const float*)c->X[2], (const double*)c->U[0],
-                                                            (const double*)c->U[1], (const double*)c->U[2], c->slot_tmp, (const double*)c->x0,
-                                                            (float*)c->tk_xnom, (double*)c->tk_unom, (double*)c->tk_xnom0, c->N, c->Np, c->TT, tchunk);
-    else
-        k_track_nominal<double><<<grid, 128, 0, c->stream>>>((const double*)c->X[0], (const double*)c->X[1], (const double*)c->X[2],
-                                                             (const double*)c->U[0], (const double*)c->U[1], (const double*)c->U[2], c->slot_tmp,
-                                                             (const double*)c->x0, (double*)c->tk_xnom, (double*)c->tk_unom, (double*)c->tk_xnom0,
-                                                             c->N, c->Np, c->TT, tchunk);
+    with_real(xf, [&](auto T) {
+        using XT = typename decltype(T)::type;
+        k_track_nominal<XT><<<grid, 128, 0, c->stream>>>((const XT*)c->X[0], (const XT*)c->X[1], (const XT*)c->X[2], (const double*)c->U[0],
+                                                         (const double*)c->U[1], (const double*)c->U[2], c->slot_tmp, (const double*)c->x0,
+                                                         (XT*)c->tk_xnom, (double*)c->tk_unom, (double*)c->tk_xnom0, c->N, c->Np, c->TT, tchunk);
+        return 0;
+    });
     CK(cudaGetLastError());
     return 0;
 }

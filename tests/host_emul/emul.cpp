@@ -15,7 +15,7 @@
 using namespace acoc;
 
 namespace {
-// dispatch on the runtime state-quantisation flag like LAUNCH_Q32 in acoc_api.cu
+// dispatch on the runtime state-quantisation flag like the kernel launches in acoc_api.cu (with_flag)
 template <bool WRITE, bool COST, typename F, typename XT>
 double rollout_q(const ProblemT<F>& P, const F* U, const F* DU, double s, XT* Xn, F* Un, int i)
 {
