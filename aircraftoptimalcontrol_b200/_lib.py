@@ -102,6 +102,12 @@ def _sig(lib):
         "acoc_measure_fp64_peak": [i, vp],
         "acoc_measure_copy_bw": [i, vp],
         "acoc_measure_fp64_latency": [i, vp],
+        "acoc_set_refs_dev": [vp] * 4,
+        "acoc_set_init_dev": [vp] * 4,
+        "acoc_get_result_dev": [vp, vp, i, vp, vp, vp],
+        "acoc_get_tracked_dev": [vp] * 4,
+        "acoc_get_track_gains_dev": [vp] * 3,
+        "acoc_track_mc_dev": [vp] * 4 + [i, vp, i, vp, vp, vp],
     }
     for name, args in table.items():
         fn = getattr(lib, name)
@@ -153,6 +159,29 @@ def out_array(a, shape, dtypes, name="out"):
     if not a.flags["C_CONTIGUOUS"] or not a.flags["WRITEABLE"]:
         raise ValueError("%s must be C-contiguous and writeable" % name)
     return a
+
+
+def dev_tensor(t, device, shape, dtype, name="tensor"):
+    """Address of a caller's CUDA tensor before it crosses the C boundary of a _dev entry point (the library reads or writes
+    prod(shape) elements of `dtype` there): a torch.Tensor of `dtype` with exactly `shape`, contiguous, on cuda:`device`."""
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise ValueError("%s must be a torch.Tensor, got %s" % (name, type(t).__name__))
+    if t.dtype != dtype:
+        raise ValueError("%s has dtype %s, expected %s" % (name, t.dtype, dtype))
+    if tuple(t.shape) != tuple(shape):
+        raise ValueError("%s has shape %s, expected %s" % (name, tuple(t.shape), tuple(shape)))
+    if not t.is_contiguous():
+        raise ValueError("%s must be contiguous" % name)
+    if not t.is_cuda or t.device.index != device:
+        raise ValueError("%s is on %s, expected cuda:%d" % (name, t.device, device))
+    return t.data_ptr()
+
+
+def dev_stream(device):
+    """The current torch stream of cuda:`device` as the stream argument of a _dev entry point."""
+    import torch
+    return torch.cuda.current_stream(device).cuda_stream
 
 
 def f64(a, shape=None, name="array"):

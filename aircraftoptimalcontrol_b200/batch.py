@@ -350,6 +350,87 @@ class BatchedNewton:
         L.check(L.lib().acoc_get_track_timing(self._h, C.addressof(ms)))
         return dict(total_ms=ms[0], nominal_ms=ms[1], gains_ms=ms[2], rollout_ms=ms[3])
 
+    # -- device-resident inputs and outputs (include/acoc.h): CUDA tensors of this context's device, no host round trip ------------
+    # Each method is the twin of the method without _dev (same shapes, state rules, refusals and bit-identical results).  Tensors
+    # must be contiguous and of the exact shape and dtype; the call is ordered after the work queued so far on the current torch
+    # stream of the device and returns once its outputs are written, so they may be used on any stream.
+    def set_refs_dev(self, xx_ref, uu_ref):
+        """set_refs from float64 CUDA tensors xx_ref (N,6,TT) / uu_ref (N,2,TT), or (6,TT) / (2,TT) with refs_shared."""
+        import torch
+        sx = (6, self.TT) if self.refs_shared else (self.N, 6, self.TT)
+        su = (2, self.TT) if self.refs_shared else (self.N, 2, self.TT)
+        xr = L.dev_tensor(xx_ref, self.device, sx, torch.float64, "xx_ref")
+        ur = L.dev_tensor(uu_ref, self.device, su, torch.float64, "uu_ref")
+        L.check(L.lib().acoc_set_refs_dev(self._h, xr, ur, L.dev_stream(self.device)))
+
+    def set_init_dev(self, xx_init, uu_init):
+        """set_init from float64 CUDA tensors xx_init (N,6,TT) / uu_init (N,2,TT)."""
+        import torch
+        xi = L.dev_tensor(xx_init, self.device, (self.N, 6, self.TT), torch.float64, "xx_init")
+        ui = L.dev_tensor(uu_init, self.device, (self.N, 2, self.TT), torch.float64, "uu_init")
+        L.check(L.lib().acoc_set_init_dev(self._h, xi, ui, L.dev_stream(self.device)))
+
+    def result_dev(self, x_dtype=None, out=None):
+        """(xx_star (N,6,TT), uu_star (N,2,TT) float64, x0 (N,6) float64) as CUDA tensors: result() with x_dtype=torch.float64 (default),
+        result_f32() with torch.float32 (refused for float64-state contexts).  x0 is the exact initial state either way.
+        out = (xx_star, uu_star) tensors to write into."""
+        import torch
+        x_dtype = torch.float64 if x_dtype is None else x_dtype
+        if x_dtype not in (torch.float32, torch.float64):
+            raise ValueError("x_dtype must be torch.float32 or torch.float64")
+        dev = torch.device("cuda", self.device)
+        if out is None:
+            xs = torch.empty((self.N, 6, self.TT), dtype=x_dtype, device=dev)
+            us = torch.empty((self.N, 2, self.TT), dtype=torch.float64, device=dev)
+        else:
+            xs, us = out
+        x0 = torch.empty((self.N, 6), dtype=torch.float64, device=dev)
+        px = L.dev_tensor(xs, self.device, (self.N, 6, self.TT), x_dtype, "xx_star")
+        pu = L.dev_tensor(us, self.device, (self.N, 2, self.TT), torch.float64, "uu_star")
+        L.check(L.lib().acoc_get_result_dev(self._h, px, int(x_dtype == torch.float32), pu, x0.data_ptr(), L.dev_stream(self.device)))
+        return xs, us, x0
+
+    def tracked_dev(self, out=None):
+        """tracked() as float64 CUDA tensors (xx_reg (N,6,TT), uu_reg (N,2,TT)); out = such tensors to write into."""
+        import torch
+        if out is None:
+            dev = torch.device("cuda", self.device)
+            out = (torch.empty((self.N, 6, self.TT), dtype=torch.float64, device=dev),
+                   torch.empty((self.N, 2, self.TT), dtype=torch.float64, device=dev))
+        xr, ur = out
+        px = L.dev_tensor(xr, self.device, (self.N, 6, self.TT), torch.float64, "xx_reg")
+        pu = L.dev_tensor(ur, self.device, (self.N, 2, self.TT), torch.float64, "uu_reg")
+        L.check(L.lib().acoc_get_tracked_dev(self._h, px, pu, L.dev_stream(self.device)))
+        return xr, ur
+
+    def track_gains_dev(self, out=None):
+        """track_gains() as a float64 CUDA tensor K (N,2,6,TT); out = such a tensor to write into."""
+        import torch
+        K = torch.empty((self.N, 2, 6, self.TT), dtype=torch.float64, device=torch.device("cuda", self.device)) if out is None else out
+        pk = L.dev_tensor(K, self.device, (self.N, 2, 6, self.TT), torch.float64, "K")
+        L.check(L.lib().acoc_get_track_gains_dev(self._h, pk, L.dev_stream(self.device)))
+        return K
+
+    def track_mc_dev(self, delta, QQt=None, RRt=None, QQT=None, tol=None, per_sample=False):
+        """track_mc() with the perturbations and every output as CUDA tensors: delta a float64 tensor (M,6) (shared by every instance)
+        or (N,M,6); returns track_mc's dict with float64 / int32 tensors in place of arrays.  The weights and tol are host arrays."""
+        import torch
+        from .lqr_tracking import default_weights, mc_call, mc_layout
+        dQ, dR, dQT = default_weights()
+        Q = L.f64(dQ if QQt is None else QQt, (6, 6), "QQt")
+        R = L.f64(dR if RRt is None else RRt, (2, 2), "RRt")
+        QT = L.f64(dQT if QQT is None else QQT, (6, 6), "QQT")
+        if not isinstance(delta, torch.Tensor):
+            raise ValueError("delta must be a torch.Tensor, got %s" % type(delta).__name__)
+        shared, M = mc_layout(delta.shape, self.N)
+        d = L.dev_tensor(delta, self.device, delta.shape, torch.float64, "delta")
+        dev, stream = torch.device("cuda", self.device), L.dev_stream(self.device)
+
+        def empty(shape, integer):
+            return torch.empty(shape, dtype=torch.int32 if integer else torch.float64, device=dev)
+        return mc_call(lambda t, out: L.lib().acoc_track_mc_dev(self._h, L.ptr(Q), L.ptr(R), L.ptr(QT), M, d, int(shared), t, out, stream),
+                       self.N, M, tol, per_sample, empty)
+
     def set_profiling(self, on=True):
         L.check(L.lib().acoc_set_profiling(self._h, int(bool(on))))
 

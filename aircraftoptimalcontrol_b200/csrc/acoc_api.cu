@@ -24,6 +24,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <initializer_list>
 #include <mutex>
 #include <string>
 #include <type_traits>
@@ -671,6 +672,16 @@ __global__ void k_from_soa(const D* __restrict__ s0, const D* __restrict__ s1, c
     }
 }
 
+// per-instance rows [rows][Np] of S -> a caller's device array (N, rows) of T: the summaries, counts and x0 of the _dev read-backs
+template <typename S, typename T>
+__global__ void k_rows_out(const S* __restrict__ src, T* __restrict__ dst, int N, int Np, int rows)
+{
+    const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= (long long)N * rows) return;
+    const int i = (int)(e / rows), k = (int)(e % rows);
+    dst[e] = (T)src[(size_t)k * Np + i];
+}
+
 // ---- result delivery straight into page-locked host memory ----------------------------------------------------------------------
 // What optimize() returns (optcon.py:503-505) for every instance of this context whose status is FINAL, written into the caller's
 // (N, C, TT) array at row uidx[n] (the instance's index in the caller's batch; NULL: identity) by the layout-conversion kernel itself:
@@ -975,6 +986,7 @@ struct acoc_ctx {
     size_t mc_sum_cap = 0, mc_delta_cap = 0;
     cudaEvent_t tk_ev[4] = {};
     double tk_ms[4] = {0, 0, 0, 0};
+    cudaEvent_t ev_caller = nullptr;  // the caller's stream -> the context's stream (_dev entry points), created on first use
 };
 
 static int dalloc_bytes(acoc_ctx* c, void** p, size_t bytes)
@@ -1107,59 +1119,140 @@ static int reset_state(acoc_ctx* c)
     return 0;
 }
 
-// host (n,C,TT) float64 -> SoA of D, chunked through the staging buffer.  row0 / inexact: see k_to_soa.
+// Layout conversion between the caller's (n,C,TT) arrays and the context's SoA buffers.  A host array goes through the staging buffer
+// in chunks, each followed by a synchronisation (the buffer is reused by the next chunk).  A device array of the context's device
+// (`dev`, the _dev entry points) is read or written by the conversion kernel itself: no staging, no copy, no synchronisation; it is
+// split only where a launch would exceed the grid's y limit.
+constexpr int CONV_MAX_ROWS = 65535 * 32;  // instances of one k_to_soa / k_from_soa launch (grid.y = ceil(n/32) <= 65535)
+
+// (n,C,TT) float64 -> SoA of D.  row0 / inexact: see k_to_soa.
 template <typename D, typename R0>
-static int upload_soa_t(acoc_ctx* c, const double* host, void* dst, int n, int C, int Np, R0* row0, int* inexact)
+static int upload_soa_t(acoc_ctx* c, const double* src, void* dst, int n, int C, int Np, R0* row0, int* inexact, bool dev = false)
 {
     const int TT = c->TT;
     const size_t per = (size_t)C * TT;
-    int chunk = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, c->stage_doubles / per));
+    const int chunk = dev ? std::min(n, CONV_MAX_ROWS)
+                          : (int)std::min<size_t>((size_t)n, std::max<size_t>(1, c->stage_doubles / per));
     for (int n0 = 0; n0 < n; n0 += chunk) {
         const int nc = std::min(chunk, n - n0);
-        CK(cudaMemcpyAsync(c->stage, host + (size_t)n0 * per, (size_t)nc * per * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+        const double* s = src + (size_t)n0 * per;
+        if (!dev) {
+            CK(cudaMemcpyAsync(c->stage, s, (size_t)nc * per * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+            s = c->stage;
+        }
         dim3 grid((TT + 31) / 32, (nc + 31) / 32, C), block(32, 8);
-        k_to_soa<D, R0><<<grid, block, 0, c->stream>>>(c->stage, (D*)dst, n0, nc, C, TT, Np, row0, inexact);
+        k_to_soa<D, R0><<<grid, block, 0, c->stream>>>(s, (D*)dst, n0, nc, C, TT, Np, row0, inexact);
         CK(cudaGetLastError());
-        CK(cudaStreamSynchronize(c->stream));  // the staging buffer is reused by the next chunk
+        if (!dev) CK(cudaStreamSynchronize(c->stream));  // the staging buffer is reused by the next chunk
     }
     return 0;
 }
 // buffers of the context's arithmetic type F (inputs, references, gains)
-static int upload_soa(acoc_ctx* c, const double* host, void* dst, int n, int C, int Np)
+static int upload_soa(acoc_ctx* c, const double* src, void* dst, int n, int C, int Np, bool dev = false)
 {
-    return c->fp32 ? upload_soa_t<float, float>(c, host, dst, n, C, Np, nullptr, nullptr)
-                   : upload_soa_t<double, double>(c, host, dst, n, C, Np, nullptr, nullptr);
+    return c->fp32 ? upload_soa_t<float, float>(c, src, dst, n, C, Np, nullptr, nullptr, dev)
+                   : upload_soa_t<double, double>(c, src, dst, n, C, Np, nullptr, nullptr, dev);
 }
 
 template <typename D, typename O = double>
-static int download_soa_t(acoc_ctx* c, const void* s0, const void* s1, const void* s2, const int* slot, const double* row0, O* host, int n,
-                          int C, int Np, int dup_last)
+static int download_soa_t(acoc_ctx* c, const void* s0, const void* s1, const void* s2, const int* slot, const double* row0, O* out, int n,
+                          int C, int Np, int dup_last, bool dev = false)
 {
     const int TT = c->TT;
     const size_t per = (size_t)C * TT;
-    int chunk = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, c->stage_doubles * (sizeof(double) / sizeof(O)) / per));
+    const int chunk = dev ? std::min(n, CONV_MAX_ROWS)
+                          : (int)std::min<size_t>((size_t)n, std::max<size_t>(1, c->stage_doubles * (sizeof(double) / sizeof(O)) / per));
     for (int n0 = 0; n0 < n; n0 += chunk) {
         const int nc = std::min(chunk, n - n0);
         dim3 grid((TT + 31) / 32, (nc + 31) / 32, C), block(32, 8);
-        k_from_soa<D, O><<<grid, block, 0, c->stream>>>((const D*)s0, (const D*)s1, (const D*)s2, slot, row0, (O*)c->stage, n0, nc, C, TT, Np, dup_last);
+        O* d = dev ? out + (size_t)n0 * per : (O*)c->stage;
+        k_from_soa<D, O><<<grid, block, 0, c->stream>>>((const D*)s0, (const D*)s1, (const D*)s2, slot, row0, d, n0, nc, C, TT, Np, dup_last);
         CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(host + (size_t)n0 * per, c->stage, (size_t)nc * per * sizeof(O), cudaMemcpyDeviceToHost, c->stream));
+        if (dev) continue;
+        CK(cudaMemcpyAsync(out + (size_t)n0 * per, c->stage, (size_t)nc * per * sizeof(O), cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
     }
     return 0;
 }
 // buffers of type F
-static int download_soa(acoc_ctx* c, const void* s0, const void* s1, const void* s2, const int* slot, double* host, int n, int C, int Np,
-                        int dup_last)
+static int download_soa(acoc_ctx* c, const void* s0, const void* s1, const void* s2, const int* slot, double* out, int n, int C, int Np,
+                        int dup_last, bool dev = false)
 {
-    return c->fp32 ? download_soa_t<float>(c, s0, s1, s2, slot, nullptr, host, n, C, Np, dup_last)
-                   : download_soa_t<double>(c, s0, s1, s2, slot, nullptr, host, n, C, Np, dup_last);
+    return c->fp32 ? download_soa_t<float>(c, s0, s1, s2, slot, nullptr, out, n, C, Np, dup_last, dev)
+                   : download_soa_t<double>(c, s0, s1, s2, slot, nullptr, out, n, C, Np, dup_last, dev);
 }
 // state slots (element type by x_float; exact t = 0 column from x0 when the slots are float but the arithmetic is float64)
-static int download_x(acoc_ctx* c, const int* slot, double* host)
+static int download_x(acoc_ctx* c, const int* slot, double* out, bool dev = false)
 {
-    if (!c->x_float) return download_soa_t<double>(c, c->X[0], c->X[1], c->X[2], slot, nullptr, host, c->N, 6, c->Np, 0);
-    return download_soa_t<float>(c, c->X[0], c->X[1], c->X[2], slot, c->fp32 ? nullptr : (const double*)c->x0, host, c->N, 6, c->Np, 0);
+    if (!c->x_float) return download_soa_t<double>(c, c->X[0], c->X[1], c->X[2], slot, nullptr, out, c->N, 6, c->Np, 0, dev);
+    return download_soa_t<float>(c, c->X[0], c->X[1], c->X[2], slot, c->fp32 ? nullptr : (const double*)c->x0, out, c->N, 6, c->Np, 0, dev);
+}
+
+// device [rows][Np] of S -> (N,rows) of T (per-instance summaries, counts, x0): into host memory through one copy and a loop, or into
+// device memory of the context's device (dev) by k_rows_out
+template <typename T, typename S = T>
+static int download_rows(acoc_ctx* c, const void* src, T* dst, int rows, bool dev = false)
+{
+    if (!dst) return 0;
+    if (dev) {
+        const long long n = (long long)c->N * rows;
+        k_rows_out<S, T><<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>((const S*)src, dst, c->N, c->Np, rows);
+        CK(cudaGetLastError());
+        return 0;
+    }
+    std::vector<S> tmp((size_t)rows * c->Np);
+    CK(cudaMemcpyAsync(tmp.data(), src, tmp.size() * sizeof(S), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    for (int i = 0; i < c->N; ++i) for (int k = 0; k < rows; ++k) dst[(size_t)i * rows + k] = (T)tmp[(size_t)k * c->Np + i];
+    return 0;
+}
+
+// ---- the _dev entry points (acoc.h "device-resident inputs and outputs") ---------------------------------------------------------
+// A _dev argument must be device (or managed) memory of the context's device: a host address handed to a conversion kernel would
+// fault on the device instead of failing here.  NULL passes (optional arguments are checked by the twin).
+static int check_dev_ptr(const acoc_ctx* c, const void* p, const char* fn, const char* name)
+{
+    if (!p) return 0;
+    cudaPointerAttributes a;
+    const cudaError_t e = cudaPointerGetAttributes(&a, p);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(ACOC_ERR_INVALID, "%s: %s is not a CUDA-visible address (%s)", fn, name, cudaGetErrorString(e));
+    }
+    const bool device_mem = a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+    if (!device_mem || a.device != c->device)
+        return fail(ACOC_ERR_INVALID, "%s: %s must be device memory of device %d, got %s%s", fn, name, c->device,
+                    a.type == cudaMemoryTypeHost ? "page-locked host memory"
+                    : a.type == cudaMemoryTypeUnregistered ? "pageable host memory" : "memory of device ",
+                    device_mem ? std::to_string(a.device).c_str() : "");
+    return 0;
+}
+
+// make the context's stream wait for the work queued so far on the caller's stream (NULL: the legacy default stream)
+static int wait_caller_stream(acoc_ctx* c, void* stream)
+{
+    if (!c->ev_caller) CK(cudaEventCreateWithFlags(&c->ev_caller, cudaEventDisableTiming));
+    CK(cudaEventRecord(c->ev_caller, stream ? (cudaStream_t)stream : cudaStreamLegacy));
+    CK(cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
+    return 0;
+}
+
+// the common start of a _dev entry point: the context, its device, every pointer argument, then the stream order
+static int dev_begin(acoc_ctx* c, void* stream, const char* fn, std::initializer_list<std::pair<const void*, const char*>> ptrs)
+{
+    if (!c) return fail(ACOC_ERR_INVALID, "%s: ctx is NULL", fn);
+    TRY(use_device(c->device));
+    for (const auto& p : ptrs) TRY(check_dev_ptr(c, p.first, fn, p.second));
+    return wait_caller_stream(c, stream);
+}
+
+// the end of a _dev entry point: the twin's status, after the context's stream has finished reading and writing the caller's arrays
+static int dev_end(acoc_ctx* c, int rc)
+{
+    const cudaError_t e = cudaStreamSynchronize(c->stream);
+    if (rc) return rc;
+    if (e != cudaSuccess) { cudaGetLastError(); return fail(ACOC_ERR_CUDA, "cudaStreamSynchronize failed: %s", cudaGetErrorString(e)); }
+    return 0;
 }
 
 static bool is_diag(const double* M, int n)
@@ -1447,6 +1540,7 @@ int acoc_ctx_destroy(acoc_ctx* c)
     if (c->dstream) { cudaStreamSynchronize(c->dstream); cudaStreamDestroy(c->dstream); }
     if (c->ev_deliver) cudaEventDestroy(c->ev_deliver);
     for (auto& e : c->tk_ev) if (e) cudaEventDestroy(e);
+    if (c->ev_caller) cudaEventDestroy(c->ev_caller);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
     return 0;
@@ -1490,20 +1584,29 @@ int acoc_set_options(acoc_ctx* c, const acoc_newton_options* o)
     return reset_state(c);
 }
 
-int acoc_set_refs(acoc_ctx* c, const double* xx_ref, const double* uu_ref)
+// acoc_set_refs (dev = false) and acoc_set_refs_dev
+static int set_refs(acoc_ctx* c, const double* xx_ref, const double* uu_ref, bool dev)
 {
     REQUIRE(c && xx_ref && uu_ref, "NULL argument");
     TRY(use_device(c->device));
     if (c->P.ref_shared) {
-        TRY(upload_soa(c, xx_ref, c->xref, 1, 6, 1));
-        TRY(upload_soa(c, uu_ref, c->uref, 1, 2, 1));
+        TRY(upload_soa(c, xx_ref, c->xref, 1, 6, 1, dev));
+        TRY(upload_soa(c, uu_ref, c->uref, 1, 2, 1, dev));
     } else {
-        TRY(upload_soa(c, xx_ref, c->xref, c->N, 6, c->Np));
-        TRY(upload_soa(c, uu_ref, c->uref, c->N, 2, c->Np));
+        TRY(upload_soa(c, xx_ref, c->xref, c->N, 6, c->Np, dev));
+        TRY(upload_soa(c, uu_ref, c->uref, c->N, 2, c->Np, dev));
     }
     c->P.ref_param = 0;
     c->have_refs = true;
     return 0;
+}
+
+int acoc_set_refs(acoc_ctx* c, const double* xx_ref, const double* uu_ref) { return set_refs(c, xx_ref, uu_ref, false); }
+
+int acoc_set_refs_dev(acoc_ctx* c, const double* xx_ref_dev, const double* uu_ref_dev, void* stream)
+{
+    TRY(dev_begin(c, stream, "acoc_set_refs_dev", {{xx_ref_dev, "xx_ref_dev"}, {uu_ref_dev, "uu_ref_dev"}}));
+    return dev_end(c, set_refs(c, xx_ref_dev, uu_ref_dev, true));
 }
 
 // device buffers of the parametric references (allocated on first use: tables, per-instance parameters, speed reference)
@@ -1567,32 +1670,41 @@ int acoc_set_refs_generated(acoc_ctx* c, const double* tt, const double* zshape,
     return 0;
 }
 
-int acoc_set_init(acoc_ctx* c, const double* xx_init, const double* uu_init)
+// acoc_set_init (dev = false) and acoc_set_init_dev
+static int set_init(acoc_ctx* c, const double* xx_init, const double* uu_init, bool dev)
 {
     REQUIRE(c && xx_init && uu_init, "NULL argument");
     TRY(use_device(c->device));
     TRY(reset_state(c));
     // x0 = xx[:,0,0] (optcon.py:398) is taken from the t = 0 column during the upload
     if (c->fp32) {
-        TRY((upload_soa_t<float, float>(c, xx_init, c->X[0], c->N, 6, c->Np, (float*)c->x0, nullptr)));
+        TRY((upload_soa_t<float, float>(c, xx_init, c->X[0], c->N, 6, c->Np, (float*)c->x0, nullptr, dev)));
     } else {
         c->x_float = false;
         if (c->P.q32) {
             // float32-quantised states: a trajectory produced by the reference's get_initial_trajectory (or by any rollout of
             // Dynamics.step) consists of float32 values for t >= 1 and is stored as float; anything else keeps float64 slots
             CK(cudaMemsetAsync(c->counters + 3, 0, sizeof(int), c->stream));
-            TRY((upload_soa_t<float, double>(c, xx_init, c->X[0], c->N, 6, c->Np, (double*)c->x0, c->counters + 3)));
+            TRY((upload_soa_t<float, double>(c, xx_init, c->X[0], c->N, 6, c->Np, (double*)c->x0, c->counters + 3, dev)));
             int inexact = 0;
             CK(cudaMemcpyAsync(&inexact, c->counters + 3, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
             CK(cudaStreamSynchronize(c->stream));
             c->x_float = !inexact && !(c->flags & ACOC_X_F64);
         }
-        if (!c->x_float) TRY((upload_soa_t<double, double>(c, xx_init, c->X[0], c->N, 6, c->Np, (double*)c->x0, nullptr)));
+        if (!c->x_float) TRY((upload_soa_t<double, double>(c, xx_init, c->X[0], c->N, 6, c->Np, (double*)c->x0, nullptr, dev)));
     }
-    TRY(upload_soa(c, uu_init, c->U[0], c->N, 2, c->Np));
+    TRY(upload_soa(c, uu_init, c->U[0], c->N, 2, c->Np, dev));
     CK(cudaStreamSynchronize(c->stream));
     c->have_init = true;
     return 0;
+}
+
+int acoc_set_init(acoc_ctx* c, const double* xx_init, const double* uu_init) { return set_init(c, xx_init, uu_init, false); }
+
+int acoc_set_init_dev(acoc_ctx* c, const double* xx_init_dev, const double* uu_init_dev, void* stream)
+{
+    TRY(dev_begin(c, stream, "acoc_set_init_dev", {{xx_init_dev, "xx_init_dev"}, {uu_init_dev, "uu_init_dev"}}));
+    return dev_end(c, set_init(c, xx_init_dev, uu_init_dev, true));
 }
 
 template <typename F, typename XT>
@@ -2732,16 +2844,19 @@ int acoc_set_scalars(acoc_ctx* c, const double* J, const double* descent)
 // ======================================================================================================
 // read-back
 // ======================================================================================================
-int acoc_get_result(acoc_ctx* c, double* xx_star, double* uu_star)
+// acoc_get_result (dev = false) and acoc_get_result_dev with x_is_f32 = 0
+static int get_result(acoc_ctx* c, double* xx_star, double* uu_star, bool dev)
 {
     TRY(ready(c));
     REQUIRE(xx_star && uu_star, "NULL output");
     k_result_slot_default<<<(c->N + 255) / 256, 256, 0, c->stream>>>(c->S.status, c->slot_tmp, c->S.result_slot, c->kk % 3, c->N);
     CK(cudaGetLastError());
-    TRY(download_x(c, c->slot_tmp, xx_star));
-    TRY(download_soa(c, c->U[0], c->U[1], c->U[2], c->slot_tmp, uu_star, c->N, 2, c->Np, 1));  // uu_star[:,-1] = uu_star[:,-2], optcon.py:505
+    TRY(download_x(c, c->slot_tmp, xx_star, dev));
+    TRY(download_soa(c, c->U[0], c->U[1], c->U[2], c->slot_tmp, uu_star, c->N, 2, c->Np, 1, dev));  // uu_star[:,-1] = uu_star[:,-2], optcon.py:505
     return 0;
 }
+
+int acoc_get_result(acoc_ctx* c, double* xx_star, double* uu_star) { return get_result(c, xx_star, uu_star, false); }
 
 int acoc_get_refs(acoc_ctx* c, double* xx_ref, double* uu_ref)
 {
@@ -2759,7 +2874,14 @@ int acoc_get_refs(acoc_ctx* c, double* xx_ref, double* uu_ref)
     return 0;
 }
 
-int acoc_get_result_f32(acoc_ctx* c, float* xx_star, double* uu_star, double* x0)
+// the exact x0 (x0 buffer [6][Np], float64 unless the context computes in FP32) -> (N,6) float64
+static int download_x0(acoc_ctx* c, double* x0, bool dev)
+{
+    return c->fp32 ? download_rows<double, float>(c, c->x0, x0, 6, dev) : download_rows<double>(c, c->x0, x0, 6, dev);
+}
+
+// acoc_get_result_f32 (dev = false) and acoc_get_result_dev with x_is_f32 = 1
+static int get_result_f32(acoc_ctx* c, float* xx_star, double* uu_star, double* x0, bool dev)
 {
     TRY(ready(c));
     REQUIRE(xx_star && uu_star, "NULL output");
@@ -2768,23 +2890,20 @@ int acoc_get_result_f32(acoc_ctx* c, float* xx_star, double* uu_star, double* x0
                                     "ACOC_X_F64 or an initial trajectory with float64 states); use acoc_get_result");
     k_result_slot_default<<<(c->N + 255) / 256, 256, 0, c->stream>>>(c->S.status, c->slot_tmp, c->S.result_slot, c->kk % 3, c->N);
     CK(cudaGetLastError());
-    TRY((download_soa_t<float, float>(c, c->X[0], c->X[1], c->X[2], c->slot_tmp, nullptr, xx_star, c->N, 6, c->Np, 0)));
-    TRY(download_soa(c, c->U[0], c->U[1], c->U[2], c->slot_tmp, uu_star, c->N, 2, c->Np, 1));  // uu_star[:,-1] = uu_star[:,-2], optcon.py:505
-    if (x0) {  // device [6][Np] -> host (N,6); float64 unless the context computes in FP32
-        const size_t Np = c->Np;
-        if (c->fp32) {
-            std::vector<float> tmp(6 * Np);
-            CK(cudaMemcpyAsync(tmp.data(), c->x0, tmp.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-            CK(cudaStreamSynchronize(c->stream));
-            for (int i = 0; i < c->N; ++i) for (int k = 0; k < 6; ++k) x0[(size_t)i * 6 + k] = tmp[k * Np + i];
-        } else {
-            std::vector<double> tmp(6 * Np);
-            CK(cudaMemcpyAsync(tmp.data(), c->x0, tmp.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-            CK(cudaStreamSynchronize(c->stream));
-            for (int i = 0; i < c->N; ++i) for (int k = 0; k < 6; ++k) x0[(size_t)i * 6 + k] = tmp[k * Np + i];
-        }
-    }
-    return 0;
+    TRY((download_soa_t<float, float>(c, c->X[0], c->X[1], c->X[2], c->slot_tmp, nullptr, xx_star, c->N, 6, c->Np, 0, dev)));
+    TRY(download_soa(c, c->U[0], c->U[1], c->U[2], c->slot_tmp, uu_star, c->N, 2, c->Np, 1, dev));  // uu_star[:,-1] = uu_star[:,-2], optcon.py:505
+    return download_x0(c, x0, dev);
+}
+
+int acoc_get_result_f32(acoc_ctx* c, float* xx_star, double* uu_star, double* x0) { return get_result_f32(c, xx_star, uu_star, x0, false); }
+
+int acoc_get_result_dev(acoc_ctx* c, void* xx_star_dev, int x_is_f32, double* uu_star_dev, double* x0_dev, void* stream)
+{
+    TRY(dev_begin(c, stream, "acoc_get_result_dev", {{xx_star_dev, "xx_star_dev"}, {uu_star_dev, "uu_star_dev"}, {x0_dev, "x0_dev"}}));
+    if (x_is_f32) return dev_end(c, get_result_f32(c, (float*)xx_star_dev, uu_star_dev, x0_dev, true));
+    int rc = get_result(c, (double*)xx_star_dev, uu_star_dev, true);
+    if (!rc) rc = download_x0(c, x0_dev, true);
+    return dev_end(c, rc);
 }
 
 int acoc_get_iterate(acoc_ctx* c, int which, double* xx, double* uu)
@@ -3137,26 +3256,14 @@ static int track_finish(acoc_ctx* c, bool xfloat, bool trajectories)
     return 0;
 }
 
-static int download_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg)
+static int download_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg, bool dev = false)
 {
     const double* row0 = (const double*)c->tk_x0;
     if (xx_reg) {
-        if (c->tk_xfloat) TRY((download_soa_t<float>(c, c->tk_x, nullptr, nullptr, nullptr, row0, xx_reg, c->N, NS, c->Np, 0)));
-        else TRY((download_soa_t<double>(c, c->tk_x, nullptr, nullptr, nullptr, row0, xx_reg, c->N, NS, c->Np, 0)));
+        if (c->tk_xfloat) TRY((download_soa_t<float>(c, c->tk_x, nullptr, nullptr, nullptr, row0, xx_reg, c->N, NS, c->Np, 0, dev)));
+        else TRY((download_soa_t<double>(c, c->tk_x, nullptr, nullptr, nullptr, row0, xx_reg, c->N, NS, c->Np, 0, dev)));
     }
-    if (uu_reg) TRY((download_soa_t<double>(c, c->tk_u, nullptr, nullptr, nullptr, nullptr, uu_reg, c->N, NI, c->Np, 0)));
-    return 0;
-}
-
-// device [6][Np] -> host (N,6)
-template <typename T>
-static int download_rows(acoc_ctx* c, const void* dev, T* host, int rows)
-{
-    if (!host) return 0;
-    std::vector<T> tmp((size_t)rows * c->Np);
-    CK(cudaMemcpyAsync(tmp.data(), dev, tmp.size() * sizeof(T), cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    for (int i = 0; i < c->N; ++i) for (int k = 0; k < rows; ++k) host[(size_t)i * rows + k] = tmp[(size_t)k * c->Np + i];
+    if (uu_reg) TRY((download_soa_t<double>(c, c->tk_u, nullptr, nullptr, nullptr, nullptr, uu_reg, c->N, NI, c->Np, 0, dev)));
     return 0;
 }
 
@@ -3206,25 +3313,27 @@ int acoc_track(acoc_ctx* c, const double* Q, const double* R, const double* QT, 
     return 0;
 }
 
-// the common part of acoc_track_mc and acoc_lqr_tracking_mc once the nominal is in place: deltas (one copy, as given), the sweeps, the
-// outputs
+// the common part of acoc_track_mc, acoc_track_mc_dev and acoc_lqr_tracking_mc once the nominal is in place: deltas (one copy, as
+// given), the sweeps, the outputs.  dev: delta and the outputs are device memory of the context's device.
 static int track_mc_run(acoc_ctx* c, bool xf, const Weights& W, int m, const double* delta, int delta_shared, const double* tol,
-                        acoc_track_mc_out* out)
+                        acoc_track_mc_out* out, bool dev = false)
 {
     const size_t per = (size_t)m * NS;
-    CK(cudaMemcpyAsync(c->mc_delta, delta, (delta_shared ? 1 : (size_t)c->N) * per * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaMemcpyAsync(c->mc_delta, delta, (delta_shared ? 1 : (size_t)c->N) * per * sizeof(double),
+                       dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, c->stream));
     const long long dstride = delta_shared ? 0 : (long long)per;
     TRY(xf ? launch_track_mc<float>(c, W, m, dstride, tol) : launch_track_mc<double>(c, W, m, dstride, tol));
     TRY(track_finish(c, xf, false));
     if (!out) return 0;
     const size_t bytes = (size_t)c->N * per * sizeof(double);
-    if (out->err_max) CK(cudaMemcpyAsync(out->err_max, c->mc_sum, bytes, cudaMemcpyDeviceToHost, c->stream));
-    if (out->err_final) CK(cudaMemcpyAsync(out->err_final, (const char*)c->mc_sum + bytes, bytes, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    TRY(download_rows(c, c->tk_emax, out->worst_max, NS));
-    TRY(download_rows(c, c->tk_efin, out->mean_final, NS));
-    if (tol) TRY(download_rows(c, c->mc_nw, out->n_within, 1));
-    TRY(download_rows(c, c->tk_nreg, out->n_reg, 1));
+    const cudaMemcpyKind kind = dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    if (out->err_max) CK(cudaMemcpyAsync(out->err_max, c->mc_sum, bytes, kind, c->stream));
+    if (out->err_final) CK(cudaMemcpyAsync(out->err_final, (const char*)c->mc_sum + bytes, bytes, kind, c->stream));
+    if (!dev) CK(cudaStreamSynchronize(c->stream));
+    TRY(download_rows(c, c->tk_emax, out->worst_max, NS, dev));
+    TRY(download_rows(c, c->tk_efin, out->mean_final, NS, dev));
+    if (tol) TRY(download_rows(c, c->mc_nw, out->n_within, 1, dev));
+    TRY(download_rows(c, c->tk_nreg, out->n_reg, 1, dev));
     return 0;
 }
 
@@ -3236,8 +3345,9 @@ static int track_mc_args(int m, const double* delta, const double* tol, acoc_tra
     return 0;
 }
 
-int acoc_track_mc(acoc_ctx* c, const double* Q, const double* R, const double* QT, int m, const double* delta, int delta_shared,
-                  const double* tol, acoc_track_mc_out* out)
+// acoc_track_mc (dev = false) and acoc_track_mc_dev
+static int track_mc(acoc_ctx* c, const double* Q, const double* R, const double* QT, int m, const double* delta, int delta_shared,
+                    const double* tol, acoc_track_mc_out* out, bool dev)
 {
     TRY(track_ctx_check(c, "acoc_track_mc"));
     TRY(track_mc_args(m, delta, tol, out, "acoc_track_mc"));
@@ -3250,24 +3360,59 @@ int acoc_track_mc(acoc_ctx* c, const double* Q, const double* R, const double* Q
     TRY(ensure_track_buffers(c, xf ? sizeof(float) : sizeof(double)));
     c->tk_done = false;  // the nominal and gains buffers are about to change
     TRY(copy_track_nominal(c, xf));
-    return track_mc_run(c, xf, W, m, delta, delta_shared, tol, out);
+    return track_mc_run(c, xf, W, m, delta, delta_shared, tol, out, dev);
 }
 
-int acoc_get_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg)
+int acoc_track_mc(acoc_ctx* c, const double* Q, const double* R, const double* QT, int m, const double* delta, int delta_shared,
+                  const double* tol, acoc_track_mc_out* out)
+{
+    return track_mc(c, Q, R, QT, m, delta, delta_shared, tol, out, false);
+}
+
+int acoc_track_mc_dev(acoc_ctx* c, const double* Q, const double* R, const double* QT, int m, const double* delta_dev, int delta_shared,
+                      const double* tol, acoc_track_mc_out* out_dev, void* stream)
+{
+    const acoc_track_mc_out o = out_dev ? *out_dev : acoc_track_mc_out{};
+    TRY(dev_begin(c, stream, "acoc_track_mc_dev", {{delta_dev, "delta_dev"}, {o.err_max, "out_dev->err_max"},
+                                                   {o.err_final, "out_dev->err_final"}, {o.worst_max, "out_dev->worst_max"},
+                                                   {o.mean_final, "out_dev->mean_final"}, {o.n_within, "out_dev->n_within"},
+                                                   {o.n_reg, "out_dev->n_reg"}}));
+    return dev_end(c, track_mc(c, Q, R, QT, m, delta_dev, delta_shared, tol, out_dev, true));
+}
+
+// acoc_get_tracked (dev = false) and acoc_get_tracked_dev
+static int get_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg, bool dev)
 {
     REQUIRE(c, "ctx is NULL");
     if (!c->tk_done) return fail(ACOC_ERR_STATE, "acoc_get_tracked: call acoc_track first");
     TRY(use_device(c->device));
-    return download_tracked(c, xx_reg, uu_reg);
+    return download_tracked(c, xx_reg, uu_reg, dev);
 }
 
-int acoc_get_track_gains(acoc_ctx* c, double* K)
+int acoc_get_tracked(acoc_ctx* c, double* xx_reg, double* uu_reg) { return get_tracked(c, xx_reg, uu_reg, false); }
+
+int acoc_get_tracked_dev(acoc_ctx* c, double* xx_reg_dev, double* uu_reg_dev, void* stream)
+{
+    TRY(dev_begin(c, stream, "acoc_get_tracked_dev", {{xx_reg_dev, "xx_reg_dev"}, {uu_reg_dev, "uu_reg_dev"}}));
+    return dev_end(c, get_tracked(c, xx_reg_dev, uu_reg_dev, true));
+}
+
+// acoc_get_track_gains (dev = false) and acoc_get_track_gains_dev
+static int get_track_gains(acoc_ctx* c, double* K, bool dev)
 {
     REQUIRE(c && K, "NULL argument");
     if (!c->tk_swept) return fail(ACOC_ERR_STATE, "acoc_get_track_gains: call acoc_track or acoc_track_mc first");
     TRY(use_device(c->device));
     // Ktrk as a trajectory with 12 components downloads to (N,12,TT) = (N,2,6,TT)
-    return download_soa_t<double>(c, c->tk_K, nullptr, nullptr, nullptr, nullptr, K, c->N, 2 * NS, c->Np, 0);
+    return download_soa_t<double>(c, c->tk_K, nullptr, nullptr, nullptr, nullptr, K, c->N, 2 * NS, c->Np, 0, dev);
+}
+
+int acoc_get_track_gains(acoc_ctx* c, double* K) { return get_track_gains(c, K, false); }
+
+int acoc_get_track_gains_dev(acoc_ctx* c, double* K_dev, void* stream)
+{
+    TRY(dev_begin(c, stream, "acoc_get_track_gains_dev", {{K_dev, "K_dev"}}));
+    return dev_end(c, get_track_gains(c, K_dev, true));
 }
 
 int acoc_get_track_timing(acoc_ctx* c, double* ms)

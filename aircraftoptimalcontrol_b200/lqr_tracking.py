@@ -75,29 +75,44 @@ def lqr_tracking_many(xx_opt, uu_opt, delta, dyn=None, QQt=None, RRt=None, QQT=N
     return xr, ur
 
 
+def mc_layout(shape, N):
+    """(shared, M) of a dispersion study's perturbations of `shape`: (M,6) shared by all N instances or (N,M,6)."""
+    shape = tuple(shape)
+    if len(shape) == 2 and shape[1] == 6:
+        shared, M = True, shape[0]
+    elif len(shape) == 3 and shape[0] == N and shape[2] == 6:
+        shared, M = False, shape[1]
+    else:
+        raise ValueError("delta has shape %s, expected (M,6) or %s" % (shape, (N, "M", 6)))
+    if M < 1:
+        raise ValueError("delta holds no sample (M = 0)")
+    return shared, M
+
+
 def mc_deltas(delta, N):
     """Perturbations of a dispersion study: (M,6) shared by all N instances or (N,M,6) -> (contiguous float64 array, shared, M)."""
     d = np.asarray(delta, dtype=np.float64)
-    if d.ndim == 2 and d.shape[1] == 6:
-        shared, M = True, d.shape[0]
-    elif d.ndim == 3 and d.shape[0] == N and d.shape[2] == 6:
-        shared, M = False, d.shape[1]
-    else:
-        raise ValueError("delta has shape %s, expected (M,6) or %s" % (d.shape, (N, "M", 6)))
-    if M < 1:
-        raise ValueError("delta holds no sample (M = 0)")
+    shared, M = mc_layout(d.shape, N)
     return np.ascontiguousarray(d), shared, M
 
 
-def mc_call(call, N, M, tol, per_sample):
-    """Run acoc_track_mc / acoc_lqr_tracking_mc through call(tol_ptr, out_ptr) and collect its outputs as a dict."""
+def _np_empty(shape, integer):
+    return np.empty(shape, dtype=np.int32 if integer else np.float64)
+
+
+def mc_call(call, N, M, tol, per_sample, empty=_np_empty):
+    """Run acoc_track_mc / acoc_lqr_tracking_mc / acoc_track_mc_dev through call(tol_ptr, out_ptr) and collect its outputs as a dict.
+    empty(shape, integer) allocates each output: int32 or float64 numpy arrays (default) or CUDA tensors (track_mc_dev)."""
     t = None if tol is None else L.f64(tol, (6,), "tol")
-    res = dict(worst_max=np.empty((N, 6)), mean_final=np.empty((N, 6)), n_reg=np.empty(N, dtype=np.int32))
+    res = dict(worst_max=empty((N, 6), False), mean_final=empty((N, 6), False), n_reg=empty((N,), True))
     if t is not None:
-        res["n_within"] = np.empty(N, dtype=np.int32)
+        res["n_within"] = empty((N,), True)
     if per_sample:
-        res["err_max"], res["err_final"] = np.empty((N, M, 6)), np.empty((N, M, 6))
-    out = L.TrackMcOut(*(L.ptr(res.get(k)) for k in ("err_max", "err_final", "worst_max", "mean_final", "n_within", "n_reg")))
+        res["err_max"], res["err_final"] = empty((N, M, 6), False), empty((N, M, 6), False)
+
+    def addr(a):
+        return L.ptr(a) if a is None or isinstance(a, np.ndarray) else a.data_ptr()
+    out = L.TrackMcOut(*(addr(res.get(k)) for k in ("err_max", "err_final", "worst_max", "mean_final", "n_within", "n_reg")))
     L.check(call(L.ptr(t), C.addressof(out)))
     return res
 

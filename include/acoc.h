@@ -11,7 +11,8 @@
  *   - every function returns 0 on success and a negative acoc_status on failure; nothing throws or
  *     calls exit() across the boundary (the reference print()+exit()s on shape errors, optcon.py:585-596);
  *     acoc_last_error() returns a human-readable message for the calling thread.
- *   - all floating-point buffers are C-contiguous IEEE float64 HOST memory unless the name ends in _dev.
+ *   - all floating-point buffers are C-contiguous IEEE float64 HOST memory unless the name ends in _dev (CUDA memory of the
+ *     context's device, see "device-resident inputs and outputs").
  *   - host trajectory layout is the reference's: one instance is (6,TT) / (2,TT) component-major
  *     (xx[i*TT + t]); a batch adds a leading instance axis (N,6,TT) / (N,2,TT).
  *   - matrices are row-major; "A" means fx.T (A[i][j] = d f_i / d x_j), "B" means fu.T.
@@ -277,6 +278,30 @@ int acoc_track_mc(acoc_ctx* ctx, const double* Q, const double* R, const double*
 int acoc_lqr_tracking_mc(int device, int n, int m, int TT, const double* params, int state_f64, const double* Q, const double* R,
                          const double* QT, const double* xx_opt, const double* uu_opt, const double* delta, int delta_shared,
                          const double* tol, acoc_track_mc_out* out);
+
+/* ------------------------------------------ device-resident inputs and outputs --------------------------- */
+/* Twins of the calls of the same name without _dev for arrays that live in CUDA memory of the context's device (e.g. torch tensors):
+ * same shapes and layouts (float64 unless stated, C-contiguous), same state rules, same refusals, same effect on the context and
+ * bit-identical results.  Only the arrays whose size grows with TT or with the number of samples have such a twin; small inputs
+ * (weights, tol, dx0, acoc_track's delta) stay in host memory.  The context's sm_100a layout-conversion kernels read and write the
+ * caller's arrays directly: no staging buffer, no host copy.
+ *   - Every _dev pointer must be device (or managed) memory of the context's device; anything else (pageable or page-locked host
+ *     memory, another GPU) is refused with ACOC_ERR_INVALID before any work is queued, naming the argument.
+ *   - stream: the caller's CUDA stream (cudaStream_t; NULL = the legacy default stream).  The context's streams are non-blocking, so
+ *     a call first makes its stream wait for the work queued on `stream` so far (the writes of the inputs, earlier reads of the
+ *     outputs).  It returns once its outputs are written and its inputs read, like the host-array calls: the arrays may then be used
+ *     on any stream. */
+int acoc_set_refs_dev(acoc_ctx* ctx, const double* xx_ref_dev, const double* uu_ref_dev, void* stream);
+int acoc_set_init_dev(acoc_ctx* ctx, const double* xx_init_dev, const double* uu_init_dev, void* stream);
+/* x_is_f32 = 0: what acoc_get_result writes; x_is_f32 = 1: xx_star_dev is float32 and receives what acoc_get_result_f32 writes
+ * (refused in the same cases).  x0_dev (N,6) float64 or NULL: the exact x0, as acoc_get_result_f32 returns it. */
+int acoc_get_result_dev(acoc_ctx* ctx, void* xx_star_dev, int x_is_f32, double* uu_star_dev, double* x0_dev, void* stream);
+int acoc_get_tracked_dev(acoc_ctx* ctx, double* xx_reg_dev, double* uu_reg_dev, void* stream);
+int acoc_get_track_gains_dev(acoc_ctx* ctx, double* K_dev, void* stream);
+/* delta_dev (M,6) or (N,M,6) and every pointer of *out_dev in device memory: per-sample values (N,M,6), aggregates (N,6), counts (N)
+ * int32.  Q, R, QT and tol stay host arrays. */
+int acoc_track_mc_dev(acoc_ctx* ctx, const double* Q, const double* R, const double* QT, int m, const double* delta_dev, int delta_shared,
+                      const double* tol, acoc_track_mc_out* out_dev, void* stream);
 
 /* Single pieces of the loop on the context's current iterate, exposed for parity tests and for the
  * reference's own method names:
