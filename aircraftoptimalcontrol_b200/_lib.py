@@ -44,6 +44,12 @@ class TrackMcOut(C.Structure):
                 ("n_within", C.c_void_p), ("n_reg", C.c_void_p)]
 
 
+class VjpOut(C.Structure):
+    """acoc_vjp_out: output addresses (0 = not wanted)."""
+    _fields_ = [("xref_bar", C.c_void_p), ("uref_bar", C.c_void_p), ("x0_bar", C.c_void_p), ("zf_bar", C.c_void_p),
+                ("vx_bar", C.c_void_p), ("n_indef", C.c_void_p)]
+
+
 _dp = C.c_void_p  # double* / int* passed as raw addresses
 
 
@@ -108,6 +114,8 @@ def _sig(lib):
         "acoc_get_tracked_dev": [vp] * 4,
         "acoc_get_track_gains_dev": [vp] * 3,
         "acoc_track_mc_dev": [vp] * 4 + [i, vp, i, vp, vp, vp],
+        "acoc_result_vjp": [vp] * 4,
+        "acoc_result_vjp_dev": [vp] * 5,
     }
     for name, args in table.items():
         fn = getattr(lib, name)

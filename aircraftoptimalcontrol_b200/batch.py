@@ -46,6 +46,10 @@ class BatchedNewton:
     identical results, A/B measurements).
     """
 
+    version = 0          # bumped by every call that changes the context's problem or iterates (autograd checks it before backward)
+    _refs_param = False  # the context holds parametric references (result_vjp's zf / vx)
+    _refs_compact = True
+
     def __init__(self, n_instances, TT=1000, device=0, state="f32", refs_shared=False, armijo="speculative", params=None, generations=True,
                  max_iters=200, stepsize_0=1.0, cc=0.5, beta=0.7, armijo_maxiters=10, term_cond=-1e-6, exact_after=8, precision="f64",
                  x_storage="auto", tma=True, split=True, fused=True, method="newton", priority=0, refs_compact=True):
@@ -60,6 +64,7 @@ class BatchedNewton:
         if method not in ("newton", "gradient"):
             raise ValueError("method must be 'newton' or 'gradient'")
         self.method = method
+        self._refs_compact = bool(refs_compact) and precision == "f64"
         self.N, self.TT, self.device = int(n_instances), int(TT), int(device)
         self.refs_shared = bool(refs_shared)
         self.precision = precision
@@ -102,14 +107,18 @@ class BatchedNewton:
 
     # -- problem data ---------------------------------------------------------------------------------
     def set_model(self, params):
+        self.version += 1
         p = L.f64(params, (9,), "params")
         L.check(L.lib().acoc_set_model(self._h, L.ptr(p)))
 
     def set_weights(self, QQt, RRt, QQT):
+        self.version += 1
         Q, R, QT = L.f64(QQt, (6, 6), "QQt"), L.f64(RRt, (2, 2), "RRt"), L.f64(QQT, (6, 6), "QQT")
         L.check(L.lib().acoc_set_weights(self._h, L.ptr(Q), L.ptr(R), L.ptr(QT)))
 
     def set_refs(self, xx_ref, uu_ref):
+        self.version += 1
+        self._refs_param = False
         sx = (6, self.TT) if self.refs_shared else (self.N, 6, self.TT)
         su = (2, self.TT) if self.refs_shared else (self.N, 2, self.TT)
         xr, ur = L.f64(xx_ref, sx, "xx_ref"), L.f64(uu_ref, su, "uu_ref")
@@ -117,6 +126,8 @@ class BatchedNewton:
 
     def set_refs_generated(self, tt, zshape, vshape, zf, vx, xconst, uconst):
         """acoc_set_refs_generated: build the per-instance references on the device from per-instance (zf, vx) and shared time bases."""
+        self.version += 1
+        self._refs_param = self._refs_compact
         if self.refs_shared:
             raise ValueError("generated references are per instance (refs_shared=False)")
         tt, zs = L.f64(tt, (self.TT,), "tt"), L.f64(zshape, (self.TT,), "zshape")
@@ -150,22 +161,26 @@ class BatchedNewton:
         return xr, ur
 
     def set_init(self, xx_init, uu_init):
+        self.version += 1
         xi, ui = L.f64(xx_init, (self.N, 6, self.TT), "xx_init"), L.f64(uu_init, (self.N, 2, self.TT), "uu_init")
         L.check(L.lib().acoc_set_init(self._h, L.ptr(xi), L.ptr(ui)))
 
     def init_guess(self, kp=5.0, kt=2.5, dx0=None):
         """Dynamics.get_initial_trajectory (aircraft_simplified.py:126-148) for every instance, on the device.
         dx0 (N,6): start from xx_ref[:,0] + dx0 (perturbed-initial-state batches)."""
+        self.version += 1
         d = None if dx0 is None else L.f64(dx0, (self.N, 6), "dx0")
         L.check(L.lib().acoc_init_guess(self._h, float(kp), float(kt), L.ptr(d)))
 
     # -- solve ------------------------------------------------------------------------------------------
     def iterate(self, n_iters=1, count_active=True):
+        self.version += 1
         na = C.c_int(-1)
         L.check(L.lib().acoc_newton_iterate(self._h, int(n_iters), C.addressof(na) if count_active else None))
         return na.value
 
     def solve(self):
+        self.version += 1
         tot = C.c_longlong(0)
         L.check(L.lib().acoc_newton_solve(self._h, C.addressof(tot)))
         return tot.value
@@ -175,6 +190,7 @@ class BatchedNewton:
         With page-locked arrays (e.g. torch pin_memory) the results are written straight into them and the finished instances are
         delivered while the last ones still iterate (acoc_newton_solve_deliver); pageable arrays get the same values through
         solve() + result().  Returns (total Newton iterations, x0 (N,6))."""
+        self.version += 1
         xs, us = out
         L.out_array(xs, (self.N, 6, self.TT), (np.float32, np.float64), "xx_star")
         L.out_array(us, (self.N, 2, self.TT), np.float64, "uu_star")
@@ -216,10 +232,12 @@ class BatchedNewton:
         return costs
 
     def set_deltau(self, deltau):
+        self.version += 1
         du = L.f64(deltau, (self.N, 2, self.TT), "deltau")
         L.check(L.lib().acoc_set_deltau(self._h, L.ptr(du)))
 
     def set_scalars(self, J=None, descent=None):
+        self.version += 1
         Jc = None if J is None else L.f64(J, (self.N,), "J")
         dc = None if descent is None else L.f64(descent, (self.N,), "descent")
         L.check(L.lib().acoc_set_scalars(self._h, L.ptr(Jc), L.ptr(dc)))
@@ -230,6 +248,7 @@ class BatchedNewton:
         return s, costs
 
     def update(self, stepsize=None):
+        self.version += 1
         s = None if stepsize is None else L.f64(np.broadcast_to(np.asarray(stepsize, dtype=np.float64), (self.N,)), (self.N,), "stepsize")
         L.check(L.lib().acoc_update(self._h, L.ptr(s)))
 
@@ -356,6 +375,8 @@ class BatchedNewton:
     # stream of the device and returns once its outputs are written, so they may be used on any stream.
     def set_refs_dev(self, xx_ref, uu_ref):
         """set_refs from float64 CUDA tensors xx_ref (N,6,TT) / uu_ref (N,2,TT), or (6,TT) / (2,TT) with refs_shared."""
+        self.version += 1
+        self._refs_param = False
         import torch
         sx = (6, self.TT) if self.refs_shared else (self.N, 6, self.TT)
         su = (2, self.TT) if self.refs_shared else (self.N, 2, self.TT)
@@ -365,6 +386,7 @@ class BatchedNewton:
 
     def set_init_dev(self, xx_init, uu_init):
         """set_init from float64 CUDA tensors xx_init (N,6,TT) / uu_init (N,2,TT)."""
+        self.version += 1
         import torch
         xi = L.dev_tensor(xx_init, self.device, (self.N, 6, self.TT), torch.float64, "xx_init")
         ui = L.dev_tensor(uu_init, self.device, (self.N, 2, self.TT), torch.float64, "uu_init")
@@ -430,6 +452,36 @@ class BatchedNewton:
             return torch.empty(shape, dtype=torch.int32 if integer else torch.float64, device=dev)
         return mc_call(lambda t, out: L.lib().acoc_track_mc_dev(self._h, L.ptr(Q), L.ptr(R), L.ptr(QT), M, d, int(shared), t, out, stream),
                        self.N, M, tol, per_sample, empty)
+
+    # -- derivative of the optimum (include/acoc.h "derivative of the optimum") ------------------------------------------------------
+    def _vjp_out(self, empty):
+        o = dict(xref=empty((self.N, 6, self.TT), False), uref=empty((self.N, 2, self.TT), False), x0=empty((self.N, 6), False),
+                 zf=empty((self.N,), False) if self._refs_param else None, vx=empty((self.N,), False) if self._refs_param else None,
+                 n_indef=empty((self.N,), True))
+        return o
+
+    def result_vjp(self, gx, gu):
+        """Reverse-mode derivative of result() (the optimum of the smooth float64 problem, linearised at the returned point) with respect
+        to the references and the initial state: upstream gradients gx (N,6,TT), gu (N,2,TT) with respect to result()'s arrays -> dict(
+        xref (N,6,TT), uref (N,2,TT), x0 (N,6), zf (N) and vx (N) with parametric references (set_refs_step / set_refs_acrobatic; else None),
+        n_indef (N) = steps whose G = R + B'PB is not positive definite).  zf / vx do not include the path through x0; see
+        aircraftoptimalcontrol_b200.autograd.  Changes nothing of the solve."""
+        g1, g2 = L.f64(gx, (self.N, 6, self.TT), "gx"), L.f64(gu, (self.N, 2, self.TT), "gu")
+        o = self._vjp_out(lambda shape, integer: np.empty(shape, dtype=np.int32 if integer else np.float64))
+        s = L.VjpOut(*(L.ptr(o[k]) for k in ("xref", "uref", "x0", "zf", "vx", "n_indef")))
+        L.check(L.lib().acoc_result_vjp(self._h, L.ptr(g1), L.ptr(g2), C.addressof(s)))
+        return o
+
+    def result_vjp_dev(self, gx, gu):
+        """result_vjp with float64 CUDA tensors gx (N,6,TT), gu (N,2,TT); returns the same dict with CUDA tensors (n_indef int32)."""
+        import torch
+        p1 = L.dev_tensor(gx, self.device, (self.N, 6, self.TT), torch.float64, "gx")
+        p2 = L.dev_tensor(gu, self.device, (self.N, 2, self.TT), torch.float64, "gu")
+        dev = torch.device("cuda", self.device)
+        o = self._vjp_out(lambda shape, integer: torch.empty(shape, dtype=torch.int32 if integer else torch.float64, device=dev))
+        s = L.VjpOut(*(None if o[k] is None else o[k].data_ptr() for k in ("xref", "uref", "x0", "zf", "vx", "n_indef")))
+        L.check(L.lib().acoc_result_vjp_dev(self._h, p1, p2, C.addressof(s), L.dev_stream(self.device)))
+        return o
 
     def set_profiling(self, on=True):
         L.check(L.lib().acoc_set_profiling(self._h, int(bool(on))))

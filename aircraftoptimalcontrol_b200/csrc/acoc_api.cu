@@ -568,6 +568,27 @@ __global__ void __launch_bounds__(128) k_track_mc_reduce(const double* __restric
     n_within[i] = nw;
 }
 
+// ---- derivative of the optimum (acoc_result_vjp) -----------------------------------------------------------------------------------
+// the adjoint sweeps with plain global loads (ACOC_NO_TMA): same per-instance functions as the TMA rings
+template <int DG, typename XT>
+__global__ void __launch_bounds__(64) k_vjp_backward(Problem P, const XT* __restrict__ Xnom, const double* __restrict__ Unom,
+                                                     const double* __restrict__ GX, const double* __restrict__ GU, double* __restrict__ VKS,
+                                                     double* __restrict__ xi_bar, int* __restrict__ n_indef)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P.N) return;
+    n_indef[i] = vjp_backward_instance<DG>(P, Xnom, Unom, GX, GU, VKS, xi_bar, i);
+}
+template <int DG, typename XT>
+__global__ void __launch_bounds__(64) k_vjp_forward(Problem P, const XT* __restrict__ Xnom, const double* __restrict__ Unom,
+                                                    const double* __restrict__ VKS, const double* __restrict__ vs, double* __restrict__ XB,
+                                                    double* __restrict__ UB, double* __restrict__ zv)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= P.N) return;
+    vjp_forward_instance<DG>(P, Xnom, Unom, VKS, vs, XB, UB, zv, i);
+}
+
 // dx0 and x0_out may alias (each thread reads its dx0 before it writes its x0)
 template <bool Q32, typename F, typename XT>
 __global__ void __launch_bounds__(ROLL_THREADS) k_init_guess(ProblemT<F> P, double kp, double kt, const F* dx0, XT* __restrict__ Xn,
@@ -987,6 +1008,14 @@ struct acoc_ctx {
     cudaEvent_t tk_ev[4] = {};
     double tk_ms[4] = {0, 0, 0, 0};
     cudaEvent_t ev_caller = nullptr;  // the caller's stream -> the context's stream (_dev entry points), created on first use
+    // derivative of the optimum (acoc_result_vjp), allocated on the first call: nominal Xnom / Unom + exact row 0 (warp-tiled, states of
+    // vj_es bytes), gbar gx | gu (overwritten by xref_bar | uref_bar), K / sigma [TT][14], per-instance rows xi_bar | zf_bar | vx_bar [8][Np],
+    // n_indef [Np], the speed table of the step maneuver [TT]
+    void *vj_xnom = nullptr, *vj_unom = nullptr, *vj_xnom0 = nullptr, *vj_gx = nullptr, *vj_gu = nullptr, *vj_ks = nullptr, *vj_rows = nullptr;
+    void* vj_vs = nullptr;
+    int* vj_nind = nullptr;
+    size_t vj_es = 0;           // 0: not allocated
+    std::vector<double> rp_vshape;  // vshape of the last acoc_set_refs_generated (empty: none), for the chain rule of zf_bar / vx_bar
 };
 
 static int dalloc_bytes(acoc_ctx* c, void** p, size_t bytes)
@@ -1651,6 +1680,8 @@ int acoc_set_refs_generated(acoc_ctx* c, const double* tt, const double* zshape,
         CK(cudaGetLastError());
         CK(cudaStreamSynchronize(c->stream));
         c->rp_has_v = vshape != nullptr;
+        if (vshape) c->rp_vshape.assign(vshape, vshape + T);
+        else c->rp_vshape.clear();
         c->P.ref_param = 1;
         for (int k = 0; k < 6; ++k) c->P.rp_xc[k] = xconst[k];
         c->P.rp_uc[0] = uconst[0]; c->P.rp_uc[1] = uconst[1];
@@ -3498,6 +3529,114 @@ int acoc_lqr_tracking_mc(int device, int n, int m, int TT, const double* params,
     TRY(ensure_mc_buffers(c, (size_t)n * m, delta_shared ? per : (size_t)n * per));
     CK(cudaEventRecord(c->tk_ev[0], c->stream));
     return track_mc_run(c, xf, W, m, delta, delta_shared, tol, out);
+}
+
+// ======================================================================================================
+// derivative of the optimum with respect to the references and the initial state (acoc_result_vjp)
+// ======================================================================================================
+static void free_vjp_buffers(acoc_ctx* c)
+{
+    dfree(c, &c->vj_xnom); dfree(c, &c->vj_unom); dfree(c, &c->vj_xnom0); dfree(c, &c->vj_gx); dfree(c, &c->vj_gu); dfree(c, &c->vj_ks);
+    dfree(c, &c->vj_rows); dfree(c, &c->vj_vs); dfree(c, &c->vj_nind);
+    c->vj_es = 0;
+}
+
+// the buffers of acoc_result_vjp for state elements of es bytes (reallocated when the storage type changes); ACOC_ERR_NOMEM leaves none
+// behind and touches nothing else of the context
+static int ensure_vjp_buffers(acoc_ctx* c, size_t es)
+{
+    if (c->vj_es == es) return 0;
+    CK(cudaStreamSynchronize(c->stream));
+    free_vjp_buffers(c);
+    const size_t T = c->TT, Np = c->Np, d = sizeof(double);
+    int rc = dalloc_bytes(c, &c->vj_xnom, T * NS * Np * es);
+    if (!rc) rc = dalloc_bytes(c, &c->vj_unom, T * NI * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->vj_xnom0, NS * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->vj_gx, T * NS * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->vj_gu, T * NI * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->vj_ks, T * 14 * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->vj_rows, 8 * Np * d);
+    if (!rc) rc = dalloc_bytes(c, &c->vj_vs, T * d);
+    if (!rc) rc = dalloc(c, &c->vj_nind, Np);
+    if (rc) { free_vjp_buffers(c); return rc; }
+    c->vj_es = es;
+    return 0;
+}
+
+// nominal (k_track_nominal into the VJP's own buffers: the tracking getters keep their answers), the two sweeps, and the outputs
+template <typename XT>
+static int vjp_sweeps(acoc_ctx* c, bool param, bool want_x, bool want_u)
+{
+    cudaStream_t st = c->stream;
+    k_result_slot_default<<<(c->N + 255) / 256, 256, 0, st>>>(c->S.status, c->slot_tmp, c->S.result_slot, c->kk % 3, c->N);
+    const int tchunk = 8;
+    const dim3 ngrid((unsigned)((c->N + 127) / 128), (unsigned)((c->TT + tchunk - 1) / tchunk));
+    k_track_nominal<XT><<<ngrid, 128, 0, st>>>((const XT*)c->X[0], (const XT*)c->X[1], (const XT*)c->X[2], (const double*)c->U[0],
+                                               (const double*)c->U[1], (const double*)c->U[2], c->slot_tmp, (const double*)c->x0, (XT*)c->vj_xnom,
+                                               (double*)c->vj_unom, (double*)c->vj_xnom0, c->N, c->Np, c->TT, tchunk);
+    CK(cudaGetLastError());
+    Problem P = prob<double>(c);
+    P.x0 = (const double*)c->vj_xnom0;
+    const XT* Xn = (const XT*)c->vj_xnom;
+    const double *Un = (const double*)c->vj_unom, *vs = param && c->rp_has_v ? (const double*)c->vj_vs : nullptr;
+    double *GX = (double*)c->vj_gx, *GU = (double*)c->vj_gu, *KS = (double*)c->vj_ks, *rows = (double*)c->vj_rows;
+    double *XB = want_x ? GX : nullptr, *UB = want_u ? GU : nullptr, *zv = param ? rows + (size_t)NS * c->Np : nullptr;
+    const int g = (c->N + 63) / 64;  // 64 threads = two tiles per CTA
+    TRY(with_flag(P.W.diag != 0, [&](auto DG) {
+        if (use_tma(c)) {
+            TRY(launch_ring(k_vjp_backward_tma<DG, XT>, g, 64, WarpRing<VJP_BWD_STAGES, VjpBwdStage<XT>::BYTES>::smem_bytes(2), st, P, Xn, Un,
+                            (const double*)GX, (const double*)GU, KS, rows, c->vj_nind));
+            return launch_ring(k_vjp_forward_tma<DG, XT>, g, 64, WarpRing<VJP_FWD_STAGES, VjpFwdStage<XT>::BYTES>::smem_bytes(2), st, P, Xn, Un,
+                               (const double*)KS, vs, XB, UB, zv);
+        }
+        k_vjp_backward<DG, XT><<<g, 64, 0, st>>>(P, Xn, Un, GX, GU, KS, rows, c->vj_nind);
+        k_vjp_forward<DG, XT><<<g, 64, 0, st>>>(P, Xn, Un, KS, vs, XB, UB, zv);
+        return 0;
+    }));
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// acoc_result_vjp (dev = false) and acoc_result_vjp_dev
+static int result_vjp(acoc_ctx* c, const double* gx, const double* gu, const acoc_vjp_out* out, bool dev)
+{
+    REQUIRE(c, "ctx is NULL");
+    if (c->fp32) return fail(ACOC_ERR_STATE, "acoc_result_vjp: not available in the FP32 mode (ACOC_FP32)");
+    if (!c->have_init) return fail(ACOC_ERR_STATE, "acoc_result_vjp: no result yet: call acoc_set_init or acoc_init_guess first");
+    if (!c->have_weights || !c->have_refs) return fail(ACOC_ERR_STATE, "acoc_result_vjp: set the weights and the references first");
+    REQUIRE(gx && gu, "acoc_result_vjp: gx and gu are required");
+    const acoc_vjp_out o = out ? *out : acoc_vjp_out{};
+    const bool param = c->P.ref_param != 0;
+    REQUIRE(param || (!o.zf_bar && !o.vx_bar), "acoc_result_vjp: zf_bar / vx_bar need parametric references (acoc_set_refs_generated)");
+    TRY(use_device(c->device));
+    const bool xf = c->x_float;
+    TRY(ensure_vjp_buffers(c, xf ? sizeof(float) : sizeof(double)));
+    if (param && c->rp_has_v)
+        CK(cudaMemcpyAsync(c->vj_vs, c->rp_vshape.data(), (size_t)c->TT * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    TRY((upload_soa_t<double, double>(c, gx, c->vj_gx, c->N, NS, c->Np, (double*)nullptr, (int*)nullptr, dev)));
+    TRY((upload_soa_t<double, double>(c, gu, c->vj_gu, c->N, NI, c->Np, (double*)nullptr, (int*)nullptr, dev)));
+    TRY(xf ? vjp_sweeps<float>(c, param, o.xref_bar, o.uref_bar) : vjp_sweeps<double>(c, param, o.xref_bar, o.uref_bar));
+    if (o.xref_bar) TRY(download_soa_t<double>(c, c->vj_gx, nullptr, nullptr, nullptr, nullptr, o.xref_bar, c->N, NS, c->Np, 0, dev));
+    if (o.uref_bar) TRY(download_soa_t<double>(c, c->vj_gu, nullptr, nullptr, nullptr, nullptr, o.uref_bar, c->N, NI, c->Np, 0, dev));
+    const double* rows = (const double*)c->vj_rows;
+    TRY(download_rows(c, rows, o.x0_bar, NS, dev));
+    TRY(download_rows(c, rows + (size_t)NS * c->Np, o.zf_bar, 1, dev));
+    TRY(download_rows(c, rows + (size_t)(NS + 1) * c->Np, o.vx_bar, 1, dev));
+    TRY(download_rows(c, c->vj_nind, o.n_indef, 1, dev));
+    CK(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int acoc_result_vjp(acoc_ctx* c, const double* gx, const double* gu, acoc_vjp_out* out) { return result_vjp(c, gx, gu, out, false); }
+
+int acoc_result_vjp_dev(acoc_ctx* c, const double* gx_dev, const double* gu_dev, acoc_vjp_out* out_dev, void* stream)
+{
+    const acoc_vjp_out o = out_dev ? *out_dev : acoc_vjp_out{};
+    TRY(dev_begin(c, stream, "acoc_result_vjp_dev", {{gx_dev, "gx_dev"}, {gu_dev, "gu_dev"}, {o.xref_bar, "out_dev->xref_bar"},
+                                                     {o.uref_bar, "out_dev->uref_bar"}, {o.x0_bar, "out_dev->x0_bar"},
+                                                     {o.zf_bar, "out_dev->zf_bar"}, {o.vx_bar, "out_dev->vx_bar"},
+                                                     {o.n_indef, "out_dev->n_indef"}}));
+    return dev_end(c, result_vjp(c, gx_dev, gu_dev, out_dev, true));
 }
 
 // ======================================================================================================

@@ -1055,6 +1055,191 @@ ACOC_HD int track_mc_reduce(const F* em, const F* ef, int M, const F* tol, F* wo
 }
 
 // ------------------------------------------------------------------------------------------------------
+// derivative of the optimum with respect to the references and the initial state (acoc_result_vjp; definition in include/acoc.h)
+// ------------------------------------------------------------------------------------------------------
+// The adjoint LQ problem along the result (x*, u*):  min 1/2 w'Hw - gbar'w  s.t.  w_{x,t+1} = A_t w_{x,t} + B_t w_{u,t},  w_{x,0} = 0,
+// H = the Hessian of the Lagrangian (Q + lam_{t+1}-contracted f_xx, S_t, R; Q_T at t = TT-1).  The backward sweep carries the adjoint's
+// value function V_t(w) = 1/2 w'P_t w + p_t'w and the costate lam of the original problem (the Newton sweep's recursion, with the
+// exact Hessian at every step).  riccati_matrix's affine terms are half the linear terms (q/2, r/2), so the sweep hands it q = -2 gbar_x,
+// r = -2 gbar_u (exact scalings).  The gains use the plain G^-1 (never G + 0.5 I): the result is then the exact solution of the KKT
+// system wherever it is nonsingular; the steps whose G is not positive definite (riccati_gain_test) are counted.
+// The sensitivity of the initial state needs no forward pass: x0 enters the adjoint only through w_{x,0}, so xi_bar = gbar_{x,0} -
+// A_0'eta_1 - S_0'w_{u,0} = -grad V_0(0) = -p_0 (with the linear term -gbar_{x,0} of step 0 folded into p_0).
+// VKS (warp-tiled, 14 components): K_t row-major 2x6, sigma_t.
+
+// terminal condition: P = QT, p = -gbar_{x,TT-1}, lam = QT (x*_{TT-1} - xref_{TT-1})
+template <int DG = -1, typename F>
+ACOC_HD void vjp_terminal(const WeightsT<F>& W, const F* x, const F* xr, const F* gx, F* Pm, F* p, F* lam)
+{
+    F dx[NS];
+#pragma unroll
+    for (int c = 0; c < NS; ++c) dx[c] = x[c] - xr[c];
+    wmul6(W.QT, (int)weights_diag<DG>(W), dx, lam);
+    track_terminal<DG>(W, Pm, p);
+#pragma unroll
+    for (int c = 0; c < NS; ++c) p[c] = -gx[c];
+}
+
+// riccati_matrix_by_columns with the plain inverse in the gains.  Returns 1 if G is not positive definite.
+template <int DG = -1, typename F>
+ACOC_HD int vjp_matrix(const ModelT<F>& M, const WeightsT<F>& W, const Lin<F>& l, const Hess<F>& h, const F* q, const F* r, F* Pm, F* p, F* K,
+                       F* sig)
+{
+    RicGain<F> gn;
+    riccati_gain_core(M, W, l, r, Pm, p, gn);
+    riccati_gain_test(gn);
+    gn.k00 = gn.gi00; gn.k01 = gn.gi01; gn.k11 = gn.gi11;
+    F Pn[NS][NS], Mx0[NS], Mx1[NS], Atp[NS];
+    riccati_cols_a_<true, DG, 0, F>(M, l, h, Pm, Pn, Mx0, Mx1);
+    riccati_p_sweep(M, l, p, Atp);
+    riccati_cols_b_<true, DG, 0, F>(W, h, gn, Pn, Mx0, Mx1, Pm);
+    riccati_p_finish(q, Atp, Mx0, Mx1, gn.y0, gn.y1, p);
+    riccati_gain_out(gn, Mx0, Mx1, K, sig);
+    return gn.reg;
+}
+
+// one backward step: (x*_t, u*_t, refs, gbar_t) and the carried (P, p, lam_{t+1}) -> K_t, sigma_t; (P, p, lam) at t.  Returns 1 if G_t is
+// not positive definite.
+template <int DG = -1, typename F>
+ACOC_HD int vjp_backward_step(const ModelT<F>& M, const WeightsT<F>& W, const F* x, const F* u, const F* xr, const F* ur, const F* gx,
+                              const F* gu, F* Pm, F* p, F* lam, F* K, F* sig)
+{
+    F dx[NS], du[NI], q[NS], r[NI], qa[NS], ra[NI], g[NI];
+#pragma unroll
+    for (int c = 0; c < NS; ++c) { dx[c] = x[c] - xr[c]; qa[c] = F(-2.0) * gx[c]; }
+#pragma unroll
+    for (int c = 0; c < NI; ++c) { du[c] = u[c] - ur[c]; ra[c] = F(-2.0) * gu[c]; }
+    wmul6(W.Q, (int)weights_diag<DG>(W), dx, q);
+    wmul2(W.R, (int)weights_diag<DG>(W), du, r);
+    const Trig<F> tg = make_trig(x);
+    const Lin<F> l = linearize(M, x, u, tg);
+    const Hess<F> h = hess_contract(M, x, u, tg, l, lam);
+    const int indef = vjp_matrix<DG, F>(M, W, l, h, qa, ra, Pm, p, K, sig);
+    riccati_costate(M, l, q, r, lam, g);
+    return indef;
+}
+
+// gbar of instance i at time t (warp-tiled GX [TT][6], GU [TT][2]); gbar_u[TT-1] is folded into t = TT-2 (result() copies u_{TT-2} there)
+template <typename F>
+ACOC_HD void vjp_load_g(const F* GX, const F* GU, int t, int TT, int Np, int i, F* gx, F* gu)
+{
+#pragma unroll
+    for (int c = 0; c < NS; ++c) gx[c] = GX[at(t, NS, c, Np, i)];
+#pragma unroll
+    for (int c = 0; c < NI; ++c) gu[c] = GU[at(t, NI, c, Np, i)];
+    if (t == TT - 2) {
+#pragma unroll
+        for (int c = 0; c < NI; ++c) gu[c] = gu[c] + GU[at(TT - 1, NI, c, Np, i)];
+    }
+}
+
+// whole backward sweep of one instance over the nominal (X, U; P.x0 = its exact row 0): VKS, xi_bar [6][Np]; returns n_indef
+template <int DG, typename F, typename XT>
+ACOC_HD int vjp_backward_instance(const ProblemT<F>& P, const XT* X, const F* U, const F* GX, const F* GU, F* VKS, F* xi_bar, int i)
+{
+    const int TT = P.TT, Np = P.Np;
+    F Pm[21], p[NS], lam[NS], x[NS], u[NI], xr[NS], ur[NI], gx[NS], gu[NI];
+    load_xref(P, TT - 1, i, xr);
+    load_x(P, X, TT - 1, i, x);
+    vjp_load_g(GX, GU, TT - 1, TT, Np, i, gx, gu);
+    vjp_terminal<DG>(P.W, x, xr, gx, Pm, p, lam);
+    int n = 0;
+    for (int t = TT - 2; t >= 0; --t) {
+        load_ref(P, t, i, xr, ur);
+        load_x(P, X, t, i, x);
+#pragma unroll
+        for (int c = 0; c < NI; ++c) u[c] = U[at(t, NI, c, Np, i)];
+        vjp_load_g(GX, GU, t, TT, Np, i, gx, gu);
+        F K[2 * NS], sig[NI];
+        n += vjp_backward_step<DG>(P.M, P.W, x, u, xr, ur, gx, gu, Pm, p, lam, K, sig);
+#pragma unroll
+        for (int c = 0; c < 12; ++c) VKS[at(t, 14, c, Np, i)] = K[c];
+        VKS[at(t, 14, 12, Np, i)] = sig[0]; VKS[at(t, 14, 13, Np, i)] = sig[1];
+    }
+#pragma unroll
+    for (int c = 0; c < NS; ++c) xi_bar[(size_t)c * Np + i] = -p[c];
+    return n;
+}
+
+// Parametric references (acoc_set_refs_generated): zf_bar, vx_bar from xref_bar by the chain rule, in ascending t.  X_t = vx tt_t,
+// Z_t = zs_t zf, and for the step maneuver V_t = sqrt((vs_t zf)^2 + vx^2): dV/dzf = vs_t^2 zf / V_t, dV/dvx = vx / V_t.
+struct VjpParamSums {
+    double z, zv, x, xv;  // sum zs_t Zbar_t, sum dV/dzf Vbar_t, sum tt_t Xbar_t, sum dV/dvx Vbar_t
+};
+// vs_t, v_t: the step maneuver's speed table entry and this instance's stored V_t (has_v); xb: xref_bar_t
+ACOC_HD void vjp_param_add(VjpParamSums& s, double tt_t, double zs_t, bool has_v, double vs_t, double v_t, double zf, double vx, const double* xb)
+{
+    s.z += zs_t * xb[1];
+    s.x += tt_t * xb[0];
+    if (has_v) {
+        s.zv += (((vs_t * vs_t) * zf) / v_t) * xb[2];
+        s.xv += (vx / v_t) * xb[2];
+    }
+}
+
+// one forward step: w_{u,t} = sigma_t + K_t w_{x,t} (ks: K_t, sigma_t), outputs xb = Q w_{x,t} (QT at TT-1, 0 at t = 0), ub = R w_{u,t},
+// w_{x,t+1} = A_t w_{x,t} + B_t w_{u,t}
+template <int DG = -1, typename F>
+ACOC_HD void vjp_forward_step(const ModelT<F>& M, const WeightsT<F>& W, int t, const F* x, const F* u, const F* ks, F* wx, F* xb, F* ub)
+{
+    F ksg[16], wu[NI];
+#pragma unroll
+    for (int c = 0; c < 14; ++c) ksg[c] = ks[c];
+    ksg[14] = F(0.0); ksg[15] = F(0.0);
+    double unused = 0.0;
+    forward_du(ksg, wx, wu, unused);
+    if (t == 0) {
+#pragma unroll
+        for (int c = 0; c < NS; ++c) xb[c] = F(0.0);
+    } else wmul6(W.Q, (int)weights_diag<DG>(W), wx, xb);
+    wmul2(W.R, (int)weights_diag<DG>(W), wu, ub);
+    forward_advance(M, x, u, wu, wx);
+}
+
+// whole forward sweep of one instance: XB (N,6) / UB (N,2) warp-tiled (either may be nullptr), zv [2][Np] (nullptr: no parametric sums)
+template <int DG, typename F, typename XT>
+ACOC_HD void vjp_forward_instance(const ProblemT<F>& P, const XT* X, const F* U, const F* VKS, const double* vs, F* XB, F* UB, double* zv, int i)
+{
+    const int TT = P.TT, Np = P.Np;
+    const bool has_v = P.ref_param && P.rp_v;
+    const double zf = zv ? (double)P.rp_zf[i] : 0.0, vx = zv ? (double)P.rp_vx[i] : 0.0;
+    VjpParamSums s = {0.0, 0.0, 0.0, 0.0};
+    F wx[NS] = {0, 0, 0, 0, 0, 0}, x[NS], u[NI], ks[14], xb[NS], ub[NI];
+    for (int t = 0; t < TT - 1; ++t) {
+        load_x(P, X, t, i, x);
+#pragma unroll
+        for (int c = 0; c < NI; ++c) u[c] = U[at(t, NI, c, Np, i)];
+#pragma unroll
+        for (int c = 0; c < 14; ++c) ks[c] = VKS[at(t, 14, c, Np, i)];
+        vjp_forward_step<DG>(P.M, P.W, t, x, u, ks, wx, xb, ub);
+        if (XB) {
+#pragma unroll
+            for (int c = 0; c < NS; ++c) XB[at(t, NS, c, Np, i)] = xb[c];
+        }
+        if (UB) {
+#pragma unroll
+            for (int c = 0; c < NI; ++c) UB[at(t, NI, c, Np, i)] = ub[c];
+        }
+        if (zv) vjp_param_add(s, P.rp_tt[t], P.rp_zs[t], has_v, has_v ? vs[t] : 0.0, has_v ? (double)param_vref(P, t, i) : 0.0, zf, vx, xb);
+    }
+    wmul6(P.W.QT, (int)weights_diag<DG>(P.W), wx, xb);
+    if (XB) {
+#pragma unroll
+        for (int c = 0; c < NS; ++c) XB[at(TT - 1, NS, c, Np, i)] = xb[c];
+    }
+    if (UB) {
+#pragma unroll
+        for (int c = 0; c < NI; ++c) UB[at(TT - 1, NI, c, Np, i)] = F(0.0);
+    }
+    if (zv) {
+        const int t = TT - 1;
+        vjp_param_add(s, P.rp_tt[t], P.rp_zs[t], has_v, has_v ? vs[t] : 0.0, has_v ? (double)param_vref(P, t, i) : 0.0, zf, vx, xb);
+        zv[i] = s.z + s.zv;
+        zv[(size_t)Np + i] = s.x + s.xv;
+    }
+}
+
+// ------------------------------------------------------------------------------------------------------
 // initial guess, aircraft_simplified.py:126-148 (float64 arithmetic; see DESIGN.md "initial guess")
 // ------------------------------------------------------------------------------------------------------
 // dx0 (optional, [6][Np]): start from xx_ref[:,0] + dx0 instead (perturbed-initial-state batches, config 5)

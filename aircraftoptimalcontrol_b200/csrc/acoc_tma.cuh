@@ -1573,4 +1573,191 @@ k_track_mc_rollout_tma(Problem P, const XT* __restrict__ Xnom, const double* __r
     for (int c = 0; c < NS; ++c) { em[o + c] = emax[c]; ef[o + c] = efin[c]; }
 }
 
+// =================================================================================================================
+// derivative of the optimum (acoc_result_vjp): the adjoint LQ problem along the result (vjp_backward_instance / vjp_forward_instance)
+// =================================================================================================================
+// backward sweep: in x*_t, u*_t, references, gbar_t (walking t = TT-2 .. 0); out K_t, sigma_t, and per instance xi_bar, n_indef.  The
+// step is k_backward_tma's exact-Hessian step (column pieces of the Riccati update, the costate recursion), plus the 64 B of gbar.
+constexpr int VJP_BWD_STAGES = 3;
+template <typename XT>
+struct VjpBwdStage {
+    static constexpr int U_B = NI * TILE * sizeof(double), XR_B = NS * TILE * sizeof(double), X_B = NS * TILE * sizeof(XT);
+    static constexpr int U_O = 0, UR_O = U_B, GU_O = 2 * U_B, XR_O = 3 * U_B, GX_O = 3 * U_B + XR_B, X_O = 3 * U_B + 2 * XR_B, BYTES = X_O + X_B;
+};
+
+template <int DG, typename XT>
+__global__ void __launch_bounds__(64) k_vjp_backward_tma(Problem P, const XT* __restrict__ X, const double* __restrict__ U,
+                                                         const double* __restrict__ GX, const double* __restrict__ GU, double* __restrict__ VKS,
+                                                         double* __restrict__ xi_bar, int* __restrict__ n_indef)
+{
+    using St = VjpBwdStage<XT>;
+    extern __shared__ __align__(128) unsigned char smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const int tile = blockIdx.x * nw + warp;
+    if (tile * TILE >= P.N) return;  // warp-uniform
+    WarpRing<VJP_BWD_STAGES, St::BYTES> ring;
+    ring.init(smem, warp, nw, lane);
+    const int TT = P.TT, Np = P.Np, i = tile * TILE + lane, nsteps = TT - 1;
+    const bool live = i < P.N;
+    const RefMode<double> rm(P, i, live);
+    auto issue = [&](int k) {  // ring step k <-> time t = TT-2-k
+        const int t = TT - 2 - k;
+        unsigned char* st = ring.stage(k);
+        uint64_t* b = ring.barrier(k);
+        mbar_arrive_expect_tx(b, 2 * St::U_B + St::XR_B + St::X_B + (rm.tiled ? St::U_B + St::XR_B : 0) +
+                                     (rm.has_v ? (uint32_t)(TILE * sizeof(double)) : 0));
+        tma_load(st + St::U_O, U + tile_base(t, NI, Np, tile), St::U_B, b);
+        tma_load(st + St::X_O, X + tile_base(t, NS, Np, tile), St::X_B, b);
+        tma_load(st + St::GU_O, GU + tile_base(t, NI, Np, tile), St::U_B, b);
+        tma_load(st + St::GX_O, GX + tile_base(t, NS, Np, tile), St::XR_B, b);
+        if (rm.tiled) {
+            tma_load(st + St::UR_O, P.uref + tile_base(t, NI, Np, tile), St::U_B, b);
+            tma_load(st + St::XR_O, P.xref + tile_base(t, NS, Np, tile), St::XR_B, b);
+        } else if (rm.has_v)
+            tma_load(st + St::XR_O, P.rp_v + tile_base(t, 1, Np, tile), (uint32_t)(TILE * sizeof(double)), b);
+    };
+    if (lane == 0)
+        for (int k = 0; k < VJP_BWD_STAGES && k < nsteps; ++k) issue(k);
+    double Pm[21], p[NS], lam[NS], x[NS], u[NI], xr[NS], ur[NI], gx[NS], gu[NI], gl[NI];
+    int n = 0;
+    if (live) {
+        load_xref(P, TT - 1, i, xr);
+        load_x(P, X, TT - 1, i, x);
+        vjp_load_g(GX, GU, TT - 1, TT, Np, i, gx, gu);
+        vjp_terminal<DG>(P.W, x, xr, gx, Pm, p, lam);
+#pragma unroll
+        for (int c = 0; c < NI; ++c) gl[c] = gu[c];  // gbar_u[TT-1], folded into step TT-2
+    }
+    for (int k = 0; k < nsteps; ++k) {
+        const int t = TT - 2 - k;
+        ring.wait(k);
+        const unsigned char* st = ring.stage(k);
+        XT xraw[NS];
+#pragma unroll
+        for (int c = 0; c < NS; ++c) xraw[c] = reinterpret_cast<const XT*>(st + St::X_O)[c * TILE + lane];
+#pragma unroll
+        for (int c = 0; c < NS; ++c) gx[c] = reinterpret_cast<const double*>(st + St::GX_O)[c * TILE + lane];
+#pragma unroll
+        for (int c = 0; c < NI; ++c) {
+            u[c] = reinterpret_cast<const double*>(st + St::U_O)[c * TILE + lane];
+            gu[c] = reinterpret_cast<const double*>(st + St::GU_O)[c * TILE + lane];
+        }
+        double vv = 0.0;
+        if (rm.tiled) {
+#pragma unroll
+            for (int c = 0; c < NI; ++c) ur[c] = reinterpret_cast<const double*>(st + St::UR_O)[c * TILE + lane];
+#pragma unroll
+            for (int c = 0; c < NS; ++c) xr[c] = reinterpret_cast<const double*>(st + St::XR_O)[c * TILE + lane];
+        } else if (rm.has_v) vv = reinterpret_cast<const double*>(st + St::XR_O)[lane];
+        stage_release();
+        if (lane == 0 && k + VJP_BWD_STAGES < nsteps) issue(k + VJP_BWD_STAGES);
+        if (live) {
+            if (t == TT - 2) {
+#pragma unroll
+                for (int c = 0; c < NI; ++c) gu[c] = gu[c] + gl[c];  // vjp_load_g's fold
+            }
+            rm.fill(P, t, i, vv, xr, ur);
+            finish_x(P, t, i, xraw, x);
+            double K[2 * NS], sig[NI];
+            n += vjp_backward_step<DG>(P.M, P.W, x, u, xr, ur, gx, gu, Pm, p, lam, K, sig);
+            double* out = VKS + tile_base(t, 14, Np, tile) + lane;
+#pragma unroll
+            for (int c = 0; c < 12; ++c) out[c * TILE] = K[c];
+            out[12 * TILE] = sig[0]; out[13 * TILE] = sig[1];
+        }
+    }
+    if (!live) return;
+#pragma unroll
+    for (int c = 0; c < NS; ++c) xi_bar[(size_t)c * Np + i] = -p[c];
+    n_indef[i] = n;
+}
+
+// forward sweep: in K_t / sigma_t, x*_t, u*_t (and the stored speed reference when the parametric sums are wanted); out xref_bar and
+// uref_bar (skipped when XB / UB are nullptr) and the sums zf_bar, vx_bar (zv [2][Np], nullptr: not parametric)
+constexpr int VJP_FWD_STAGES = 3;
+template <typename XT>
+struct VjpFwdStage {
+    static constexpr int KS_B = 14 * TILE * sizeof(double), U_B = NI * TILE * sizeof(double), V_B = TILE * sizeof(double),
+                         X_B = NS * TILE * sizeof(XT);
+    static constexpr int KS_O = 0, U_O = KS_B, V_O = KS_B + U_B, X_O = KS_B + U_B + V_B, BYTES = X_O + X_B;
+};
+
+template <int DG, typename XT>
+__global__ void __launch_bounds__(64) k_vjp_forward_tma(Problem P, const XT* __restrict__ X, const double* __restrict__ U,
+                                                        const double* __restrict__ VKS, const double* __restrict__ vs, double* __restrict__ XB,
+                                                        double* __restrict__ UB, double* __restrict__ zv)
+{
+    using St = VjpFwdStage<XT>;
+    extern __shared__ __align__(128) unsigned char smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const int tile = blockIdx.x * nw + warp;
+    if (tile * TILE >= P.N) return;  // warp-uniform
+    WarpRing<VJP_FWD_STAGES, St::BYTES> ring;
+    ring.init(smem, warp, nw, lane);
+    const int TT = P.TT, Np = P.Np, i = tile * TILE + lane, nsteps = TT - 1;
+    const bool live = i < P.N;
+    const bool has_v = zv && P.ref_param && P.rp_v;
+    auto issue = [&](int t) {
+        unsigned char* st = ring.stage(t);
+        uint64_t* b = ring.barrier(t);
+        mbar_arrive_expect_tx(b, St::KS_B + St::U_B + St::X_B + (has_v ? St::V_B : 0));
+        tma_load(st + St::KS_O, VKS + tile_base(t, 14, Np, tile), St::KS_B, b);
+        tma_load(st + St::U_O, U + tile_base(t, NI, Np, tile), St::U_B, b);
+        tma_load(st + St::X_O, X + tile_base(t, NS, Np, tile), St::X_B, b);
+        if (has_v) tma_load(st + St::V_O, P.rp_v + tile_base(t, 1, Np, tile), St::V_B, b);
+    };
+    if (lane == 0)
+        for (int t = 0; t < VJP_FWD_STAGES && t < nsteps; ++t) issue(t);
+    const double zf = (zv && live) ? P.rp_zf[i] : 0.0, vx = (zv && live) ? P.rp_vx[i] : 0.0;
+    VjpParamSums s = {0.0, 0.0, 0.0, 0.0};
+    double wx[NS] = {0, 0, 0, 0, 0, 0}, xb[NS], ub[NI];
+    for (int t = 0; t < nsteps; ++t) {
+        ring.wait(t);
+        const unsigned char* st = ring.stage(t);
+        double ks[14], u[NI];
+        XT xraw[NS];
+#pragma unroll
+        for (int c = 0; c < 14; ++c) ks[c] = reinterpret_cast<const double*>(st + St::KS_O)[c * TILE + lane];
+#pragma unroll
+        for (int c = 0; c < NS; ++c) xraw[c] = reinterpret_cast<const XT*>(st + St::X_O)[c * TILE + lane];
+#pragma unroll
+        for (int c = 0; c < NI; ++c) u[c] = reinterpret_cast<const double*>(st + St::U_O)[c * TILE + lane];
+        const double vv = has_v ? reinterpret_cast<const double*>(st + St::V_O)[lane] : 0.0;
+        stage_release();
+        if (lane == 0 && t + VJP_FWD_STAGES < nsteps) issue(t + VJP_FWD_STAGES);
+        if (live) {
+            double x[NS];
+            finish_x(P, t, i, xraw, x);
+            vjp_forward_step<DG>(P.M, P.W, t, x, u, ks, wx, xb, ub);
+            if (XB) {
+                double* o = XB + tile_base(t, NS, Np, tile) + lane;
+#pragma unroll
+                for (int c = 0; c < NS; ++c) o[c * TILE] = xb[c];
+            }
+            if (UB) {
+                double* o = UB + tile_base(t, NI, Np, tile) + lane;
+#pragma unroll
+                for (int c = 0; c < NI; ++c) o[c * TILE] = ub[c];
+            }
+            if (zv) vjp_param_add(s, P.rp_tt[t], P.rp_zs[t], has_v, has_v ? vs[t] : 0.0, vv, zf, vx, xb);
+        }
+    }
+    if (!live) return;
+    wmul6(P.W.QT, (int)weights_diag<DG>(P.W), wx, xb);
+    if (XB) {
+#pragma unroll
+        for (int c = 0; c < NS; ++c) XB[at(TT - 1, NS, c, Np, i)] = xb[c];
+    }
+    if (UB) {
+#pragma unroll
+        for (int c = 0; c < NI; ++c) UB[at(TT - 1, NI, c, Np, i)] = 0.0;
+    }
+    if (zv) {
+        const int t = TT - 1;
+        vjp_param_add(s, P.rp_tt[t], P.rp_zs[t], has_v, has_v ? vs[t] : 0.0, has_v ? param_vref(P, t, i) : 0.0, zf, vx, xb);
+        zv[i] = s.z + s.zv;
+        zv[(size_t)Np + i] = s.x + s.xv;
+    }
+}
+
 }  // namespace acoc

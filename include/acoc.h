@@ -303,6 +303,48 @@ int acoc_get_track_gains_dev(acoc_ctx* ctx, double* K_dev, void* stream);
 int acoc_track_mc_dev(acoc_ctx* ctx, const double* Q, const double* R, const double* QT, int m, const double* delta_dev, int delta_shared,
                       const double* tol, acoc_track_mc_out* out_dev, void* stream);
 
+/* ------------------------------------------ derivative of the optimum (vector-Jacobian product) ------------ */
+/* The derivative of what acoc_get_result returns with respect to the references and the initial state, applied to upstream gradients
+ * (reverse mode): the backward pass of a differentiable solve (aircraftoptimalcontrol_b200/autograd.py).
+ * Definition.  For instance i, the optimum is that of the problem the Newton driver solves, with the smooth float64 model (the next
+ * state is NOT rounded to float32: the derivative of a float32-rounded map is zero almost everywhere):
+ *     J = sum_{t=0}^{TT-2} 1/2 (x_t - xref_t)'Q(x_t - xref_t) + 1/2 (u_t - uref_t)'R(u_t - uref_t) + 1/2 (x_{TT-1} - xref_{TT-1})'QT(...)
+ *     s.t. x_{t+1} = f(x_t, u_t),  x_0 = xi.
+ * It is linearised at the returned point (x*, u*) (what acoc_get_result returns now) with the costates lam_{TT-1} = QT (x*_{TT-1} -
+ * xref_{TT-1}), lam_t = A_t' lam_{t+1} + Q (x*_t - xref_t) and H = the Hessian of the Lagrangian there (Q + sum_k lam_{t+1,k} d2f_k,
+ * S_t = the lam-contracted d2f/dudx, R; QT at TT-1) -- the Newton sweep's exact-Hessian terms.  Given gx (N,6,TT) and gu (N,2,TT), the
+ * upstream gradients with respect to the arrays acoc_get_result writes:
+ *   1. gu[:,:,TT-1] is added to gu[:,:,TT-2] (the result repeats u_{TT-2} there); gx[:,:,0] is a gradient of xi itself.
+ *   2. w = argmin 1/2 w'Hw - g'w  s.t.  w_{x,t+1} = A_t w_{x,t} + B_t w_{u,t},  w_{x,0} = 0  (a Riccati sweep with the plain G^-1 in
+ *      the recursion and the gains -- never G + 0.5 I -- and a forward pass): the exact solution of the KKT system wherever that
+ *      system is nonsingular.
+ *   3. xref_bar_t = Q w_{x,t} (1 <= t <= TT-2), QT w_{x,TT-1} at TT-1, 0 at t = 0;  uref_bar_t = R w_{u,t} (t <= TT-2), 0 at TT-1;
+ *      x0_bar = gx_0 - A_0' eta_1 - S_0' w_{u,0} (eta_1: multiplier of the first dynamics constraint of the adjoint problem) = -p_0 of
+ *      the adjoint's Riccati sweep;  n_indef = steps whose G = R + B'PB is not positive definite (there the second-order sufficient
+ *      condition fails: the point is not a strict local optimum and the derivative is that of a KKT point).
+ *   With parametric references (acoc_set_refs_generated) the per-instance chain rule, summed on the device in ascending t:
+ *      zf_bar = sum_t zs_t Xbar_{t,Z} + sum_t (vs_t^2 zf / V_t) Xbar_{t,V},   vx_bar = sum_t tt_t Xbar_{t,X} + sum_t (vx / V_t) Xbar_{t,V}
+ *   (Xbar = xref_bar; the V terms for a stored speed reference only, the step maneuver; V_t the stored table).  They do not include
+ *   the dependence of xi on the references: a caller whose x0 is xref_0 + dx0 (acoc_init_guess) adds x0_bar to that chain itself.
+ * Not built: gradients with respect to the weights or the model parameters, forward mode, the FP32 mode, the tracking calls.
+ * Outputs (any pointer may be NULL): */
+typedef struct acoc_vjp_out {
+    double* xref_bar; /* (N,6,TT); per instance also for ACOC_REFS_SHARED contexts (the caller sums them) */
+    double* uref_bar; /* (N,2,TT) */
+    double* x0_bar;   /* (N,6) */
+    double* zf_bar;   /* (N)  parametric references only (ACOC_ERR_INVALID otherwise) */
+    double* vx_bar;   /* (N)  parametric references only */
+    int* n_indef;     /* (N) */
+} acoc_vjp_out;
+/* Writes nothing of the Newton state (iterates, gains, deltau, histories, statistics) and changes no answer of the tracking getters.  Its
+ * buffers (~(72 + 6 s) * TT + 100 bytes per instance, s = 4 or 8 bytes per stored state) are allocated on the first call and freed with
+ * the context (ACOC_ERR_NOMEM leaves the context unchanged).  An instance whose result is the zero slot or not finite gets NaN and disturbs
+ * no other.  ACOC_ERR_STATE for ACOC_FP32 contexts and before the weights, the references and acoc_set_init / acoc_init_guess;
+ * ACOC_ERR_INVALID for a NULL gx or gu. */
+int acoc_result_vjp(acoc_ctx* ctx, const double* gx, const double* gu, acoc_vjp_out* out);
+/* the twin for device memory (see "device-resident inputs and outputs"): gx_dev, gu_dev and every pointer of *out_dev (n_indef int32) */
+int acoc_result_vjp_dev(acoc_ctx* ctx, const double* gx_dev, const double* gu_dev, acoc_vjp_out* out_dev, void* stream);
+
 /* Single pieces of the loop on the context's current iterate, exposed for parity tests and for the
  * reference's own method names:
  *   acoc_eval_cost        optcon.py:417-424   -> J[N]
